@@ -8,7 +8,11 @@ device by the integer-hash generator the CPU oracle can replay); at --gpus 8 the
 A step = one pass of the scan kernel over the rank's resident shard (inputs 40 GB >> 126 MB L2, so no flush).
 The other BASELINE configs are reported in the same JSON line under the top-level keys "c2", "c4", "c5" and "text".
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--loci-per-gpu L]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--loci-per-gpu L] [--dump-outputs DIR]
+
+--dump-outputs DIR writes the records of the last timed step (a fixed, seeded sample of the shard's loci, the output
+rows of each) as DIR/<name>.npy in f64, so that two builds can be compared output for output on the same synthetic
+inputs.
 """
 from __future__ import annotations
 
@@ -30,6 +34,8 @@ LOCI_PER_GPU = 1_250_000
 SEED = 0x5EED0003
 ALG_BYTES_PER_LOCUS = 8 * N_POOLS * N_ALLELES + 32 * (N_ALLELES - 1) * N_PHEN  # SURVEY.md 8(d): 32,288 B
 METRIC = "loci/sec for ols_iter (f64)"
+DUMP_BYTES = 60_000_000  # all ranks' --dump-outputs files together, below 64 MB with room for the .npy headers
+DUMP_SEED = 0x5EED00D
 
 
 def measured_peaks():
@@ -222,6 +228,23 @@ def run_reference(args):
     return 0
 
 
+def sample_records(res, first_locus: int, world: int) -> dict:
+    """the ScanResults of a shard reduced to a fixed, seeded sample of its loci (all of them when they fit), every
+    array in f64; the samples of all ranks together stay under DUMP_BYTES.  The library leaves the slots of a locus that
+    hold no output row NaN (all of them when the locus is filtered or failed): freq_mean [rows] and stats [rows, k, 4]
+    keep the output rows only, in locus order, and status / n_out say which locus each row belongs to."""
+    L, S = res.freq_mean.shape
+    per_locus = 8 * (1 + 1 + 1 + res.alleles.shape[1] + S + res.stats[0].size)
+    n = min(L, DUMP_BYTES // (world * per_locus))
+    idx = np.arange(L) if n == L else np.sort(np.random.default_rng(DUMP_SEED).choice(L, n, replace=False))
+    from poolgen_b200.capi import LOCUS_OK
+    status, n_out = res.status[idx], res.n_out[idx]
+    rows = (status == LOCUS_OK)[:, None] & (np.arange(S)[None, :] < n_out[:, None])
+    return {"locus": (first_locus + idx).astype(np.float64), "status": status.astype(np.float64),
+            "n_out": n_out.astype(np.float64), "alleles": res.alleles[idx].astype(np.float64),
+            "freq_mean": res.freq_mean[idx][rows], "stats": res.stats[idx][rows]}
+
+
 def bind_to_gpu_numa_node(gpu_index: int):
     """pin this process to the CPUs next to its GPU (NVML's ideal affinity) BEFORE any pinned host memory is allocated:
     with 8 ranks on one box the slabs of the end-to-end leg otherwise sit on one socket and every copy crosses it"""
@@ -278,6 +301,14 @@ def run_cuda(args):
     barrier()
     ms, launches = batch.time_runs(args.steps)  # CUDA events on the stream the kernels are launched on
     barrier()
+    # the records of the last timed step, copied out before the batch runs again: the OK fraction (a sanity check, not a
+    # parity test: tests/ does that) and the --dump-outputs sample
+    batch.download()
+    batch.sync()
+    rv = batch.results_view()
+    meta = np.ctypeslib.as_array(rv.meta, shape=(L,))
+    ok_frac = float(((meta & 0xFF) == pb.LOCUS_OK).mean())
+    dump = sample_records(pb.ScanResults.from_c(rv), rank * L, world) if args.dump_outputs else None
     # the timed region can be shorter than nvidia-smi's sampling period: keep the same kernel running (untimed) until
     # at least three clock samples were taken under load
     t_end = time.time() + 4.0
@@ -324,13 +355,6 @@ def run_cuda(args):
     h2d = slab * N_ALLELES * N_POOLS * host.dtype.itemsize
     d2h = slab * (8 + 8 * (N_ALLELES - 1) + 32 * (N_ALLELES - 1) * N_PHEN)
     ctx.pinned_free(hptr)
-
-    # sanity on the results of the timed scan (not a parity test: tests/ does that)
-    batch.download()
-    batch.sync()
-    rv = batch.results_view()
-    meta = np.ctypeslib.as_array(rv.meta, shape=(L,))
-    ok_frac = float(((meta & 0xFF) == pb.LOCUS_OK).mean())
 
     batch.close()
     scan.close()
@@ -398,6 +422,10 @@ def run_cuda(args):
         if cpus is not None:
             line["config"]["cpu_affinity"] = f"each rank bound to the {len(cpus)} CPUs next to its GPU (NVML)"
         os.write(real_stdout, (json.dumps(line) + "\n").encode())
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + (f".rank{rank}" if world > 1 else "") + ".npy"), a)
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
@@ -709,7 +737,12 @@ def main():
     ap.add_argument("--c5-loci", type=int, default=50_000_000, help="loci of the C5 leg (BASELINE: 50M)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg (profiling runs)")
     ap.add_argument("--cpu-seconds", type=float, default=2.5, help="target seconds per step of the --impl reference arm")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the records of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs needs --impl cuda: the reference arm times a sample whose size depends on the CPU")
     if args.impl == "reference":
         return run_reference(args)
     return run_cuda(args)
