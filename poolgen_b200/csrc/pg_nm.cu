@@ -282,15 +282,38 @@ __global__ void __launch_bounds__(kMleWarps * 32) mle_kernel(const NmParams p) {
             const unsigned cg = __shfl_sync(PG_FULL_MASK, colw, g), kg = __shfl_sync(PG_FULL_MASK, kept, g);
             const double *fl = p.freq + (size_t)(l0 + g) * p.lay.freq_stride();
             const uint32_t *dl = p.depth + (size_t)(l0 + g) * p.lay.depth_stride();
-            double sx[PG_MAX_SLOTS];
-            for (int a = 0; a < PG_MAX_SLOTS; a++) sx[a] = 0.0;
+            double sx[PG_MAX_SLOTS], lo[PG_MAX_SLOTS], hi[PG_MAX_SLOTS];
+            for (int a = 0; a < PG_MAX_SLOTS; a++) sx[a] = 0.0, lo[a] = INFINITY, hi[a] = -INFINITY;
             for (int i = lane; i < n; i += 32) {
                 double F[PG_MAX_ALLELES];
                 renorm_generic(p, fl, dl, i, kg, F);
-                for (int a = 0; a < mg; a++) sx[a] += F[(cg >> (4 * a)) & 0xfu];
+                for (int a = 0; a < mg; a++) {
+                    const double f = F[(cg >> (4 * a)) & 0xfu];
+                    sx[a] += f;
+                    lo[a] = fmin(lo[a], f);
+                    hi[a] = fmax(hi[a], f);
+                }
             }
+            // A column that is the same double in every pool is a multiple of the intercept.  Its mean is that double,
+            // exactly: the sum / n form leaves an ulp-sized residue in every centred value for most n (1/3, 0.1), and
+            // whether that residue is zero decides r = 0 / 0 (kept) or r = +-1 against another such column (removed),
+            // and a zero or a 1e-31 pivot.  Centred to zero, the column is never removed, removes nothing, and its
+            // zero row of Sxx makes the locus FAILED -- X'X is singular (DESIGN.md 11)
             double xb[PG_MAX_SLOTS];
-            for (int a = 0; a < PG_MAX_SLOTS; a++) xb[a] = (a < mg) ? warp_sum_fixed(sx[a]) / (double)n : 0.0;
+            for (int a = 0; a < PG_MAX_SLOTS; a++) {
+                if (a >= mg) {
+                    xb[a] = 0.0;
+                    continue;
+                }
+                double l = lo[a], h = hi[a];
+#pragma unroll
+                for (int off = 16; off >= 1; off >>= 1) {
+                    l = fmin(l, __shfl_xor_sync(PG_FULL_MASK, l, off));
+                    h = fmax(h, __shfl_xor_sync(PG_FULL_MASK, h, off));
+                }
+                const double mean = warp_sum_fixed(sx[a]) / (double)n;
+                xb[a] = (l == h && mean == mean) ? l : mean;
+            }
             double sxx[15];
             for (int e = 0; e < 15; e++) sxx[e] = 0.0;
             for (int i = lane; i < n; i += 32) {
@@ -460,7 +483,8 @@ __global__ void __launch_bounds__(kMleWarps * 32) mle_kernel(const NmParams p) {
                             vb[c] = ve * dgi[c];
                         }
                     }
-                    if (!act) continue;
+                    // a locus the scan did not pass on keeps NaN records for every phenotype: its filter-only pass
+                    // writes phenotype 0 only, and the rows of the others would be whatever the buffer held
                     for (int s = 0; s < S; s++) {
                         double o0 = nan(""), o1 = nan(""), o2 = nan(""), o3 = nan("");
                         if (status == PG_LOCUS_OK && s < m) {

@@ -14,6 +14,7 @@ import pytest
 import poolgen_b200 as pb
 from oracle import pgo
 from tests import helpers as H
+from tests.test_nm_edges_gpu import check_mle_status
 
 pytestmark = pytest.mark.gpu
 
@@ -89,8 +90,10 @@ def test_mle_iter_synthetic(ctx, n, A, k, L):
     dev = pb.mle_iterate(ctx, full, phen, fs, codes)
     orc = pgo.scan_batch(pgo.SCAN_MLE, full, codes, phen, H.oracle_fs(fs), 8)
     assert ((orc.status == pgo.FILTERED) == (dev.status == pb.LOCUS_FILTERED)).all()
-    both = (orc.status == pgo.OK) & (dev.status == pb.LOCUS_OK)
-    assert both.sum() > 0.5 * L and ((orc.status == pgo.OK) == (dev.status == pb.LOCUS_OK)).mean() > 0.98
+    # statuses: UNSUPPORTED exactly where the reference's design has fewer pools than columns, OK against FAILED only
+    # at a numerically singular X'X (cond > 1e12), nothing else
+    both, why = check_mle_status(full, codes, fs, dev, orc, f"mle_iter n={n} k={k}")
+    assert both.sum() > 0.5 * L, why
     assert (orc.n_out[both] == dev.n_out[both]).all() and (orc.allele[both] == dev.alleles[both]).all()
     S = dev.stats.shape[1]
     slot = np.broadcast_to((np.arange(S)[None, :] < orc.n_out[both][:, None])[:, :, None], (both.sum(), S, k))
