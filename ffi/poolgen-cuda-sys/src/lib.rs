@@ -84,6 +84,8 @@ extern "C" {
     pub fn pg_destroy(ctx: *mut pg_ctx);
     pub fn pg_last_error(ctx: *const pg_ctx) -> *const c_char;
     pub fn pg_device_info(ctx: *mut pg_ctx, sm_count: *mut c_int, cc_major: *mut c_int, cc_minor: *mut c_int, total_mem: *mut usize) -> c_int;
+    /// free and total device memory now (cudaMemGetInfo): size device blocks from what is free on a shared GPU
+    pub fn pg_device_mem_info(ctx: *mut pg_ctx, free_bytes: *mut usize, total_bytes: *mut usize) -> c_int;
     pub fn pg_pinned_alloc(ctx: *mut pg_ctx, bytes: usize, out: *mut *mut c_void) -> c_int;
     pub fn pg_pinned_free(ctx: *mut pg_ctx, p: *mut c_void) -> c_int;
     // ---- scan configuration
@@ -127,6 +129,8 @@ extern "C" {
     pub fn pg_kin_synth(kin: *mut pg_kin, seed: u64, first_locus: i64, n_loci: i64) -> c_int;
     pub fn pg_kin_get_columns(kin: *mut pg_kin, first: i64, count: i64, out: *mut f64) -> c_int;
     pub fn pg_kin_gram(kin: *mut pg_kin) -> c_int;
+    /// K += G G' of the resident columns (blocks 2..B of a column set larger than the device; pg_kin_reset keeps K)
+    pub fn pg_kin_gram_accumulate(kin: *mut pg_kin) -> c_int;
     pub fn pg_kin_gram_time(kin: *mut pg_kin, iters: c_int, ms_total: *mut f32) -> c_int;
     pub fn pg_kin_partial(kin: *mut pg_kin, device_ptr: *mut *mut f64, n_elems: *mut usize) -> c_int;
     pub fn pg_kin_partial_get(kin: *mut pg_kin, out_host: *mut f64) -> c_int;

@@ -103,6 +103,9 @@ int pg_init(int device, pg_ctx **out);
 void pg_destroy(pg_ctx *ctx);
 const char *pg_last_error(const pg_ctx *ctx); /* ctx may be NULL: last error of a failed pg_init */
 int pg_device_info(pg_ctx *ctx, int *sm_count, int *cc_major, int *cc_minor, size_t *total_mem);
+/* free and total device memory at the time of the call (cudaMemGetInfo): the GPU may be shared, so a budget for device
+ * blocks is taken from free_bytes, not from the card's total */
+int pg_device_mem_info(pg_ctx *ctx, size_t *free_bytes, size_t *total_bytes);
 /* pinned host slabs the reader threads parse into */
 int pg_pinned_alloc(pg_ctx *ctx, size_t bytes, void **out);
 int pg_pinned_free(pg_ctx *ctx, void *p);
@@ -202,8 +205,14 @@ int pg_kin_text_labels(pg_kin *kin, const uint64_t **line_offsets, const uint64_
 /* synthetic biallelic columns (two per locus) generated on the device from the integer-hash workload */
 int pg_kin_synth(pg_kin *kin, uint64_t seed, int64_t first_locus, int64_t n_loci);
 int pg_kin_get_columns(pg_kin *kin, int64_t first, int64_t count, double *out /* [count][n_pools] */);
-/* partial Gram matrix of the resident columns (FP64 tensor cores), asynchronous */
+/* partial Gram matrix of the resident columns (FP64 tensor cores), asynchronous: K = G G' */
 int pg_kin_gram(pg_kin *kin);
+/* K += G G' of the resident columns, asynchronous like pg_kin_gram.  Columns beyond one device's memory are taken in
+ * blocks: pg_kin_gram on block 1, then pg_kin_reset + load + pg_kin_gram_accumulate for blocks 2..B (pg_kin_reset
+ * keeps K), then pg_kin_eig_select with P_total = the columns of all blocks.  Each slice sum is added to K in a fixed
+ * order and both triangles get the same value: K is exactly symmetric and a given split is bit-repeatable.  Composes
+ * with pg_kin_allreduce: each GPU accumulates its own blocks, the all-reduce sums the GPUs' totals. */
+int pg_kin_gram_accumulate(pg_kin *kin);
 int pg_kin_gram_time(pg_kin *kin, int iters, float *ms_total);
 int pg_kin_partial(pg_kin *kin, double **device_ptr, size_t *n_elems); /* n_pools x n_pools, synchronises */
 int pg_kin_partial_get(pg_kin *kin, double *out_host);

@@ -27,7 +27,7 @@ ALLELE_NAMES = "ATCGND"  # sync column order, src/base/sync.rs:134-137
 
 # every symbol include/poolgen_cuda.h declares (tests check the library exports each of them)
 ABI_SYMBOLS = [
-    "pg_abi_version", "pg_init", "pg_destroy", "pg_last_error", "pg_device_info", "pg_pinned_alloc",
+    "pg_abi_version", "pg_init", "pg_destroy", "pg_last_error", "pg_device_info", "pg_device_mem_info", "pg_pinned_alloc",
     "pg_pinned_free", "pg_scan_open", "pg_scan_close", "pg_batch_create", "pg_batch_destroy",
     "pg_batch_upload_counts", "pg_batch_upload_counts_u16", "pg_batch_upload_counts_u8", "pg_batch_upload_freq", "pg_batch_upload_sync_text", "pg_batch_text_labels",
     "pg_scan_submit_sync_text", "pg_batch_synth",
@@ -35,7 +35,7 @@ ABI_SYMBOLS = [
     "pg_batch_bytes", "pg_scan_stream_begin", "pg_scan_submit_counts", "pg_scan_submit_counts_u16",
     "pg_scan_submit_counts_u8", "pg_scan_submit_freq", "pg_scan_collect", "pg_scan_text_labels",
     "pg_kin_open", "pg_kin_close", "pg_kin_reset", "pg_kin_columns", "pg_kin_append_columns", "pg_kin_append_counts",
-    "pg_kin_last_labels", "pg_kin_append_sync_text", "pg_kin_text_labels", "pg_kin_synth", "pg_kin_get_columns", "pg_kin_gram", "pg_kin_gram_time", "pg_kin_partial",
+    "pg_kin_last_labels", "pg_kin_append_sync_text", "pg_kin_text_labels", "pg_kin_synth", "pg_kin_get_columns", "pg_kin_gram", "pg_kin_gram_accumulate", "pg_kin_gram_time", "pg_kin_partial",
     "pg_kin_partial_get", "pg_kin_partial_set", "pg_kin_eig_select", "pg_kin_eigvals", "pg_kin_set_covariates",
     "pg_kin_covar_scan", "pg_kin_mle_scan", "pg_format_header", "pg_format_rows", "pg_format_rows_ex", "pg_format_kinship_rows", "pg_format_f64", "pg_sort_loci",
     "pg_format_frequency_header", "pg_format_frequency_rows",
@@ -102,6 +102,7 @@ def lib():
             "pg_destroy": (None, [vp]),
             "pg_last_error": (C.c_char_p, [vp]),
             "pg_device_info": (i, [vp, C.POINTER(i), C.POINTER(i), C.POINTER(i), C.POINTER(C.c_size_t)]),
+            "pg_device_mem_info": (i, [vp, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]),
             "pg_pinned_alloc": (i, [vp, C.c_size_t, pvp]),
             "pg_pinned_free": (i, [vp, vp]),
             "pg_scan_open": (i, [vp, i, C.POINTER(_Filter), i, i, C.POINTER(C.c_uint8), C.POINTER(C.c_double), i, pvp]),
@@ -141,6 +142,7 @@ def lib():
             "pg_kin_synth": (i, [vp, u64, i64, i64]),
             "pg_kin_get_columns": (i, [vp, i64, i64, vp]),
             "pg_kin_gram": (i, [vp]),
+            "pg_kin_gram_accumulate": (i, [vp]),
             "pg_kin_gram_time": (i, [vp, i, C.POINTER(C.c_float)]),
             "pg_kin_partial": (i, [vp, pvp, C.POINTER(C.c_size_t)]),
             "pg_kin_partial_get": (i, [vp, vp]),
@@ -414,6 +416,12 @@ class Context:
         _check(lib().pg_device_info(self._h, C.byref(sm), C.byref(ma), C.byref(mi), C.byref(mem)), self._h, "pg_device_info")
         return {"sm_count": sm.value, "cc": (ma.value, mi.value), "total_mem": mem.value}
 
+    def mem_info(self):
+        """(free, total) device bytes now; free is what other processes on a shared GPU left"""
+        f, t = C.c_size_t(), C.c_size_t()
+        _check(lib().pg_device_mem_info(self._h, C.byref(f), C.byref(t)), self._h, "pg_device_mem_info")
+        return int(f.value), int(t.value)
+
     def pinned_empty(self, shape, dtype):
         """numpy array over a library-owned pinned host slab (freed with the returned handle's .free())."""
         dt = np.dtype(dtype)
@@ -659,8 +667,13 @@ class Kinship:
         self._ck(lib().pg_kin_get_columns(self._h, int(first), int(count), out.ctypes.data), "pg_kin_get_columns")
         return out
 
-    def gram(self):
-        self._ck(lib().pg_kin_gram(self._h), "pg_kin_gram")
+    def gram(self, accumulate: bool = False):
+        """K = G G' of the resident columns; with accumulate, K += G G' (a later block of a column set larger than the
+        device: reset() keeps K)"""
+        if accumulate:
+            self._ck(lib().pg_kin_gram_accumulate(self._h), "pg_kin_gram_accumulate")
+        else:
+            self._ck(lib().pg_kin_gram(self._h), "pg_kin_gram")
 
     def gram_time(self, iters: int) -> float:
         ms = C.c_float()

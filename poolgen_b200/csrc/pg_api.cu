@@ -97,6 +97,18 @@ int pg_device_info(pg_ctx *ctx, int *sm_count, int *cc_major, int *cc_minor, siz
     return PG_OK;
 }
 
+// free and total device memory now (cudaMemGetInfo): other processes share the GPU, so a caller that sizes its blocks
+// from the device takes them from what is free
+int pg_device_mem_info(pg_ctx *ctx, size_t *free_bytes, size_t *total_bytes) {
+    if (!ctx) return PG_ERR_ARG;
+    PG_CUDA(ctx, cudaSetDevice(ctx->device));
+    size_t f = 0, t = 0;
+    PG_CUDA(ctx, cudaMemGetInfo(&f, &t));
+    if (free_bytes) *free_bytes = f;
+    if (total_bytes) *total_bytes = t;
+    return PG_OK;
+}
+
 int pg_pinned_alloc(pg_ctx *ctx, size_t bytes, void **out) {
     if (!ctx || !out) return PG_ERR_ARG;
     PG_CUDA(ctx, cudaSetDevice(ctx->device));

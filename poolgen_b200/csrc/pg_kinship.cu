@@ -339,8 +339,11 @@ __global__ void __launch_bounds__((kGramWarps + 1) * 32, 1) gram_kernel(const Gr
     }
 }
 
-// K[i][j] = K[j][i] = sum over the slices (fixed order) of the partial tiles
-__global__ void __launch_bounds__(256) gram_reduce_kernel(const double *ws, int nt, int n_slices, int n, double *K) {
+// K[i][j] = K[j][i] = sum over the slices (fixed order) of the partial tiles; with `accumulate` that sum is added to the
+// K a previous block left (read from the upper triangle, both triangles written from the one value: K stays exactly
+// symmetric and a given split into blocks is bit-repeatable)
+__global__ void __launch_bounds__(256) gram_reduce_kernel(const double *ws, int nt, int n_slices, int n, int accumulate,
+                                                          double *K) {
     const int ntiles = nt * (nt + 1) / 2;
     const int64_t total = (int64_t)ntiles * kTile * kTile;
     for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
@@ -358,6 +361,7 @@ __global__ void __launch_bounds__(256) gram_reduce_kernel(const double *ws, int 
         if (i >= n || j >= n || j < i) continue;
         double s = 0.0;
         for (int sl = 0; sl < n_slices; sl++) s += ws[((size_t)sl * ntiles + tile_id) * (kTile * kTile) + e];
+        if (accumulate) s = K[(size_t)i * n + j] + s;
         K[(size_t)i * n + j] = s;
         K[(size_t)j * n + i] = s;
     }
@@ -1246,7 +1250,7 @@ int pg_kin_get_columns(pg_kin *h, int64_t first, int64_t count, double *out) {
     return PG_OK;
 }
 
-static int gram_launch(pg_kin *h) {
+static int gram_launch(pg_kin *h, bool accumulate) {
     pg_ctx *ctx = h->ctx;
     const int ntiles = h->nt * (h->nt + 1) / 2;
     const int64_t P_pad = round_up(std::max<int64_t>(h->P, 1), pg::kKC);
@@ -1278,7 +1282,8 @@ static int gram_launch(pg_kin *h) {
     const int grid = (int)std::min<int64_t>(items, ctx->sm_count);
     pg::gram_kernel<<<grid, (pg::kGramWarps + 1) * 32, smem, h->stream>>>(gp);
     KCUDA(ctx, cudaGetLastError());
-    pg::gram_reduce_kernel<<<ctx->sm_count * 4, 256, 0, h->stream>>>(h->d_ws, h->nt, n_slices, h->n, h->d_K);
+    pg::gram_reduce_kernel<<<ctx->sm_count * 4, 256, 0, h->stream>>>(h->d_ws, h->nt, n_slices, h->n, accumulate ? 1 : 0,
+                                                                     h->d_K);
     KCUDA(ctx, cudaGetLastError());
     return PG_OK;
 }
@@ -1286,7 +1291,15 @@ static int gram_launch(pg_kin *h) {
 int pg_kin_gram(pg_kin *h) {
     if (!h) return PG_ERR_ARG;
     KCUDA(h->ctx, cudaSetDevice(h->ctx->device));
-    return gram_launch(h);
+    return gram_launch(h, false);
+}
+
+// K += G G' of the resident columns: a file larger than the device is taken in blocks (pg_kin_gram on the first,
+// pg_kin_gram_accumulate on the others, pg_kin_reset in between), and K ends up the Gram matrix of all of them
+int pg_kin_gram_accumulate(pg_kin *h) {
+    if (!h) return PG_ERR_ARG;
+    KCUDA(h->ctx, cudaSetDevice(h->ctx->device));
+    return gram_launch(h, true);
 }
 
 int pg_kin_gram_time(pg_kin *h, int iters, float *ms_total) {
@@ -1296,7 +1309,7 @@ int pg_kin_gram_time(pg_kin *h, int iters, float *ms_total) {
     KCUDA(ctx, cudaStreamSynchronize(h->stream));
     KCUDA(ctx, cudaEventRecord(h->ev0, h->stream));
     for (int i = 0; i < iters; i++) {
-        int rc = gram_launch(h);
+        int rc = gram_launch(h, false);
         if (rc) return rc;
     }
     KCUDA(ctx, cudaEventRecord(h->ev1, h->stream));

@@ -297,52 +297,135 @@ def _load_all(ctx: Context, fname: str, n_pools: int, fs: FilterStats, keep_p_mi
               block_bytes: int) -> _LoadedColumns:
     """LoadAll::load over the whole file, block by block through the device parser and loader"""
     kin = capi.Kinship(ctx, n_pools, max_columns)
-    max_loci = block_bytes // (12 * n_pools + 5) + 2
-    names, index_of = [], {}
-    chr_index, positions, col_locus, col_allele = [], [], [], []
-    base = 0
+    max_loci = block_bytes // _line_min_bytes(n_pools) + 2
+    lab = _Labels()
     try:
-        with open(fname, "rb") as fh:
-            carry = b""
-            while True:
-                data = fh.read(block_bytes)
-                if not data and not carry:
-                    break
-                block = carry + data
-                if data:
-                    cut = block.rfind(b"\n") + 1
-                    if cut == 0:
-                        raise PgError(f"a line of {fname} is longer than the block size {block_bytes}")
-                    block, carry = block[:cut], block[cut:]
-                else:
-                    carry = b""
-                L, off, pos, loc, alle = kin.append_sync_text(block, fs, max_loci, keep_p_minus_1)
-                for o in off:  # chromosome = the text up to the first tab of the locus' line
-                    o = int(o)
-                    nm = block[o:block.index(b"\t", o)]
-                    if nm not in index_of:
-                        index_of[nm] = len(names)
-                        names.append(nm)
-                    chr_index.append(index_of[nm])
-                positions.append(pos)
-                col_locus.append(loc + base)
-                col_allele.append(alle)
-                base += L
-                if not data:
-                    break
+        for _, block in _text_blocks(fname, block_bytes):
+            lab.add(block, *kin.append_sync_text(block, fs, max_loci, keep_p_minus_1))
     except Exception:
         kin.close()
         raise
-    cat = lambda parts, dt: np.concatenate(parts).astype(dt) if parts else np.zeros(0, dt)
-    return _LoadedColumns(kin, cat(col_locus, np.int64), cat(col_allele, np.uint8), names,
-                          np.array(chr_index, dtype=np.uint32), cat(positions, np.uint64))
+    return lab.finish(kin)
+
+
+# ---- columns beyond one device: the handle holds a device block of columns at a time -------------------------------
+_COLS_PER_LINE = 6  # a locus emits at most six allele columns (--keep-ns with MAF 0 and no --keep-p-minus-1)
+_KIN_RESERVE_BYTES = 1 << 30  # outside the handle: cuSOLVER's and cuBLAS' handles, kernel modules loaded on first use
+
+
+def _line_min_bytes(n_pools: int) -> int:
+    """a locus line holds at least "c\\t0\\tN" + n_pools * "\\t0:0:0:0:0:0" bytes"""
+    return 12 * n_pools + 5
+
+
+def text_block_columns(n_bytes: int, n_pools: int, n_lines: int = None) -> int:
+    """an upper bound of the allele columns a text block of n_bytes bytes (n_lines newlines, if known) can emit: six
+    per line, as many lines as the bytes can hold"""
+    lines = n_bytes // _line_min_bytes(n_pools) + 1
+    if n_lines is not None:
+        lines = min(lines, n_lines + 1)
+    return _COLS_PER_LINE * lines
+
+
+def _grow(need: int, elem: int) -> int:
+    """bytes of a text-scratch buffer of `need` elements (pg_text.cu: grow() keeps an eighth and 64 Ki elements spare)"""
+    return (need + need // 8 + 65536) * elem
+
+
+def kin_device_bytes(n_pools: int, columns: int, k: int, block_bytes: int, sm_count: int) -> int:
+    """Device bytes (plus the pinned copy of the records) a pg_kin handle of `columns` columns takes at most when it is
+    filled from text blocks of at most block_bytes bytes, its Gram matrix formed, its eigen step run and k phenotypes
+    scanned (pg_kinship.cu, pg_text.cu; every buffer at its largest)"""
+    n, ldg = int(n_pools), (int(n_pools) + 3) & ~3
+    cap = -(-max(int(columns), 1) // 16) * 16  # pg_kin_open rounds up to kKC = 16 columns
+    nt = -(-ldg // 128)
+    ntiles = nt * (nt + 1) // 2
+    tile = 128 * 128 * 8
+    # G (+ one tile of slack) and K
+    total = (cap * ldg + 128) * 8 + n * n * 8
+    # Gram workspace: one partial tile per (column slice, tile); slices of >= 16 columns, ~8 waves over the SMs
+    total += min(-(-8 * sm_count // ntiles), cap // 16) * ntiles * tile
+    # eigen step: the matrix, the eigenvalues, syevd's workspace (1 + 6 n + 2 n^2 doubles), info
+    total += n * n * 8 + n * 8 + (1 + 6 * n + 2 * n * n) * 8 + 4
+    # loader scratch of one text block (max_loci loci of six columns) and the device parser's buffers
+    L = block_bytes // _line_min_bytes(n) + 2
+    total += L * 4 + (L + 1) * 8 + L * 6 * 8 + L * 6 + (8 * L + (64 << 10)) + L * 6 * n * 4 + n * 8
+    nb = block_bytes + 1
+    total += _grow(nb + 32, 1) + _grow(nb, 4) + _grow(-(-nb // 4096) + 1, 8)
+    total += nb * (4 + 1 + 4 + 8) + (nb // 256 + 2) * 4 + 2 * L * 8 + (8 * nb // 4096 + (64 << 10)) + 16
+    # records [3][k][columns] on the device and pinned, the list of deferred columns (one entry per column and
+    # phenotype pass), the partial sums of the DMMA scan's pool passes, Q and y~, the Student-t table, the MLE moments
+    total += 2 * 3 * k * cap * 8 + (cap * k + 2) * 8 + -(-cap // 8) * 17 * 64
+    total += (n + 1 + k) * ldg * 8 + (8 << 20) + ((13 + k) * ldg + 13 + 2 * 13 * 13 + k * 15) * 8
+    return total
+
+
+def kin_block_columns(device_bytes: int, n_pools: int, k: int, block_bytes: int, sm_count: int) -> int:
+    """the most columns a handle can hold within device_bytes (kin_device_bytes), 0 if not even one"""
+    lo, hi = 0, max(int(device_bytes), 0) // ((n_pools + 3 & ~3) * 8) + 16
+    while lo < hi:  # kin_device_bytes grows with the columns: the largest count that fits
+        mid = (lo + hi + 1) // 2
+        if kin_device_bytes(n_pools, mid, k, block_bytes, sm_count) <= device_bytes:
+            lo = mid
+        else:
+            hi = mid - 1
+    return lo
+
+
+def _text_blocks(fname: str, block_bytes: int):
+    """(byte offset, text) of line-aligned blocks of at most block_bytes bytes over the whole file"""
+    with open(fname, "rb") as fh:
+        at, carry = 0, b""
+        while True:
+            data = fh.read(block_bytes - len(carry))
+            if not data and not carry:
+                return
+            block = carry + data
+            if data:
+                cut = block.rfind(b"\n") + 1
+                if cut == 0:
+                    raise PgError(f"a line of {fname} is longer than the block size {block_bytes}")
+                block, carry = block[:cut], block[cut:]
+            else:
+                carry = b""
+            yield at, block
+            at += len(block)
+            if not data:
+                return
+
+
+class _Labels:
+    """labels of the loaded loci over the text blocks of a file, in file order"""
+
+    def __init__(self):
+        self.names, self.index_of = [], {}
+        self.chr_index, self.positions, self.col_locus, self.col_allele = [], [], [], []
+        self.base = 0
+
+    def add(self, block, L, off, pos, loc, alle):
+        for o in off:  # chromosome = the text up to the first tab of the locus' line
+            o = int(o)
+            nm = block[o:block.index(b"\t", o)]
+            if nm not in self.index_of:
+                self.index_of[nm] = len(self.names)
+                self.names.append(nm)
+            self.chr_index.append(self.index_of[nm])
+        self.positions.append(pos)
+        self.col_locus.append(loc + self.base)
+        self.col_allele.append(alle)
+        self.base += L
+
+    def finish(self, kin) -> _LoadedColumns:
+        cat = lambda parts, dt: np.concatenate(parts).astype(dt) if parts else np.zeros(0, dt)
+        return _LoadedColumns(kin, cat(self.col_locus, np.int64), cat(self.col_allele, np.uint8), self.names,
+                              np.array(self.chr_index, dtype=np.uint32), cat(self.positions, np.uint64))
 
 
 def _count_columns_bound(fname: str) -> int:
-    """an upper bound of the allele columns LoadAll can emit: five per line"""
+    """an upper bound of the allele columns LoadAll can emit: six per line"""
     with open(fname, "rb") as fh:
         lines = sum(chunk.count(b"\n") for chunk in iter(lambda: fh.read(1 << 24), b"")) + 1
-    return 5 * lines
+    return _COLS_PER_LINE * lines
 
 
 def write_csv(self, ctx: Context, filter_stats: FilterStats, keep_p_minus_1: bool, out: str, n_threads: int,
@@ -374,24 +457,93 @@ def write_csv(self, ctx: Context, filter_stats: FilterStats, keep_p_minus_1: boo
 
 
 def _iter_with_kinship(self, ctx: Context, filter_stats: FilterStats, keep_p_minus_1: bool,
-                       xxt_eigen_variance_explained: float, out: str, n_threads: int, block_bytes: int, method: str) -> str:
+                       xxt_eigen_variance_explained: float, out: str, n_threads: int, block_bytes: int, method: str,
+                       device_bytes: int = None, timings: dict = None) -> str:
+    """One code path for any file size.  The handle holds up to the columns `device_bytes` allows (None: the free device
+    memory less a reserve for the library's fixed allocations).  Pass 1 loads text blocks into the handle and, before
+    a block whose column bound does not fit, forms the Gram matrix of what is resident (pg_kin_gram on the first device
+    block, pg_kin_gram_accumulate on the later ones) and resets the columns.  The eigen step runs once over the sum.
+    With more than one device block, pass 2 scans the block still resident, then re-reads the byte ranges of the others
+    and scans them; their records go to their columns' place.  With one block this is load, Gram, eigen step, scan.
+    `timings` (measurement only): filled with wall seconds per phase; the stream is synchronised after every Gram."""
     if out != "" and os.path.exists(out):
         raise PgError("Cannot write to output file")
     if np.isnan(self.phen_matrix).any():
         raise PgError("pools with missing phenotypes: remove them before the scan (the reference's remove_missing, "
                       "src/gwas/ols.rs:286)")
-    ld = _load_all(ctx, self.filename_sync, len(self.pool_names), filter_stats, keep_p_minus_1,
-                   _count_columns_bound(self.filename_sync), block_bytes)
+    n = len(self.pool_names)
+    k = int(np.asarray(self.phen_matrix).reshape(n, -1).shape[1])
+    sm_count = ctx.info()["sm_count"]
+    if device_bytes is None:
+        device_bytes = ctx.mem_info()[0] - _KIN_RESERVE_BYTES
+    file_cols = _count_columns_bound(self.filename_sync)
+    need = min(text_block_columns(block_bytes, n), file_cols)
+    cap = min(kin_block_columns(device_bytes, n, k, block_bytes, sm_count), file_cols)
+    if cap < need:
+        raise PgError(f"device_bytes {device_bytes} cannot hold one text block of {block_bytes} bytes: its "
+                      f"{need} columns take {kin_device_bytes(n, need, k, block_bytes, sm_count)} bytes")
+    max_loci = block_bytes // _line_min_bytes(n) + 2
+    clock = time.perf_counter
+    tm = {"pass1_load_s": 0.0, "pass1_gram_s": 0.0, "eig_s": 0.0, "pass2_load_s": 0.0, "scan_s": 0.0}
+    kin = capi.Kinship(ctx, n, cap)
+    lab = _Labels()
+    dev_blocks = [[]]  # per device block: (byte offset, bytes, columns) of its text blocks
     try:
-        P = ld.kin.columns
+        def flush():
+            t0 = clock()
+            kin.gram(accumulate=len(dev_blocks) > 1)
+            if timings is not None:
+                kin.partial_device_ptr()  # synchronises the handle's stream
+            tm["pass1_gram_s"] += clock() - t0
+
+        for at, block in _text_blocks(self.filename_sync, block_bytes):
+            if kin.columns + text_block_columns(len(block), n, block.count(b"\n")) > cap:
+                flush()
+                kin.reset()
+                dev_blocks.append([])
+            t0 = clock()
+            L, off, pos, loc, alle = kin.append_sync_text(block, filter_stats, max_loci, keep_p_minus_1)
+            tm["pass1_load_s"] += clock() - t0
+            lab.add(block, L, off, pos, loc, alle)
+            dev_blocks[-1].append((at, len(block), int(loc.size)))
+        ld = lab.finish(kin)
+        P = int(ld.col_locus.size)
         if P == 0:
             raise PgError("No data passed the filtering variables.")
-        ld.kin.gram()
-        n_eigenvecs = ld.kin.eig_select(P, float(xxt_eigen_variance_explained))
-        scan = ld.kin.covar_scan if method == "ols" else ld.kin.mle_scan
-        beta, _var, pval = scan(self.phen_matrix)   # [k, P] in file order
+        flush()
+        t0 = clock()
+        n_eigenvecs = kin.eig_select(P, float(xxt_eigen_variance_explained))
+        tm["eig_s"] = clock() - t0
+        scan = kin.covar_scan if method == "ols" else kin.mle_scan
+        if len(dev_blocks) == 1:
+            t0 = clock()
+            beta, _var, pval = scan(self.phen_matrix)   # [k, P] in file order
+            tm["scan_s"] = clock() - t0
+        else:
+            beta, pval = np.empty((k, P)), np.empty((k, P))
+            offsets = np.cumsum([0] + [sum(c for _, _, c in tb) for tb in dev_blocks])
+            order = [len(dev_blocks) - 1] + list(range(len(dev_blocks) - 1))  # the last block is still resident
+            with open(self.filename_sync, "rb") as fh:
+                for d in order:
+                    if d != order[0]:
+                        t0 = clock()
+                        kin.reset()
+                        for at, nbytes, cols in dev_blocks[d]:
+                            fh.seek(at)
+                            block = fh.read(nbytes)
+                            got = kin.append_sync_text(block, filter_stats, max_loci, keep_p_minus_1)[3].size
+                            if len(block) != nbytes or got != cols:
+                                raise PgError(f"{self.filename_sync} changed between passes: the {nbytes} bytes at "
+                                              f"offset {at} gave {got} columns, {cols} before")
+                        tm["pass2_load_s"] += clock() - t0
+                    t0 = clock()
+                    b, _var, pv = scan(self.phen_matrix)
+                    tm["scan_s"] += clock() - t0
+                    beta[:, offsets[d]:offsets[d + 1]] = b
+                    pval[:, offsets[d]:offsets[d + 1]] = pv
     finally:
-        ld.kin.close()
+        kin.close()
+    t0 = clock()
     # the matrix columns follow the loci sorted by (chromosome, position): permute the records into that order
     order = capi.sort_loci(ld.positions, chr_names=ld.chr_names, chr_index=ld.chr_index)
     first = np.full(int(ld.positions.size) + 1, -1, dtype=np.int64)
@@ -412,28 +564,34 @@ def _iter_with_kinship(self, ctx: Context, filter_stats: FilterStats, keep_p_min
     with open(out, "xb") as fo:
         fo.write(capi.format_header(capi.KIND_OLS_KINSHIP))
         fo.write(rows)
+    if timings is not None:
+        tm["write_s"] = clock() - t0
+        tm["device_blocks"] = len(dev_blocks)
+        tm["columns"] = P
+        tm["capacity"] = cap
+        timings.update(tm)
     return out
 
 
 def ols_iter_with_kinship(self, ctx: Context, filter_stats: FilterStats, keep_p_minus_1: bool,
                           xxt_eigen_variance_explained: float, out: str, n_threads: int,
-                          block_bytes: int = 32 << 20) -> str:
+                          block_bytes: int = 32 << 20, device_bytes: int = None) -> str:
     """`poolgen ols_iter_with_kinship` (src/main.rs:280-298): into_genotypes_and_phenotypes (src/base/sync.rs:1106-1179)
     then ols_with_covariate (src/gwas/ols.rs:278-436) and its writer, including the label indexing of
     src/gwas/ols.rs:421-424 (row i of the allele columns carries entry i of the label vectors, whose entry 0 is the
     intercept's)"""
     return _iter_with_kinship(self, ctx, filter_stats, keep_p_minus_1, xxt_eigen_variance_explained, out, n_threads,
-                              block_bytes, "ols")
+                              block_bytes, "ols", device_bytes)
 
 
 def mle_iter_with_kinship(self, ctx: Context, filter_stats: FilterStats, keep_p_minus_1: bool,
                           xxt_eigen_variance_explained: float, out: str, n_threads: int,
-                          block_bytes: int = 32 << 20) -> str:
+                          block_bytes: int = 32 << 20, device_bytes: int = None) -> str:
     """`poolgen mle_iter_with_kinship` (src/main.rs:316-326): the same loader, then mle_with_covariate
     (src/gwas/mle.rs:307-463) -- kinship matrix, PCs by the same rule, one maximum-likelihood fit per column and
     phenotype -- and its writer (same header and row layout, labels indexed the same way, mle.rs:449-460)"""
     return _iter_with_kinship(self, ctx, filter_stats, keep_p_minus_1, xxt_eigen_variance_explained, out, n_threads,
-                              block_bytes, "mle")
+                              block_bytes, "mle", device_bytes)
 
 
 FileSyncPhen.write_csv = write_csv
