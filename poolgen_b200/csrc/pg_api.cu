@@ -34,25 +34,28 @@ cudaError_t launch_scan(const ScanParams &p, int sm_count, cudaStream_t s) {
 // file chunk), and the thread that made the failing call is the one that asks for the message.
 static thread_local std::string g_last_err;
 
-void pg::set_error(pg_ctx *, const char *msg) { g_last_err = msg; }
-
-static int fail(pg_ctx *ctx, int code, const char *fmt, ...) {
+int pg::fail(pg_ctx *, int code, const char *fmt, ...) {
     char buf[512];
     va_list ap;
     va_start(ap, fmt);
     vsnprintf(buf, sizeof buf, fmt, ap);
     va_end(ap);
-    pg::set_error(ctx, buf);
+    g_last_err = buf;
     return code;
 }
 
-#define PG_CUDA(ctx, call)                                                                          \
-    do {                                                                                            \
-        cudaError_t e_ = (call);                                                                    \
-        if (e_ != cudaSuccess)                                                                      \
-            return fail((ctx), PG_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), \
-                        __FILE__, __LINE__);                                                        \
-    } while (0)
+using pg::fail;
+
+pg_scan::~pg_scan() {
+    for (pg_batch *b : slabs) delete b;
+}
+
+pg_batch::~pg_batch() {
+    if (stream) cudaStreamSynchronize(stream);
+    if (ev0) cudaEventDestroy(ev0);
+    if (ev1) cudaEventDestroy(ev1);
+    if (stream) cudaStreamDestroy(stream);
+}
 
 extern "C" {
 
@@ -259,9 +262,9 @@ int pg_scan_open(pg_ctx *ctx, int kind, const pg_filter *filter, int n_pools, in
         if (s->df > 0.0 && !(pv_mode && strcmp(pv_mode, "cf") == 0)) {
             pg::PTable tab = pg::build_ptable(s->df);
             if (tab.max_err < 2e-9) {  // otherwise keep the continued fraction
-                cudaError_t et = cudaMalloc(&s->d_ptab, tab.coef.size() * 8);
+                cudaError_t et = s->d_ptab.reserve(tab.coef.size(), nullptr);
                 if (et == cudaSuccess)
-                    et = cudaMemcpy(s->d_ptab, tab.coef.data(), tab.coef.size() * 8, cudaMemcpyHostToDevice);
+                    et = cudaMemcpy(s->d_ptab.get(), tab.coef.data(), tab.coef.size() * 8, cudaMemcpyHostToDevice);
                 if (et != cudaSuccess) {
                     delete s;
                     return fail(ctx, PG_ERR_CUDA, "pg_scan_open: p-value table upload: %s", cudaGetErrorString(et));
@@ -272,18 +275,17 @@ int pg_scan_open(pg_ctx *ctx, int kind, const pg_filter *filter, int n_pools, in
                 s->ptab_err = tab.max_err;
             }
         }
-        cudaError_t e = cudaMalloc(&s->d_yc, s->yc_host.size() * 8);
-        if (e == cudaSuccess) e = cudaMemcpy(s->d_yc, s->yc_host.data(), s->yc_host.size() * 8, cudaMemcpyHostToDevice);
+        cudaError_t e = s->d_yc.reserve(s->yc_host.size(), nullptr);
+        if (e == cudaSuccess) e = cudaMemcpy(s->d_yc.get(), s->yc_host.data(), s->yc_host.size() * 8, cudaMemcpyHostToDevice);
         if (e != cudaSuccess) {
             delete s;
             return fail(ctx, PG_ERR_CUDA, "pg_scan_open: phenotype upload: %s", cudaGetErrorString(e));
         }
     }
     {
-        cudaError_t e = cudaMalloc(&s->d_w, s->w_host.size() * 8);
-        if (e == cudaSuccess) e = cudaMemcpy(s->d_w, s->w_host.data(), s->w_host.size() * 8, cudaMemcpyHostToDevice);
+        cudaError_t e = s->d_w.reserve(s->w_host.size(), nullptr);
+        if (e == cudaSuccess) e = cudaMemcpy(s->d_w.get(), s->w_host.data(), s->w_host.size() * 8, cudaMemcpyHostToDevice);
         if (e != cudaSuccess) {
-            if (s->d_yc) cudaFree(s->d_yc);
             delete s;
             return fail(ctx, PG_ERR_CUDA, "pg_scan_open: weight upload: %s", cudaGetErrorString(e));
         }
@@ -305,10 +307,10 @@ int pg_scan_open(pg_ctx *ctx, int kind, const pg_filter *filter, int n_pools, in
             for (int j = 0; j < k; j++)
                 for (int i = 0; i < n_pools; i++) raw[(size_t)j * np + i] = phen[(size_t)i * k + j];
         }
-        cudaError_t e = cudaMalloc(&s->d_yraw, raw.size() * 8);
-        if (e == cudaSuccess) e = cudaMemcpy(s->d_yraw, raw.data(), raw.size() * 8, cudaMemcpyHostToDevice);
+        cudaError_t e = s->d_yraw.reserve(raw.size(), nullptr);
+        if (e == cudaSuccess) e = cudaMemcpy(s->d_yraw.get(), raw.data(), raw.size() * 8, cudaMemcpyHostToDevice);
         if (e != cudaSuccess) {
-            pg_scan_close(s);
+            delete s;
             return fail(ctx, PG_ERR_CUDA, "pg_scan_open: phenotype upload: %s", cudaGetErrorString(e));
         }
     }
@@ -317,7 +319,7 @@ int pg_scan_open(pg_ctx *ctx, int kind, const pg_filter *filter, int n_pools, in
     {
         cudaError_t e = cudaDeviceSynchronize();
         if (e != cudaSuccess) {
-            pg_scan_close(s);
+            delete s;
             return fail(ctx, PG_ERR_CUDA, "pg_scan_open: %s", cudaGetErrorString(e));
         }
     }
@@ -326,13 +328,6 @@ int pg_scan_open(pg_ctx *ctx, int kind, const pg_filter *filter, int n_pools, in
 }
 
 int pg_scan_close(pg_scan *s) {
-    if (!s) return PG_OK;
-    for (int i = 0; i < PG_STREAM_DEPTH; i++)
-        if (s->slabs[i]) pg_batch_destroy(s->slabs[i]);
-    if (s->d_yc) cudaFree(s->d_yc);
-    if (s->d_w) cudaFree(s->d_w);
-    if (s->d_ptab) cudaFree(s->d_ptab);
-    if (s->d_yraw) cudaFree(s->d_yraw);
     delete s;
     return PG_OK;
 }
@@ -354,18 +349,18 @@ int pg_batch_create(pg_scan *s, int64_t cap, pg_batch **out) {
     if (e == cudaSuccess) e = cudaEventCreate(&b->ev0);
     if (e == cudaSuccess) e = cudaEventCreate(&b->ev1);
     if (e == cudaSuccess && is_regression(s)) {
-        e = cudaMalloc(&b->d_freq, (size_t)cap * s->lay.freq_stride() * 8);
-        if (e == cudaSuccess) e = cudaMalloc(&b->d_depth, (size_t)cap * s->lay.depth_stride() * 4);
-        if (e == cudaSuccess) e = cudaMalloc(&b->d_dmin, (size_t)cap * 4);
-        if (e == cudaSuccess) e = cudaMalloc(&b->d_defer, (size_t)(cap + 1) * 8);
-        if (e == cudaSuccess) e = cudaMalloc(&b->d_hint, (size_t)cap);
+        e = b->d_freq.reserve((size_t)cap * s->lay.freq_stride(), b->stream);
+        if (e == cudaSuccess) e = b->d_depth.reserve((size_t)cap * s->lay.depth_stride(), b->stream);
+        if (e == cudaSuccess) e = b->d_dmin.reserve((size_t)cap, b->stream);
+        if (e == cudaSuccess) e = b->d_defer.reserve((size_t)cap + 1, b->stream);
+        if (e == cudaSuccess) e = b->d_hint.reserve((size_t)cap, b->stream);
     }
     const size_t S = s->n_slots, K = s->k;
-    if (e == cudaSuccess) e = cudaMalloc(&b->d_meta, (size_t)cap * 8);
-    if (e == cudaSuccess) e = cudaMalloc(&b->d_fmean, (size_t)cap * S * 8);
-    if (e == cudaSuccess) e = cudaMalloc(&b->d_stats, (size_t)cap * S * K * 32);
+    if (e == cudaSuccess) e = b->d_meta.reserve((size_t)cap, b->stream);
+    if (e == cudaSuccess) e = b->d_fmean.reserve((size_t)cap * S, b->stream);
+    if (e == cudaSuccess) e = b->d_stats.reserve((size_t)cap * S * K * 4, b->stream);
     if (e != cudaSuccess) {
-        pg_batch_destroy(b);
+        delete b;
         return fail(ctx, PG_ERR_CUDA, "pg_batch_create(%lld loci): %s", (long long)cap, cudaGetErrorString(e));
     }
     *out = b;
@@ -373,24 +368,6 @@ int pg_batch_create(pg_scan *s, int64_t cap, pg_batch **out) {
 }
 
 int pg_batch_destroy(pg_batch *b) {
-    if (!b) return PG_OK;
-    if (b->stream) cudaStreamSynchronize(b->stream);
-    cudaFree(b->d_freq);
-    cudaFree(b->d_depth);
-    cudaFree(b->d_dmin);
-    cudaFree(b->d_defer);
-    cudaFree(b->d_hint);
-    pg::text_scratch_free(b->text);
-    cudaFree(b->d_stage);
-    cudaFree(b->d_meta);
-    cudaFree(b->d_fmean);
-    cudaFree(b->d_stats);
-    if (b->h_meta) cudaFreeHost(b->h_meta);
-    if (b->h_fmean) cudaFreeHost(b->h_fmean);
-    if (b->h_stats) cudaFreeHost(b->h_stats);
-    if (b->ev0) cudaEventDestroy(b->ev0);
-    if (b->ev1) cudaEventDestroy(b->ev1);
-    if (b->stream) cudaStreamDestroy(b->stream);
     delete b;
     return PG_OK;
 }
@@ -398,32 +375,24 @@ int pg_batch_destroy(pg_batch *b) {
 static pg::IngestOut ingest_out(pg_batch *b, int64_t first_locus) {
     pg_scan *s = b->scan;
     pg::IngestOut o;
-    o.freq = b->d_freq + (size_t)first_locus * s->lay.freq_stride();
-    o.depth = b->d_depth + (size_t)first_locus * s->lay.depth_stride();
-    o.dmin = b->d_dmin + first_locus;
-    o.hint = b->d_hint + first_locus;
-    o.w = s->d_w;
+    o.freq = b->d_freq.get() + (size_t)first_locus * s->lay.freq_stride();
+    o.depth = b->d_depth.get() + (size_t)first_locus * s->lay.depth_stride();
+    o.dmin = b->d_dmin.get() + first_locus;
+    o.hint = b->d_hint.get() + first_locus;
+    o.w = s->d_w.get();
     o.maf = s->maf;
     o.one_minus_maf = 1.00 - s->maf;
     o.min_depth_f = (double)s->min_depth;
     return o;
 }
 
+}  // extern "C"
+
+// the staging area of the uploads: at least `bytes` bytes
 static int ensure_stage(pg_batch *b, size_t bytes) {
-    pg_ctx *ctx = b->scan->ctx;
-    if (b->stage_bytes >= bytes) return PG_OK;
-    if (b->d_stage) {
-        PG_CUDA(ctx, cudaStreamSynchronize(b->stream));
-        PG_CUDA(ctx, cudaFree(b->d_stage));
-        b->d_stage = nullptr;
-        b->stage_bytes = 0;
-    }
-    PG_CUDA(ctx, cudaMalloc(&b->d_stage, bytes));
-    b->stage_bytes = bytes;
+    PG_CUDA(b->scan->ctx, b->d_stage.reserve(bytes, b->stream));
     return PG_OK;
 }
-
-}  // extern "C"
 
 template <typename CT>
 static int upload_counts_t(pg_batch *b, const CT *counts, int64_t n_loci) {
@@ -442,22 +411,22 @@ static int upload_counts_t(pg_batch *b, const CT *counts, int64_t n_loci) {
     int rc = ensure_stage(b, reg ? (size_t)b->cap * s->A_in * s->n * sizeof(CT) : wide_bytes + (sizeof(CT) == 4 ? 0 : bytes));
     if (rc) return rc;
     if (reg) {
-        PG_CUDA(ctx, cudaMemcpyAsync(b->d_stage, counts, bytes, cudaMemcpyHostToDevice, b->stream));
+        PG_CUDA(ctx, cudaMemcpyAsync(b->d_stage.get(), counts, bytes, cudaMemcpyHostToDevice, b->stream));
         if constexpr (sizeof(CT) == 4)
-            PG_CUDA(ctx, pg::launch_ingest_u32((const uint32_t *)b->d_stage, n_loci, s->n, s->A_in, s->drop_col, s->lay,
+            PG_CUDA(ctx, pg::launch_ingest_u32((const uint32_t *)b->d_stage.get(), n_loci, s->n, s->A_in, s->drop_col, s->lay,
                                                ingest_out(b, 0), b->stream));
         else if constexpr (sizeof(CT) == 1)
-            PG_CUDA(ctx, pg::launch_ingest_u8((const uint8_t *)b->d_stage, n_loci, s->n, s->A_in, s->drop_col, s->lay,
+            PG_CUDA(ctx, pg::launch_ingest_u8((const uint8_t *)b->d_stage.get(), n_loci, s->n, s->A_in, s->drop_col, s->lay,
                                               ingest_out(b, 0), b->stream));
         else
-            PG_CUDA(ctx, pg::launch_ingest_u16((const uint16_t *)b->d_stage, n_loci, s->n, s->A_in, s->drop_col, s->lay,
+            PG_CUDA(ctx, pg::launch_ingest_u16((const uint16_t *)b->d_stage.get(), n_loci, s->n, s->A_in, s->drop_col, s->lay,
                                                ingest_out(b, 0), b->stream));
     } else if constexpr (sizeof(CT) == 4) {
-        PG_CUDA(ctx, cudaMemcpyAsync(b->d_stage, counts, bytes, cudaMemcpyHostToDevice, b->stream));
+        PG_CUDA(ctx, cudaMemcpyAsync(b->d_stage.get(), counts, bytes, cudaMemcpyHostToDevice, b->stream));
     } else {
-        void *narrow = (char *)b->d_stage + wide_bytes;
+        void *narrow = (char *)b->d_stage.get() + wide_bytes;
         PG_CUDA(ctx, cudaMemcpyAsync(narrow, counts, bytes, cudaMemcpyHostToDevice, b->stream));
-        PG_CUDA(ctx, pg::launch_widen(narrow, (int)sizeof(CT), (uint32_t *)b->d_stage, (size_t)n_loci * s->A_in * s->n,
+        PG_CUDA(ctx, pg::launch_widen(narrow, (int)sizeof(CT), (uint32_t *)b->d_stage.get(), (size_t)n_loci * s->A_in * s->n,
                                       b->stream));
     }
     b->input_is_counts = 1;
@@ -491,8 +460,8 @@ int pg_batch_upload_freq(pg_batch *b, const double *freq, const uint32_t *depth,
     const size_t fbytes_cap = (size_t)b->cap * s->A_dev * s->n * 8, dbytes_cap = (size_t)b->cap * s->n * 4;
     int rc = ensure_stage(b, fbytes_cap + dbytes_cap);
     if (rc) return rc;
-    double *sf = (double *)b->d_stage;
-    uint32_t *sd = (uint32_t *)((char *)b->d_stage + fbytes_cap);
+    double *sf = (double *)b->d_stage.get();
+    uint32_t *sd = (uint32_t *)((char *)b->d_stage.get() + fbytes_cap);
     PG_CUDA(ctx, cudaMemcpyAsync(sf, freq, (size_t)n_loci * s->A_dev * s->n * 8, cudaMemcpyHostToDevice, b->stream));
     PG_CUDA(ctx, cudaMemcpyAsync(sd, depth, (size_t)n_loci * s->n * 4, cudaMemcpyHostToDevice, b->stream));
     PG_CUDA(ctx, pg::launch_ingest_freq(sf, sd, n_loci, s->n, s->lay, ingest_out(b, 0), b->stream));
@@ -516,7 +485,7 @@ static int text_stage_a(pg_batch *b, const char *text, size_t n_bytes, size_t li
     b->text_bytes = n_bytes;
     int rc = ensure_stage(b, (size_t)b->cap * 6 * s->n * 4);
     if (rc) return rc;
-    const cudaError_t pe = pg::text_parse_async(&b->text, text, n_bytes, s->n, (uint32_t *)b->d_stage, b->cap, line_cap,
+    const cudaError_t pe = pg::text_parse_async(&b->text, text, n_bytes, s->n, (uint32_t *)b->d_stage.get(), b->cap, line_cap,
                                                 ctx->sm_count, b->stream);
     if (pe != cudaSuccess) {
         b->have_input = 0;  // nothing usable is resident: a later run / collect must not scan the previous chunk
@@ -533,21 +502,17 @@ static int text_stage_b(pg_batch *b, int64_t *n_loci_out) {
     if (n_loci_out) *n_loci_out = 0;
     cudaError_t ce = cudaSuccess;
     uint64_t at = 0;
-    int64_t L = pg::text_parse_finish(b->text, b->stream, &ce, &at);
+    int64_t L = pg::text_parse_finish(&b->text, b->stream, &ce, &at);
     if (L == -5) {  // more (comment / blank) lines than the default bound: repeat with the exact number
         int rc = text_stage_a(b, b->text_src, b->text_bytes, (size_t)at + 1);
         if (rc) return rc;
-        L = pg::text_parse_finish(b->text, b->stream, &ce, &at);
+        L = pg::text_parse_finish(&b->text, b->stream, &ce, &at);
     }
-    if (L == -1) return fail(ctx, PG_ERR_CUDA, "upload_sync_text: %s", cudaGetErrorString(ce));
-    if (L == -2) return fail(ctx, PG_ERR_ARG, "upload_sync_text: more loci in the chunk than the batch capacity %lld", (long long)b->cap);
-    if (L == -3) return fail(ctx, PG_ERR_ARG, "upload_sync_text: the line at byte %llu does not hold %d pools (the reference asserts the pool count, src/base/sync.rs:254-257)", (unsigned long long)at, s->n);
-    if (L == -4) return fail(ctx, PG_ERR_ARG, "upload_sync_text: malformed pool field at byte %llu (the reference panics: allele counts are not valid integers, src/base/sync.rs:146)", (unsigned long long)at);
-    if (L < 0) return fail(ctx, PG_ERR_ARG, "upload_sync_text: the chunk could not be parsed (%lld)", (long long)L);
+    if (L < 0) return pg::text_parse_fail(ctx, "upload_sync_text", L, ce, at, s->n, b->cap);
     b->n_loci = L;
     if (n_loci_out) *n_loci_out = L;
     if (L > 0 && is_regression(s))
-        PG_CUDA(ctx, pg::launch_ingest_u32((const uint32_t *)b->d_stage, L, s->n, s->A_in, s->drop_col, s->lay,
+        PG_CUDA(ctx, pg::launch_ingest_u32((const uint32_t *)b->d_stage.get(), L, s->n, s->A_in, s->drop_col, s->lay,
                                            ingest_out(b, 0), b->stream));
     return PG_OK;
 }
@@ -564,9 +529,9 @@ int pg_batch_upload_sync_text(pg_batch *b, const char *text, size_t n_bytes, int
 
 int pg_batch_text_labels(pg_batch *b, const uint64_t **line_offsets, const uint64_t **positions) {
     if (!b) return PG_ERR_ARG;
-    if (!b->text) return fail(b->scan->ctx, PG_ERR_STATE, "pg_batch_text_labels before pg_batch_upload_sync_text");
-    if (line_offsets) *line_offsets = pg::text_offsets(b->text);
-    if (positions) *positions = pg::text_positions(b->text);
+    if (!b->text.parsed) return fail(b->scan->ctx, PG_ERR_STATE, "pg_batch_text_labels before pg_batch_upload_sync_text");
+    if (line_offsets) *line_offsets = b->text.h_out_offset.get();
+    if (positions) *positions = b->text.h_out_pos.get();
     return PG_OK;
 }
 
@@ -583,7 +548,7 @@ int pg_batch_synth(pg_batch *b, uint64_t seed, int64_t first_locus, int64_t n_lo
     if (!is_regression(s)) {
         int rc = ensure_stage(b, (size_t)b->cap * per_locus);
         if (rc) return rc;
-        PG_CUDA(ctx, pg::launch_synth(seed, first_locus, n_loci, s->n, s->A_in, (uint32_t *)b->d_stage, b->stream));
+        PG_CUDA(ctx, pg::launch_synth(seed, first_locus, n_loci, s->n, s->A_in, (uint32_t *)b->d_stage.get(), b->stream));
         b->input_is_counts = 1;
         return PG_OK;
     }
@@ -591,17 +556,17 @@ int pg_batch_synth(pg_batch *b, uint64_t seed, int64_t first_locus, int64_t n_lo
     int64_t slice = (int64_t)((size_t)256 << 20) / (int64_t)per_locus;
     if (slice < 1) slice = 1;
     if (slice > n_loci) slice = n_loci;
-    if (b->stage_bytes < (size_t)slice * per_locus) {
+    if (b->d_stage.capacity() < (size_t)slice * per_locus) {
         int rc = ensure_stage(b, (size_t)slice * per_locus);
         if (rc) return rc;
     } else {
-        slice = (int64_t)(b->stage_bytes / per_locus);
+        slice = (int64_t)(b->d_stage.capacity() / per_locus);
         if (slice > n_loci) slice = n_loci;
     }
     for (int64_t l0 = 0; l0 < n_loci; l0 += slice) {
         const int64_t m = (n_loci - l0 < slice) ? n_loci - l0 : slice;
-        PG_CUDA(ctx, pg::launch_synth(seed, first_locus + l0, m, s->n, s->A_in, (uint32_t *)b->d_stage, b->stream));
-        PG_CUDA(ctx, pg::launch_ingest_u32((const uint32_t *)b->d_stage, m, s->n, s->A_in, s->drop_col, s->lay,
+        PG_CUDA(ctx, pg::launch_synth(seed, first_locus + l0, m, s->n, s->A_in, (uint32_t *)b->d_stage.get(), b->stream));
+        PG_CUDA(ctx, pg::launch_ingest_u32((const uint32_t *)b->d_stage.get(), m, s->n, s->A_in, s->drop_col, s->lay,
                                            ingest_out(b, l0), b->stream));
     }
     b->input_is_counts = 1;
@@ -630,10 +595,10 @@ static int run_once(pg_batch *b, int *launches) {
             pg::ScanParams p;
             memset(&p, 0, sizeof p);
             p.lay = s->lay;
-            p.freq = b->d_freq;
-            p.depth = b->d_depth;
-            p.dmin = b->d_dmin;
-            p.hint = b->d_hint;
+            p.freq = b->d_freq.get();
+            p.depth = b->d_depth.get();
+            p.dmin = b->d_dmin.get();
+            p.hint = b->d_hint.get();
             p.n_loci = b->n_loci;
             p.kind = is_nm(s) ? PG_KIND_OLS : s->kind;
             p.filter_only = is_nm(s) ? 1 : 0;
@@ -648,25 +613,25 @@ static int run_once(pg_batch *b, int *launches) {
             p.inv_n = 1.0 / (double)s->n;
             p.inv_nm2 = 1.0 / ((double)s->n - 2.0);
             p.ln_beta = s->ln_beta;
-            p.ptab = s->d_ptab;
+            p.ptab = s->d_ptab.get();
             p.ptab_isd = s->ptab_isd;
             p.ptab_bits = s->ptab_bits;
             p.ptab_M = s->ptab_M;
             p.K = std::min(kpass, s->k - base);
             p.y_has_nan = s->y_has_nan;
-            p.yc = s->d_yc + (size_t)base * s->lay.n_pad;
-            p.w = s->d_w;
+            p.yc = s->d_yc.get() + (size_t)base * s->lay.n_pad;
+            p.w = s->d_w.get();
             for (int j = 0; j < p.K; j++) {
                 p.ysum[j] = s->ysum[base + j];
                 p.syy[j] = s->syy[base + j];
                 p.ymean[j] = s->ymean[base + j];
             }
             for (int j = 0; j < s->A_dev; j++) p.codes[j] = s->codes_dev[j];
-            p.meta = b->d_meta;
-            p.freq_mean = b->d_fmean;
-            p.stats = b->d_stats;
-            p.defer_list = b->d_defer;
-            p.defer_count = reinterpret_cast<uint32_t *>(b->d_defer + b->cap);
+            p.meta = b->d_meta.get();
+            p.freq_mean = b->d_fmean.get();
+            p.stats = b->d_stats.get();
+            p.defer_list = b->d_defer.get();
+            p.defer_count = reinterpret_cast<uint32_t *>(b->d_defer.get() + b->cap);
             p.k_total = s->k;
             p.phen_base = base;
             p.write_meta = base == 0;
@@ -681,31 +646,31 @@ static int run_once(pg_batch *b, int *launches) {
             pg::NmParams q;
             memset(&q, 0, sizeof q);
             q.lay = s->lay;
-            q.freq = b->d_freq;
-            q.depth = b->d_depth;
+            q.freq = b->d_freq.get();
+            q.depth = b->d_depth.get();
             q.n_loci = b->n_loci;
             q.kind = s->kind;
             q.k = s->k;
-            q.yraw = s->d_yraw;
+            q.yraw = s->d_yraw.get();
             q.gw_sig = s->gw_sig;
             q.gw_min = s->gw_min;
             q.gw_max = s->gw_max;
             q.df = s->df;
             q.ln_beta = s->ln_beta;
-            q.ptab = s->d_ptab;
+            q.ptab = s->d_ptab.get();
             q.ptab_isd = s->ptab_isd;
             q.ptab_bits = s->ptab_bits;
             q.ptab_M = s->ptab_M;
             for (int j = 0; j < s->A_dev; j++) q.codes[j] = s->codes_dev[j];
-            q.meta = b->d_meta;
-            q.stats = b->d_stats;
+            q.meta = b->d_meta.get();
+            q.stats = b->d_stats.get();
             PG_CUDA(ctx, pg::launch_nm(q, ctx->sm_count, b->stream));
             if (launches) (*launches)++;
         }
     } else {
         pg::TableParams p;
         memset(&p, 0, sizeof p);
-        p.counts = (const uint32_t *)b->d_stage;
+        p.counts = (const uint32_t *)b->d_stage.get();
         p.n_loci = b->n_loci;
         p.n = s->n;
         p.A_in = s->A_in;
@@ -715,10 +680,10 @@ static int run_once(pg_batch *b, int *launches) {
         p.one_minus_maf = 1.00 - s->maf;
         p.max_miss = s->max_miss;
         p.min_depth_f = (double)s->min_depth;
-        p.w = s->d_w;
+        p.w = s->d_w.get();
         for (int j = 0; j < s->A_in; j++) p.codes[j] = s->codes_in[j];
-        p.meta = b->d_meta;
-        p.stats = b->d_stats;
+        p.meta = b->d_meta.get();
+        p.stats = b->d_stats.get();
         PG_CUDA(ctx, pg::launch_tables(p, ctx->sm_count, b->stream));
         if (launches) (*launches)++;
     }
@@ -747,11 +712,11 @@ int pg_batch_time_runs(pg_batch *b, int iters, float *ms_total, int *n_launches)
     PG_CUDA(ctx, cudaEventElapsedTime(ms_total, b->ev0, b->ev1));
     if (n_launches) *n_launches = launches;
     static const bool report = getenv("PG_REPORT_DEFER") != nullptr;  // diagnostic: why loci went to the fix-up kernel
-    if (report && b->d_defer && is_regression(b->scan)) {
+    if (report && b->d_defer.get() && is_regression(b->scan)) {
         uint32_t count = 0;
-        PG_CUDA(ctx, cudaMemcpy(&count, b->d_defer + b->cap, 4, cudaMemcpyDeviceToHost));
+        PG_CUDA(ctx, cudaMemcpy(&count, b->d_defer.get() + b->cap, 4, cudaMemcpyDeviceToHost));
         std::vector<uint64_t> list(count);
-        if (count) PG_CUDA(ctx, cudaMemcpy(list.data(), b->d_defer, (size_t)count * 8, cudaMemcpyDeviceToHost));
+        if (count) PG_CUDA(ctx, cudaMemcpy(list.data(), b->d_defer.get(), (size_t)count * 8, cudaMemcpyDeviceToHost));
         uint32_t h[8] = {0, 0, 0, 0, 0, 0, 0, 0};
         for (uint64_t e : list) {
             const unsigned why = (unsigned)(e >> 56);
@@ -785,16 +750,14 @@ int pg_batch_download(pg_batch *b) {
     pg_ctx *ctx = s->ctx;
     PG_CUDA(ctx, cudaSetDevice(ctx->device));
     const size_t S = s->n_slots, K = s->k;
-    if (!b->h_meta) {
-        PG_CUDA(ctx, cudaHostAlloc((void **)&b->h_meta, (size_t)b->cap * 8, cudaHostAllocDefault));
-        PG_CUDA(ctx, cudaHostAlloc((void **)&b->h_fmean, (size_t)b->cap * S * 8, cudaHostAllocDefault));
-        PG_CUDA(ctx, cudaHostAlloc((void **)&b->h_stats, (size_t)b->cap * S * K * 32, cudaHostAllocDefault));
-    }
+    PG_CUDA(ctx, b->h_meta.reserve((size_t)b->cap, b->stream));
+    PG_CUDA(ctx, b->h_fmean.reserve((size_t)b->cap * S, b->stream));
+    PG_CUDA(ctx, b->h_stats.reserve((size_t)b->cap * S * K * 4, b->stream));
     const size_t L = (size_t)b->n_loci;
     if (L == 0) return PG_OK;
-    PG_CUDA(ctx, cudaMemcpyAsync(b->h_meta, b->d_meta, L * 8, cudaMemcpyDeviceToHost, b->stream));
-    PG_CUDA(ctx, cudaMemcpyAsync(b->h_fmean, b->d_fmean, L * S * 8, cudaMemcpyDeviceToHost, b->stream));
-    PG_CUDA(ctx, cudaMemcpyAsync(b->h_stats, b->d_stats, L * S * K * 32, cudaMemcpyDeviceToHost, b->stream));
+    PG_CUDA(ctx, cudaMemcpyAsync(b->h_meta.get(), b->d_meta.get(), L * 8, cudaMemcpyDeviceToHost, b->stream));
+    PG_CUDA(ctx, cudaMemcpyAsync(b->h_fmean.get(), b->d_fmean.get(), L * S * 8, cudaMemcpyDeviceToHost, b->stream));
+    PG_CUDA(ctx, cudaMemcpyAsync(b->h_stats.get(), b->d_stats.get(), L * S * K * 32, cudaMemcpyDeviceToHost, b->stream));
     return PG_OK;
 }
 
@@ -806,13 +769,13 @@ int pg_batch_sync(pg_batch *b) {
 
 int pg_batch_results(pg_batch *b, pg_results *out) {
     if (!b || !out) return PG_ERR_ARG;
-    if (!b->h_meta && b->n_loci > 0) return fail(b->scan->ctx, PG_ERR_STATE, "pg_batch_results before pg_batch_download");
+    if (b->n_loci > 0 && !(b->h_meta.get() && b->h_fmean.get() && b->h_stats.get())) return fail(b->scan->ctx, PG_ERR_STATE, "pg_batch_results before pg_batch_download");
     out->n_loci = b->n_loci;
     out->n_slots = b->scan->n_slots;
     out->n_phen = b->scan->k;
-    out->meta = b->h_meta;
-    out->freq_mean = b->h_fmean;
-    out->stats = b->h_stats;
+    out->meta = b->h_meta.get();
+    out->freq_mean = b->h_fmean.get();
+    out->stats = b->h_stats.get();
     return PG_OK;
 }
 
@@ -820,10 +783,8 @@ int pg_batch_results(pg_batch *b, pg_results *out) {
 int pg_scan_stream_begin(pg_scan *s, int64_t max_loci) {
     if (!s || max_loci < 1) return PG_ERR_ARG;
     for (int i = 0; i < PG_STREAM_DEPTH; i++) {
-        if (s->slabs[i]) {
-            pg_batch_destroy(s->slabs[i]);
-            s->slabs[i] = nullptr;
-        }
+        delete s->slabs[i];
+        s->slabs[i] = nullptr;
         int rc = pg_batch_create(s, max_loci, &s->slabs[i]);
         if (rc) return rc;
     }
@@ -876,7 +837,7 @@ int pg_scan_submit_freq(pg_scan *s, const double *freq, const uint32_t *depth, i
 // a slab submitted as text whose parse has been enqueued but whose scan has not: finish it (stage B, scan, download)
 static int finish_text_slab(pg_scan *s, int slab, int64_t *n_loci) {
     pg_batch *b = s->slabs[slab];
-    if (!b || !pg::text_parse_pending(b->text)) return PG_OK;
+    if (!b || !b->text.pending) return PG_OK;
     int rc = text_stage_b(b, n_loci);
     if (rc) return rc;
     if ((rc = pg_batch_run(b))) return rc;

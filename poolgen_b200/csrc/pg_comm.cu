@@ -13,7 +13,6 @@
 // process that already holds a libnccl.so.2 (e.g. one that imported torch) shares that copy.
 #include <dlfcn.h>
 #include <nccl.h>
-#include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -74,18 +73,9 @@ const NcclApi &nccl_api() {
     }();
     return api;
 }
-
-int cfail(pg_ctx *ctx, int code, const char *fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    pg::set_error(ctx, buf);
-    return code;
-}
-
 }  // namespace
+
+using pg::fail;
 
 static_assert(sizeof(ncclUniqueId) == PG_COMM_ID_BYTES, "PG_COMM_ID_BYTES must equal sizeof(ncclUniqueId)");
 
@@ -95,30 +85,37 @@ struct pg_comm {
     int first_rank = 0;  // rank of local index 0 (local ranks are consecutive)
     std::vector<ncclComm_t> comms;
     std::vector<pg_ctx *> ctxs;
-    std::vector<int64_t *> d_count;  // one device int64 per local rank (column counts summed with the matrices)
-    std::vector<int64_t *> h_count;  // pinned
+    // one int64 per local rank on its device and pinned on the host: the column counts summed with the matrices
+    std::vector<pg::DeviceBuffer<int64_t>> d_count;
+    std::vector<pg::PinnedBuffer<int64_t>> h_count;
+    ~pg_comm();
 };
+
+// each local rank's counter is freed, and its communicator destroyed, with that rank's device current
+pg_comm::~pg_comm() {
+    const NcclApi &nccl = nccl_api();
+    for (int i = 0; i < n_local; i++) {
+        if (i < (int)ctxs.size() && ctxs[i]) cudaSetDevice(ctxs[i]->device);
+        if (i < (int)d_count.size()) d_count[i] = {};
+        if (i < (int)h_count.size()) h_count[i] = {};
+        if (nccl.ok && i < (int)comms.size() && comms[i]) nccl.comm_destroy(comms[i]);
+    }
+}
 
 #define CNCCL(ctx, call)                                                                                     \
     do {                                                                                                     \
         ncclResult_t r_ = (call);                                                                            \
         if (r_ != ncclSuccess)                                                                               \
-            return cfail((ctx), PG_ERR_NCCL, "%s failed: %s (%s:%d)", #call, nccl.error_string(r_), __FILE__, __LINE__); \
-    } while (0)
-#define CCUDA(ctx, call)                                                                                     \
-    do {                                                                                                     \
-        cudaError_t e_ = (call);                                                                             \
-        if (e_ != cudaSuccess)                                                                               \
-            return cfail((ctx), PG_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
+            return fail((ctx), PG_ERR_NCCL, "%s failed: %s (%s:%d)", #call, nccl.error_string(r_), __FILE__, __LINE__); \
     } while (0)
 
 static int comm_alloc_counters(pg_comm *c) {
-    c->d_count.assign(c->n_local, nullptr);
-    c->h_count.assign(c->n_local, nullptr);
+    c->d_count.resize(c->n_local);
+    c->h_count.resize(c->n_local);
     for (int i = 0; i < c->n_local; i++) {
-        CCUDA(c->ctxs[i], cudaSetDevice(c->ctxs[i]->device));
-        CCUDA(c->ctxs[i], cudaMalloc(&c->d_count[i], 8));
-        CCUDA(c->ctxs[i], cudaHostAlloc((void **)&c->h_count[i], 8, cudaHostAllocDefault));
+        PG_CUDA(c->ctxs[i], cudaSetDevice(c->ctxs[i]->device));
+        PG_CUDA(c->ctxs[i], c->d_count[i].reserve(1, nullptr));
+        PG_CUDA(c->ctxs[i], c->h_count[i].reserve(1, nullptr));
     }
     return PG_OK;
 }
@@ -127,7 +124,7 @@ extern "C" {
 
 int pg_shard_range(int64_t total, int rank, int world, int64_t *begin, int64_t *end) {
     if (world < 1 || rank < 0 || rank >= world || total < 0 || !begin || !end)
-        return cfail(nullptr, PG_ERR_ARG, "pg_shard_range(total=%lld, rank=%d, world=%d)", (long long)total, rank, world);
+        return fail(nullptr, PG_ERR_ARG, "pg_shard_range(total=%lld, rank=%d, world=%d)", (long long)total, rank, world);
     const int64_t base = total / world, rem = total % world;
     *begin = rank * base + (rank < rem ? rank : rem);
     *end = *begin + base + (rank < rem ? 1 : 0);
@@ -137,20 +134,20 @@ int pg_shard_range(int64_t total, int rank, int world, int64_t *begin, int64_t *
 int pg_nccl_version(int *version) {
     const NcclApi &nccl = nccl_api();
     if (!version) return PG_ERR_ARG;
-    if (!nccl.ok) return cfail(nullptr, PG_ERR_NCCL, "pg_nccl_version: %s", nccl.why);
+    if (!nccl.ok) return fail(nullptr, PG_ERR_NCCL, "pg_nccl_version: %s", nccl.why);
     CNCCL(nullptr, nccl.get_version(version));
     return PG_OK;
 }
 
 int pg_init_multi(const int *devices, int n, pg_ctx **ctxs_out, pg_comm **comm_out) {
-    if (!devices || n < 1 || !ctxs_out || !comm_out) return cfail(nullptr, PG_ERR_ARG, "pg_init_multi: bad argument");
+    if (!devices || n < 1 || !ctxs_out || !comm_out) return fail(nullptr, PG_ERR_ARG, "pg_init_multi: bad argument");
     *comm_out = nullptr;
     for (int i = 0; i < n; i++) ctxs_out[i] = nullptr;
     for (int i = 0; i < n; i++)
         for (int j = 0; j < i; j++)
-            if (devices[i] == devices[j]) return cfail(nullptr, PG_ERR_ARG, "pg_init_multi: device %d listed twice", devices[i]);
+            if (devices[i] == devices[j]) return fail(nullptr, PG_ERR_ARG, "pg_init_multi: device %d listed twice", devices[i]);
     const NcclApi &nccl = nccl_api();
-    if (!nccl.ok) return cfail(nullptr, PG_ERR_NCCL, "pg_init_multi: %s", nccl.why);
+    if (!nccl.ok) return fail(nullptr, PG_ERR_NCCL, "pg_init_multi: %s", nccl.why);
     auto undo = [&] {
         for (int i = 0; i < n; i++) {
             pg_destroy(ctxs_out[i]);
@@ -167,7 +164,7 @@ int pg_init_multi(const int *devices, int n, pg_ctx **ctxs_out, pg_comm **comm_o
     pg_comm *c = new (std::nothrow) pg_comm();
     if (!c) {
         undo();
-        return cfail(nullptr, PG_ERR_ARG, "out of host memory");
+        return fail(nullptr, PG_ERR_ARG, "out of host memory");
     }
     c->world = n;
     c->n_local = n;
@@ -178,11 +175,11 @@ int pg_init_multi(const int *devices, int n, pg_ctx **ctxs_out, pg_comm **comm_o
     if (r != ncclSuccess) {
         delete c;
         undo();
-        return cfail(nullptr, PG_ERR_NCCL, "ncclCommInitAll(%d devices) failed: %s", n, nccl.error_string(r));
+        return fail(nullptr, PG_ERR_NCCL, "ncclCommInitAll(%d devices) failed: %s", n, nccl.error_string(r));
     }
     int rc = comm_alloc_counters(c);
     if (rc) {
-        pg_comm_destroy(c);
+        delete c;
         undo();
         return rc;
     }
@@ -193,7 +190,7 @@ int pg_init_multi(const int *devices, int n, pg_ctx **ctxs_out, pg_comm **comm_o
 int pg_comm_unique_id(uint8_t *id) {
     if (!id) return PG_ERR_ARG;
     const NcclApi &nccl = nccl_api();
-    if (!nccl.ok) return cfail(nullptr, PG_ERR_NCCL, "pg_comm_unique_id: %s", nccl.why);
+    if (!nccl.ok) return fail(nullptr, PG_ERR_NCCL, "pg_comm_unique_id: %s", nccl.why);
     ncclUniqueId u;
     CNCCL(nullptr, nccl.get_unique_id(&u));
     memcpy(id, &u, sizeof u);
@@ -202,13 +199,13 @@ int pg_comm_unique_id(uint8_t *id) {
 
 int pg_comm_init_rank(pg_ctx *ctx, const uint8_t *id, int rank, int world, pg_comm **out) {
     if (!ctx || !id || !out || world < 1 || rank < 0 || rank >= world)
-        return cfail(ctx, PG_ERR_ARG, "pg_comm_init_rank: bad argument (rank %d of %d)", rank, world);
+        return fail(ctx, PG_ERR_ARG, "pg_comm_init_rank: bad argument (rank %d of %d)", rank, world);
     *out = nullptr;
     const NcclApi &nccl = nccl_api();
-    if (!nccl.ok) return cfail(ctx, PG_ERR_NCCL, "pg_comm_init_rank: %s", nccl.why);
-    CCUDA(ctx, cudaSetDevice(ctx->device));
+    if (!nccl.ok) return fail(ctx, PG_ERR_NCCL, "pg_comm_init_rank: %s", nccl.why);
+    PG_CUDA(ctx, cudaSetDevice(ctx->device));
     pg_comm *c = new (std::nothrow) pg_comm();
-    if (!c) return cfail(ctx, PG_ERR_ARG, "out of host memory");
+    if (!c) return fail(ctx, PG_ERR_ARG, "out of host memory");
     c->world = world;
     c->n_local = 1;
     c->first_rank = rank;
@@ -219,11 +216,11 @@ int pg_comm_init_rank(pg_ctx *ctx, const uint8_t *id, int rank, int world, pg_co
     ncclResult_t r = nccl.comm_init_rank(&c->comms[0], world, u, rank);
     if (r != ncclSuccess) {
         delete c;
-        return cfail(ctx, PG_ERR_NCCL, "ncclCommInitRank(rank %d of %d) failed: %s", rank, world, nccl.error_string(r));
+        return fail(ctx, PG_ERR_NCCL, "ncclCommInitRank(rank %d of %d) failed: %s", rank, world, nccl.error_string(r));
     }
     int rc = comm_alloc_counters(c);
     if (rc) {
-        pg_comm_destroy(c);
+        delete c;
         return rc;
     }
     *out = c;
@@ -239,14 +236,6 @@ int pg_comm_info(const pg_comm *c, int *world, int *n_local, int *first_rank) {
 }
 
 int pg_comm_destroy(pg_comm *c) {
-    if (!c) return PG_OK;
-    const NcclApi &nccl = nccl_api();
-    for (int i = 0; i < c->n_local; i++) {
-        if (i < (int)c->ctxs.size() && c->ctxs[i]) cudaSetDevice(c->ctxs[i]->device);
-        if (i < (int)c->d_count.size()) cudaFree(c->d_count[i]);
-        if (i < (int)c->h_count.size() && c->h_count[i]) cudaFreeHost(c->h_count[i]);
-        if (nccl.ok && i < (int)c->comms.size() && c->comms[i]) nccl.comm_destroy(c->comms[i]);
-    }
     delete c;
     return PG_OK;
 }
@@ -254,48 +243,49 @@ int pg_comm_destroy(pg_comm *c) {
 // K_total = sum over the ranks of the partial Gram matrices, in place on every rank's device buffer; the column counts
 // are summed in the same group.  kins[i] belongs to local rank i of the communicator (its context's device).
 int pg_kin_allreduce(pg_comm *c, pg_kin *const *kins, int n_local, int64_t *P_total, float *ms) {
-    if (!c || !kins || n_local != c->n_local) return cfail(nullptr, PG_ERR_ARG, "pg_kin_allreduce: %d handles for %d local ranks", n_local, c ? c->n_local : -1);
+    if (!c || !kins || n_local != c->n_local) return fail(nullptr, PG_ERR_ARG, "pg_kin_allreduce: %d handles for %d local ranks", n_local, c ? c->n_local : -1);
     const NcclApi &nccl = nccl_api();
-    if (!nccl.ok) return cfail(nullptr, PG_ERR_NCCL, "pg_kin_allreduce: %s", nccl.why);
+    if (!nccl.ok) return fail(nullptr, PG_ERR_NCCL, "pg_kin_allreduce: %s", nccl.why);
     for (int i = 0; i < n_local; i++) {
-        if (!kins[i]) return cfail(nullptr, PG_ERR_ARG, "pg_kin_allreduce: handle %d is NULL", i);
+        if (!kins[i]) return fail(nullptr, PG_ERR_ARG, "pg_kin_allreduce: handle %d is NULL", i);
         if (kins[i]->ctx->device != c->ctxs[i]->device)
-            return cfail(kins[i]->ctx, PG_ERR_ARG, "pg_kin_allreduce: handle %d lives on device %d, local rank %d on device %d", i,
+            return fail(kins[i]->ctx, PG_ERR_ARG, "pg_kin_allreduce: handle %d lives on device %d, local rank %d on device %d", i,
                          kins[i]->ctx->device, i, c->ctxs[i]->device);
-        if (kins[i]->n != kins[0]->n) return cfail(kins[i]->ctx, PG_ERR_ARG, "pg_kin_allreduce: pool counts differ");
+        if (kins[i]->n != kins[0]->n) return fail(kins[i]->ctx, PG_ERR_ARG, "pg_kin_allreduce: pool counts differ");
     }
     const size_t elems = (size_t)kins[0]->n * kins[0]->n;
     for (int i = 0; i < n_local; i++) {
         pg_kin *h = kins[i];
-        CCUDA(h->ctx, cudaSetDevice(h->ctx->device));
-        *c->h_count[i] = h->P;
-        CCUDA(h->ctx, cudaMemcpyAsync(c->d_count[i], c->h_count[i], 8, cudaMemcpyHostToDevice, h->stream));
-        if (ms && i == 0) CCUDA(h->ctx, cudaEventRecord(h->ev0, h->stream));
+        PG_CUDA(h->ctx, cudaSetDevice(h->ctx->device));
+        *c->h_count[i].get() = h->P;
+        PG_CUDA(h->ctx, cudaMemcpyAsync(c->d_count[i].get(), c->h_count[i].get(), 8, cudaMemcpyHostToDevice, h->stream));
+        if (ms && i == 0) PG_CUDA(h->ctx, cudaEventRecord(h->ev0, h->stream));
     }
     CNCCL(kins[0]->ctx, nccl.group_start());
     for (int i = 0; i < n_local; i++) {
         pg_kin *h = kins[i];
-        ncclResult_t r = nccl.all_reduce(h->d_K, h->d_K, elems, ncclDouble, ncclSum, c->comms[i], h->stream);
-        if (r == ncclSuccess) r = nccl.all_reduce(c->d_count[i], c->d_count[i], 1, ncclInt64, ncclSum, c->comms[i], h->stream);
+        ncclResult_t r = nccl.all_reduce(h->d_K.get(), h->d_K.get(), elems, ncclDouble, ncclSum, c->comms[i], h->stream);
+        if (r == ncclSuccess)
+            r = nccl.all_reduce(c->d_count[i].get(), c->d_count[i].get(), 1, ncclInt64, ncclSum, c->comms[i], h->stream);
         if (r != ncclSuccess) {
             nccl.group_end();
-            return cfail(h->ctx, PG_ERR_NCCL, "ncclAllReduce (local rank %d) failed: %s", i, nccl.error_string(r));
+            return fail(h->ctx, PG_ERR_NCCL, "ncclAllReduce (local rank %d) failed: %s", i, nccl.error_string(r));
         }
     }
     CNCCL(kins[0]->ctx, nccl.group_end());
     for (int i = 0; i < n_local; i++) {
         pg_kin *h = kins[i];
-        CCUDA(h->ctx, cudaSetDevice(h->ctx->device));
-        if (ms && i == 0) CCUDA(h->ctx, cudaEventRecord(h->ev1, h->stream));
-        CCUDA(h->ctx, cudaMemcpyAsync(c->h_count[i], c->d_count[i], 8, cudaMemcpyDeviceToHost, h->stream));
+        PG_CUDA(h->ctx, cudaSetDevice(h->ctx->device));
+        if (ms && i == 0) PG_CUDA(h->ctx, cudaEventRecord(h->ev1, h->stream));
+        PG_CUDA(h->ctx, cudaMemcpyAsync(c->h_count[i].get(), c->d_count[i].get(), 8, cudaMemcpyDeviceToHost, h->stream));
     }
     for (int i = 0; i < n_local; i++) {
         pg_kin *h = kins[i];
-        CCUDA(h->ctx, cudaSetDevice(h->ctx->device));
-        CCUDA(h->ctx, cudaStreamSynchronize(h->stream));
-        h->P_total = *c->h_count[i];
+        PG_CUDA(h->ctx, cudaSetDevice(h->ctx->device));
+        PG_CUDA(h->ctx, cudaStreamSynchronize(h->stream));
+        h->P_total = *c->h_count[i].get();
     }
-    if (ms) CCUDA(kins[0]->ctx, cudaEventElapsedTime(ms, kins[0]->ev0, kins[0]->ev1));
+    if (ms) PG_CUDA(kins[0]->ctx, cudaEventElapsedTime(ms, kins[0]->ev0, kins[0]->ev1));
     if (P_total) *P_total = kins[0]->P_total;
     return PG_OK;
 }

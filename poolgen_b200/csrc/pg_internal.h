@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "poolgen_cuda.h"
@@ -179,22 +180,89 @@ cudaError_t launch_synth(uint64_t seed, int64_t first_locus, int64_t n_loci, int
 // u8 / u16 counts -> u32 (the count tests read u32)
 cudaError_t launch_widen(const void *src, int elem_bytes, uint32_t *dst, size_t count, cudaStream_t s);
 
+// ---- host-side ownership ---------------------------------------------------------------------
+// One allocation of device memory (Pinned = false) or pinned host memory (Pinned = true), freed by the destructor.
+// The handles below own every buffer through this type.  A handle's destructor synchronises its stream before the
+// buffers (members) are freed, so no queued work still reads or writes one; its events and stream are destroyed after
+// that synchronisation.
+template <typename T, bool Pinned>
+class Buffer {
+  public:
+    Buffer() = default;
+    Buffer(const Buffer &) = delete;
+    Buffer &operator=(const Buffer &) = delete;
+    Buffer(Buffer &&o) noexcept : p_(o.p_), cap_(o.cap_) { o.p_ = nullptr, o.cap_ = 0; }
+    Buffer &operator=(Buffer &&o) noexcept {
+        std::swap(p_, o.p_);
+        std::swap(cap_, o.cap_);
+        return *this;
+    }
+    ~Buffer() { release(); }
+
+    // Nothing when `count` elements fit.  Otherwise waits for `stream` (queued work may still use the old allocation),
+    // frees it and allocates exactly `count` elements.  After a failed reserve the buffer is empty: get() is null and
+    // capacity() is 0, so the next reserve allocates again.
+    cudaError_t reserve(size_t count, cudaStream_t stream) {
+        if (cap_ >= count) return cudaSuccess;
+        cudaError_t e = p_ ? cudaStreamSynchronize(stream) : cudaSuccess;
+        release();
+        if (e != cudaSuccess) return e;
+        void *q = nullptr;
+        if constexpr (Pinned)
+            e = cudaHostAlloc(&q, count * sizeof(T), cudaHostAllocDefault);
+        else
+            e = cudaMalloc(&q, count * sizeof(T));
+        if (e != cudaSuccess) {
+            (void)cudaGetLastError();  // the error is returned here: a later launch check must not report it again
+            return e;
+        }
+        p_ = static_cast<T *>(q);
+        cap_ = count;
+        return cudaSuccess;
+    }
+    T *get() const { return p_; }
+    size_t capacity() const { return cap_; }
+
+  private:
+    void release() {
+        if constexpr (Pinned) {
+            if (p_) cudaFreeHost(p_);
+        } else {
+            cudaFree(p_);
+        }
+        p_ = nullptr;
+        cap_ = 0;
+    }
+    T *p_ = nullptr;
+    size_t cap_ = 0;
+};
+template <typename T>
+using DeviceBuffer = Buffer<T, false>;
+template <typename T>
+using PinnedBuffer = Buffer<T, true>;
+
 // sync text -> counts[locus][6][n_pools] on the device (pg_text.cu)
-struct TextScratch;
-cudaError_t text_parse_async(TextScratch **scratch, const char *text, size_t n_bytes, int n_pools, uint32_t *d_counts,
+struct TextScratch {
+    DeviceBuffer<char> d_text;
+    DeviceBuffer<uint32_t> d_sep;
+    DeviceBuffer<uint64_t> d_tok_blk;
+    DeviceBuffer<uint32_t> d_nl, d_first, d_grp;
+    DeviceBuffer<uint8_t> d_keep;
+    DeviceBuffer<uint64_t> d_line_pos;
+    DeviceBuffer<uint32_t> d_info;  // [4]: n_loci, error code, error offset, n_lines
+    PinnedBuffer<uint32_t> h_info;  // its copy
+    DeviceBuffer<uint8_t> d_tmp;
+    DeviceBuffer<uint64_t> d_out_offset, d_out_pos;
+    PinnedBuffer<uint64_t> h_out_offset, h_out_pos;  // the labels of the parsed loci: line offsets, positions
+    cudaEvent_t parsed = nullptr;  // created by the first text_parse_async
+    bool pending = false;          // text_parse_async issued, text_parse_finish not yet called
+    int64_t max_loci = 0;
+    ~TextScratch();  // the owner has synchronised the stream the parse ran on
+};
+cudaError_t text_parse_async(TextScratch *t, const char *text, size_t n_bytes, int n_pools, uint32_t *d_counts,
                              int64_t max_loci, size_t line_cap, int sm_count, cudaStream_t s);
 int64_t text_parse_finish(TextScratch *t, cudaStream_t s, cudaError_t *cuda_err, uint64_t *err_offset);
-bool text_parse_pending(const TextScratch *t);
-void text_scratch_free(TextScratch *t);
-const uint64_t *text_offsets(const TextScratch *t);
-const uint64_t *text_positions(const TextScratch *t);
 
-}  // namespace pg
-
-struct pg_ctx;
-namespace pg {
-// records the message pg_last_error() returns to the calling thread (pg_api.cu)
-void set_error(pg_ctx *ctx, const char *msg);
 }  // namespace pg
 
 // opaque ABI types
@@ -204,6 +272,23 @@ struct pg_ctx {
     int cc_major = 0, cc_minor = 0;
     size_t total_mem = 0;
 };
+
+namespace pg {
+// sets the message pg_last_error() returns to the calling thread (printf format) and returns `code` (pg_api.cu)
+int fail(pg_ctx *ctx, int code, const char *fmt, ...);
+// the return code and message of a negative text_parse_finish result: `who` names the caller, `cap` is the number of
+// loci the chunk may hold (pg_text.cu)
+int text_parse_fail(pg_ctx *ctx, const char *who, int64_t status, cudaError_t cuda_err, uint64_t err_offset,
+                    int n_pools, int64_t cap);
+}  // namespace pg
+
+#define PG_CUDA(ctx, call)                                                                              \
+    do {                                                                                                \
+        cudaError_t e_ = (call);                                                                        \
+        if (e_ != cudaSuccess)                                                                          \
+            return pg::fail((ctx), PG_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), \
+                            __FILE__, __LINE__);                                                        \
+    } while (0)
 
 struct pg_scan {
     pg_ctx *ctx = nullptr;
@@ -225,11 +310,11 @@ struct pg_scan {
     std::vector<double> ysum, syy, ymean;
     int y_has_nan = 0;
     double df = 0, ln_beta = 0;
-    double *d_yc = nullptr;
-    double *d_w = nullptr;
-    double *d_yraw = nullptr;   // mle_iter: raw phenotypes [k][n_pad]; gwalpha: bins [n_pad], q [n_pad]
+    pg::DeviceBuffer<double> d_yc;
+    pg::DeviceBuffer<double> d_w;
+    pg::DeviceBuffer<double> d_yraw;  // mle_iter: raw phenotypes [k][n_pad]; gwalpha: bins [n_pad], q [n_pad]
     double gw_sig = 0, gw_min = 0, gw_max = 0;  // gwalpha_fmt: sig, MIN, MAX
-    double *d_ptab = nullptr;
+    pg::DeviceBuffer<double> d_ptab;
     double ptab_isd = 0, ptab_bits = 0, ptab_err = 0;
     int ptab_M = 0;
     int n_slots = 0;
@@ -237,6 +322,7 @@ struct pg_scan {
     pg_batch *slabs[PG_STREAM_DEPTH] = {nullptr, nullptr, nullptr};
     int next_slab = 0;
     int64_t slab_cap = 0;
+    ~pg_scan();  // destroys the slabs
 };
 
 struct pg_batch {
@@ -245,23 +331,24 @@ struct pg_batch {
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     // device
-    double *d_freq = nullptr;
-    uint32_t *d_depth = nullptr;
-    uint32_t *d_dmin = nullptr;
-    uint64_t *d_defer = nullptr;  // [cap + 1]: list then its counter
-    uint8_t *d_hint = nullptr;    // [cap]
-    void *d_stage = nullptr;  // raw uploaded slab (counts u32/u16 or unpadded freq+depth)
-    size_t stage_bytes = 0;
-    uint64_t *d_meta = nullptr;
-    double *d_fmean = nullptr;
-    double *d_stats = nullptr;
+    pg::DeviceBuffer<double> d_freq;
+    pg::DeviceBuffer<uint32_t> d_depth;
+    pg::DeviceBuffer<uint32_t> d_dmin;
+    pg::DeviceBuffer<uint64_t> d_defer;  // [cap + 1]: list then its counter
+    pg::DeviceBuffer<uint8_t> d_hint;    // [cap]
+    pg::DeviceBuffer<uint8_t> d_stage;   // raw uploaded slab (counts u32/u16 or unpadded freq+depth)
+    pg::DeviceBuffer<uint64_t> d_meta;
+    pg::DeviceBuffer<double> d_fmean;
+    pg::DeviceBuffer<double> d_stats;
     // pinned host results
-    uint64_t *h_meta = nullptr;
-    double *h_fmean = nullptr;
-    double *h_stats = nullptr;
+    pg::PinnedBuffer<uint64_t> h_meta;
+    pg::PinnedBuffer<double> h_fmean;
+    pg::PinnedBuffer<double> h_stats;
     int have_input = 0;
     int input_is_counts = 0;
-    pg::TextScratch *text = nullptr;
+    pg::TextScratch text;
     const char *text_src = nullptr;  // the caller's chunk of the last text upload (valid until its slab is collected)
     size_t text_bytes = 0;
+    ~pg_batch();
 };
+

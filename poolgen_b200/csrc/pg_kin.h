@@ -15,10 +15,9 @@ struct pg_kin {
     int64_t P_total = 0;      // columns over all shards (pg_kin_allreduce); 0 = this handle holds them all
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    double *d_G = nullptr;
-    double *d_K = nullptr;    // [n][n] partial Gram matrix (sum over the resident columns)
-    double *d_ws = nullptr;   // split-K workspace
-    size_t ws_bytes = 0;
+    pg::DeviceBuffer<double> d_G;
+    pg::DeviceBuffer<double> d_K;   // [n][n] partial Gram matrix (sum over the resident columns)
+    pg::DeviceBuffer<double> d_ws;  // split-K workspace
     int nt = 0, n_slices = 0;
     // covariates
     int m = -1;
@@ -26,37 +25,29 @@ struct pg_kin {
     std::vector<double> eigvals;  // descending
     std::vector<double> Q;        // [1+m][ldg] orthonormal basis of [1 | PCs] (host)
     std::vector<double> C;        // [m][ldg] the covariates themselves (pg_kin_mle_scan: the simplex search is not basis-invariant)
-    double *d_mle = nullptr;      // pg_kin_mle_scan: centred covariates and phenotypes, then the fixed moments
-    size_t mle_bytes = 0;
-    double *d_V = nullptr;        // [(1+m) + k][ldg]
-    size_t V_bytes = 0;
-    double *d_ptab = nullptr;
+    pg::DeviceBuffer<double> d_mle;  // pg_kin_mle_scan: centred covariates and phenotypes, then the fixed moments
+    pg::DeviceBuffer<double> d_V;    // [(1+m) + k][ldg]
+    pg::DeviceBuffer<double> d_ptab;
     double ptab_isd = 0, ptab_bits = 0;
     int ptab_M = 0;
     // results
     int k = 0;
-    double *d_res = nullptr;  // [3][k][P]
-    double *h_res = nullptr;  // pinned
-    size_t res_elems = 0;
-    void *d_defer = nullptr;  // covariate scan: [count | columns left to the two-pass kernel]
-    size_t defer_bytes = 0;
-    double *d_part = nullptr;  // covariate scan (DMMA form in pool passes): partial sums per column block
-    size_t part_bytes = 0;
+    pg::DeviceBuffer<double> d_res;  // [3][k][P]
+    pg::PinnedBuffer<double> h_res;
+    pg::DeviceBuffer<int64_t> d_defer;  // covariate scan: [count | columns left to the two-pass kernel]
+    pg::DeviceBuffer<double> d_part;    // covariate scan (DMMA form in pool passes): partial sums per column block
     // loader scratch
-    uint32_t *d_sel = nullptr;
-    int64_t *d_off = nullptr;
-    int64_t *d_col_locus = nullptr;
-    uint8_t *d_col_allele = nullptr;
-    void *d_scan_tmp = nullptr;
-    size_t scan_tmp_bytes = 0;
-    int64_t load_cap = 0;
-    void *d_counts = nullptr;
-    size_t counts_bytes = 0;
-    double *d_w = nullptr;
-    pg::TextScratch *text = nullptr;  // sync text parsed on the device (pg_kin_append_sync_text)
+    pg::DeviceBuffer<uint32_t> d_sel;
+    pg::DeviceBuffer<int64_t> d_off;
+    pg::DeviceBuffer<int64_t> d_col_locus;
+    pg::DeviceBuffer<uint8_t> d_col_allele;
+    pg::DeviceBuffer<uint8_t> d_scan_tmp;
+    pg::DeviceBuffer<uint32_t> d_counts;
+    pg::DeviceBuffer<double> d_w;
+    pg::TextScratch text;  // sync text parsed on the device (pg_kin_append_sync_text)
     // eigen step: cuSOLVER is mapped and its handle created by a background thread started in pg_kin_open and joined
-    // by pg_kin_eig_select / pg_kin_close
+    // by pg_kin_eig_select / the destructor
     std::thread warm;
     void *solver = nullptr;  // cusolverDnHandle_t
+    ~pg_kin();
 };
-

@@ -15,7 +15,6 @@
 #include <cusolverDn.h>
 #include <dlfcn.h>
 #include <math.h>
-#include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -950,22 +949,7 @@ const CusolverApi &cusolver_api() {
 }
 }  // namespace
 
-
-static int kfail(pg_ctx *ctx, int code, const char *fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    pg::set_error(ctx, buf);
-    return code;
-}
-#define KCUDA(ctx, call)                                                                                  \
-    do {                                                                                                  \
-        cudaError_t e_ = (call);                                                                          \
-        if (e_ != cudaSuccess)                                                                            \
-            return kfail((ctx), PG_ERR_CUDA, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
-    } while (0)
+using pg::fail;
 
 static int64_t round_up(int64_t v, int64_t m) { return (v + m - 1) / m * m; }
 
@@ -985,12 +969,22 @@ static void kin_warm_solver(pg_kin *h) {
     if (sol.create(&cs) == CUSOLVER_STATUS_SUCCESS) h->solver = cs;
 }
 
+// the warm-up thread is joined, and the cuSOLVER handle bound to the stream destroyed, before anything else
+pg_kin::~pg_kin() {
+    if (warm.joinable()) warm.join();
+    if (solver) cusolver_api().destroy(static_cast<cusolverDnHandle_t>(solver));
+    if (stream) cudaStreamSynchronize(stream);
+    if (ev0) cudaEventDestroy(ev0);
+    if (ev1) cudaEventDestroy(ev1);
+    if (stream) cudaStreamDestroy(stream);
+}
+
 int pg_kin_open(pg_ctx *ctx, int n_pools, int64_t max_columns, pg_kin **out) {
-    if (!ctx || !out || n_pools < 2 || max_columns < 1) return kfail(ctx, PG_ERR_ARG, "pg_kin_open: bad argument");
+    if (!ctx || !out || n_pools < 2 || max_columns < 1) return fail(ctx, PG_ERR_ARG, "pg_kin_open: bad argument");
     *out = nullptr;
-    KCUDA(ctx, cudaSetDevice(ctx->device));
+    PG_CUDA(ctx, cudaSetDevice(ctx->device));
     pg_kin *h = new (std::nothrow) pg_kin();
-    if (!h) return kfail(ctx, PG_ERR_ARG, "out of host memory");
+    if (!h) return fail(ctx, PG_ERR_ARG, "out of host memory");
     h->ctx = ctx;
     h->n = n_pools;
     h->ldg = (n_pools + 3) & ~3;
@@ -1000,14 +994,14 @@ int pg_kin_open(pg_ctx *ctx, int n_pools, int64_t max_columns, pg_kin **out) {
     if (e == cudaSuccess) e = cudaEventCreate(&h->ev0);
     if (e == cudaSuccess) e = cudaEventCreate(&h->ev1);
     // + one tile of slack: the last tile of a row reads past ldg into the next column
-    const size_t g_bytes = ((size_t)h->cap * h->ldg + pg::kTile) * 8;
-    if (e == cudaSuccess) e = cudaMalloc(&h->d_G, g_bytes);
-    if (e == cudaSuccess) e = cudaMemsetAsync(h->d_G, 0, g_bytes, h->stream);
-    if (e == cudaSuccess) e = cudaMalloc(&h->d_K, (size_t)n_pools * n_pools * 8);
-    if (e == cudaSuccess) e = cudaMemsetAsync(h->d_K, 0, (size_t)n_pools * n_pools * 8, h->stream);
+    const size_t g_elems = (size_t)h->cap * h->ldg + pg::kTile;
+    if (e == cudaSuccess) e = h->d_G.reserve(g_elems, h->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(h->d_G.get(), 0, g_elems * 8, h->stream);
+    if (e == cudaSuccess) e = h->d_K.reserve((size_t)n_pools * n_pools, h->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(h->d_K.get(), 0, (size_t)n_pools * n_pools * 8, h->stream);
     if (e != cudaSuccess) {
-        pg_kin_close(h);
-        return kfail(ctx, PG_ERR_CUDA, "pg_kin_open(%d pools, %lld columns): %s", n_pools, (long long)max_columns,
+        delete h;
+        return fail(ctx, PG_ERR_CUDA, "pg_kin_open(%d pools, %lld columns): %s", n_pools, (long long)max_columns,
                      cudaGetErrorString(e));
     }
     h->warm = std::thread(kin_warm_solver, h);
@@ -1016,39 +1010,14 @@ int pg_kin_open(pg_ctx *ctx, int n_pools, int64_t max_columns, pg_kin **out) {
 }
 
 int pg_kin_close(pg_kin *h) {
-    if (!h) return PG_OK;
-    if (h->warm.joinable()) h->warm.join();
-    if (h->solver) cusolver_api().destroy(static_cast<cusolverDnHandle_t>(h->solver));
-    if (h->stream) cudaStreamSynchronize(h->stream);
-    cudaFree(h->d_G);
-    cudaFree(h->d_K);
-    cudaFree(h->d_ws);
-    cudaFree(h->d_V);
-    cudaFree(h->d_ptab);
-    cudaFree(h->d_res);
-    cudaFree(h->d_defer);
-    cudaFree(h->d_mle);
-    cudaFree(h->d_part);
-    if (h->h_res) cudaFreeHost(h->h_res);
-    cudaFree(h->d_sel);
-    cudaFree(h->d_off);
-    cudaFree(h->d_col_locus);
-    cudaFree(h->d_col_allele);
-    cudaFree(h->d_scan_tmp);
-    cudaFree(h->d_counts);
-    cudaFree(h->d_w);
-    pg::text_scratch_free(h->text);
-    if (h->ev0) cudaEventDestroy(h->ev0);
-    if (h->ev1) cudaEventDestroy(h->ev1);
-    if (h->stream) cudaStreamDestroy(h->stream);
     delete h;
     return PG_OK;
 }
 
 int pg_kin_reset(pg_kin *h) {
     if (!h) return PG_ERR_ARG;
-    KCUDA(h->ctx, cudaSetDevice(h->ctx->device));
-    KCUDA(h->ctx, cudaMemsetAsync(h->d_G, 0, ((size_t)h->cap * h->ldg + pg::kTile) * 8, h->stream));
+    PG_CUDA(h->ctx, cudaSetDevice(h->ctx->device));
+    PG_CUDA(h->ctx, cudaMemsetAsync(h->d_G.get(), 0, h->d_G.capacity() * 8, h->stream));
     h->P = 0;
     h->P_total = 0;
     return PG_OK;
@@ -1059,11 +1028,11 @@ int64_t pg_kin_columns(pg_kin *h) { return h ? h->P : -1; }
 int pg_kin_append_columns(pg_kin *h, const double *cols, int64_t P_add) {
     if (!h || (!cols && P_add > 0) || P_add < 0) return PG_ERR_ARG;
     pg_ctx *ctx = h->ctx;
-    if (h->P + P_add > h->cap) return kfail(ctx, PG_ERR_ARG, "pg_kin_append_columns: %lld + %lld columns > capacity %lld",
+    if (h->P + P_add > h->cap) return fail(ctx, PG_ERR_ARG, "pg_kin_append_columns: %lld + %lld columns > capacity %lld",
                                             (long long)h->P, (long long)P_add, (long long)h->cap);
-    KCUDA(ctx, cudaSetDevice(ctx->device));
+    PG_CUDA(ctx, cudaSetDevice(ctx->device));
     if (P_add == 0) return PG_OK;
-    KCUDA(ctx, cudaMemcpy2DAsync(h->d_G + (size_t)h->P * h->ldg, (size_t)h->ldg * 8, cols, (size_t)h->n * 8,
+    PG_CUDA(ctx, cudaMemcpy2DAsync(h->d_G.get() + (size_t)h->P * h->ldg, (size_t)h->ldg * 8, cols, (size_t)h->n * 8,
                                  (size_t)h->n * 8, (size_t)P_add, cudaMemcpyHostToDevice, h->stream));
     h->P += P_add;
     return PG_OK;
@@ -1072,32 +1041,14 @@ int pg_kin_append_columns(pg_kin *h, const double *cols, int64_t P_add) {
 // loader scratch for n_loci loci of n_alleles stored columns
 static int kin_reserve(pg_kin *h, int64_t n_loci, int n_alleles) {
     pg_ctx *ctx = h->ctx;
-    if (h->load_cap < n_loci) {
-        KCUDA(ctx, cudaStreamSynchronize(h->stream));
-        cudaFree(h->d_sel);
-        cudaFree(h->d_off);
-        cudaFree(h->d_col_locus);
-        cudaFree(h->d_col_allele);
-        cudaFree(h->d_scan_tmp);
-        h->d_sel = nullptr, h->d_off = nullptr, h->d_col_locus = nullptr, h->d_col_allele = nullptr, h->d_scan_tmp = nullptr;
-        KCUDA(ctx, cudaMalloc(&h->d_sel, (size_t)n_loci * 4));
-        KCUDA(ctx, cudaMalloc(&h->d_off, (size_t)(n_loci + 1) * 8));
-        KCUDA(ctx, cudaMalloc(&h->d_col_locus, (size_t)n_loci * PG_MAX_ALLELES * 8));
-        KCUDA(ctx, cudaMalloc(&h->d_col_allele, (size_t)n_loci * PG_MAX_ALLELES));
-        size_t tmp = 0;
-        cub::DeviceScan::ExclusiveSum(nullptr, tmp, h->d_off, h->d_off, (int)(n_loci + 1), h->stream);
-        KCUDA(ctx, cudaMalloc(&h->d_scan_tmp, tmp));
-        h->scan_tmp_bytes = tmp;
-        h->load_cap = n_loci;
-    }
-    const size_t cbytes = (size_t)n_loci * n_alleles * h->n * 4;
-    if (h->counts_bytes < cbytes) {
-        KCUDA(ctx, cudaStreamSynchronize(h->stream));
-        cudaFree(h->d_counts);
-        h->d_counts = nullptr;
-        KCUDA(ctx, cudaMalloc(&h->d_counts, cbytes));
-        h->counts_bytes = cbytes;
-    }
+    PG_CUDA(ctx, h->d_sel.reserve((size_t)n_loci, h->stream));
+    PG_CUDA(ctx, h->d_off.reserve((size_t)n_loci + 1, h->stream));
+    PG_CUDA(ctx, h->d_col_locus.reserve((size_t)n_loci * PG_MAX_ALLELES, h->stream));
+    PG_CUDA(ctx, h->d_col_allele.reserve((size_t)n_loci * PG_MAX_ALLELES, h->stream));
+    size_t tmp = 0;
+    cub::DeviceScan::ExclusiveSum(nullptr, tmp, h->d_off.get(), h->d_off.get(), (int)(n_loci + 1), h->stream);
+    PG_CUDA(ctx, h->d_scan_tmp.reserve(tmp, h->stream));
+    PG_CUDA(ctx, h->d_counts.reserve((size_t)n_loci * n_alleles * h->n, h->stream));
     return PG_OK;
 }
 
@@ -1105,18 +1056,18 @@ static int kin_reserve(pg_kin *h, int64_t n_loci, int n_alleles) {
 static int kin_load_resident(pg_kin *h, const pg_filter *filter, int n_alleles, const uint8_t *codes, int64_t n_loci,
                              int keep_p_minus_1, int64_t *n_cols_added, const char *who) {
     pg_ctx *ctx = h->ctx;
-    if (!h->d_w) KCUDA(ctx, cudaMalloc(&h->d_w, (size_t)h->n * 8));
+    PG_CUDA(ctx, h->d_w.reserve((size_t)h->n, h->stream));
     {
         std::vector<double> w(h->n);
         double S = 0.0;
         for (int i = 0; i < h->n; i++) S = S + filter->pool_sizes[i];
         for (int i = 0; i < h->n; i++) w[i] = filter->pool_sizes[i] / S;  // sync.rs:262-270
-        KCUDA(ctx, cudaMemcpyAsync(h->d_w, w.data(), (size_t)h->n * 8, cudaMemcpyHostToDevice, h->stream));
-        KCUDA(ctx, cudaStreamSynchronize(h->stream));
+        PG_CUDA(ctx, cudaMemcpyAsync(h->d_w.get(), w.data(), (size_t)h->n * 8, cudaMemcpyHostToDevice, h->stream));
+        PG_CUDA(ctx, cudaStreamSynchronize(h->stream));
     }
     pg::LoadParams lp;
     memset(&lp, 0, sizeof lp);
-    lp.counts = (const uint32_t *)h->d_counts;
+    lp.counts = h->d_counts.get();
     lp.n_loci = n_loci;
     lp.n = h->n;
     lp.A_in = n_alleles;
@@ -1131,27 +1082,28 @@ static int kin_load_resident(pg_kin *h, const pg_filter *filter, int n_alleles, 
     lp.one_minus_maf = 1.00 - filter->min_allele_frequency;
     lp.max_miss = filter->max_missingness_rate;
     lp.min_depth_f = (double)filter->min_coverage_depth;
-    lp.w = h->d_w;
-    lp.sel = h->d_sel;
-    lp.offsets = h->d_off;
-    lp.G = h->d_G;
+    lp.w = h->d_w.get();
+    lp.sel = h->d_sel.get();
+    lp.offsets = h->d_off.get();
+    lp.G = h->d_G.get();
     lp.col_base = h->P;
-    lp.col_locus = h->d_col_locus;
-    lp.col_allele = h->d_col_allele;
+    lp.col_locus = h->d_col_locus.get();
+    lp.col_allele = h->d_col_allele.get();
     const int grid = (int)std::min<int64_t>((n_loci * 32 + 255) / 256, (int64_t)ctx->sm_count * 8);
     pg::load_decide_kernel<<<grid, 256, 0, h->stream>>>(lp);
-    KCUDA(ctx, cudaGetLastError());
-    KCUDA(ctx, cudaMemsetAsync(h->d_off + n_loci, 0, 8, h->stream));
-    size_t tmp = h->scan_tmp_bytes;
-    KCUDA(ctx, cub::DeviceScan::ExclusiveSum(h->d_scan_tmp, tmp, h->d_off, h->d_off, (int)(n_loci + 1), h->stream));
+    PG_CUDA(ctx, cudaGetLastError());
+    PG_CUDA(ctx, cudaMemsetAsync(h->d_off.get() + n_loci, 0, 8, h->stream));
+    size_t tmp = h->d_scan_tmp.capacity();
+    PG_CUDA(ctx, cub::DeviceScan::ExclusiveSum(h->d_scan_tmp.get(), tmp, h->d_off.get(), h->d_off.get(), (int)(n_loci + 1),
+                                               h->stream));
     int64_t added = 0;
-    KCUDA(ctx, cudaMemcpyAsync(&added, h->d_off + n_loci, 8, cudaMemcpyDeviceToHost, h->stream));
-    KCUDA(ctx, cudaStreamSynchronize(h->stream));
+    PG_CUDA(ctx, cudaMemcpyAsync(&added, h->d_off.get() + n_loci, 8, cudaMemcpyDeviceToHost, h->stream));
+    PG_CUDA(ctx, cudaStreamSynchronize(h->stream));
     if (h->P + added > h->cap)
-        return kfail(ctx, PG_ERR_ARG, "%s: %lld + %lld columns > capacity %lld", who, (long long)h->P,
+        return fail(ctx, PG_ERR_ARG, "%s: %lld + %lld columns > capacity %lld", who, (long long)h->P,
                      (long long)added, (long long)h->cap);
     pg::load_emit_kernel<<<grid, 256, 0, h->stream>>>(lp);
-    KCUDA(ctx, cudaGetLastError());
+    PG_CUDA(ctx, cudaGetLastError());
     h->P += added;
     if (n_cols_added) *n_cols_added = added;
     return PG_OK;
@@ -1163,13 +1115,13 @@ int pg_kin_append_counts(pg_kin *h, const pg_filter *filter, int n_alleles, cons
         return PG_ERR_ARG;
     pg_ctx *ctx = h->ctx;
     if (filter->n_pool_sizes != h->n || !filter->pool_sizes)
-        return kfail(ctx, PG_ERR_ARG, "pg_kin_append_counts: %d pool sizes for %d pools", filter->n_pool_sizes, h->n);
-    KCUDA(ctx, cudaSetDevice(ctx->device));
+        return fail(ctx, PG_ERR_ARG, "pg_kin_append_counts: %d pool sizes for %d pools", filter->n_pool_sizes, h->n);
+    PG_CUDA(ctx, cudaSetDevice(ctx->device));
     if (n_cols_added) *n_cols_added = 0;
     if (n_loci == 0) return PG_OK;
     int rc = kin_reserve(h, n_loci, n_alleles);
     if (rc) return rc;
-    KCUDA(ctx, cudaMemcpyAsync(h->d_counts, counts, (size_t)n_loci * n_alleles * h->n * 4, cudaMemcpyHostToDevice,
+    PG_CUDA(ctx, cudaMemcpyAsync(h->d_counts.get(), counts, (size_t)n_loci * n_alleles * h->n * 4, cudaMemcpyHostToDevice,
                                h->stream));
     return kin_load_resident(h, filter, n_alleles, codes, n_loci, keep_p_minus_1, n_cols_added, "pg_kin_append_counts");
 }
@@ -1181,8 +1133,8 @@ int pg_kin_append_sync_text(pg_kin *h, const pg_filter *filter, const char *text
     if (!h || !filter || (!text && n_bytes > 0) || max_loci < 1) return PG_ERR_ARG;
     pg_ctx *ctx = h->ctx;
     if (filter->n_pool_sizes != h->n || !filter->pool_sizes)
-        return kfail(ctx, PG_ERR_ARG, "pg_kin_append_sync_text: %d pool sizes for %d pools", filter->n_pool_sizes, h->n);
-    KCUDA(ctx, cudaSetDevice(ctx->device));
+        return fail(ctx, PG_ERR_ARG, "pg_kin_append_sync_text: %d pool sizes for %d pools", filter->n_pool_sizes, h->n);
+    PG_CUDA(ctx, cudaSetDevice(ctx->device));
     if (n_cols_added) *n_cols_added = 0;
     if (n_loci_out) *n_loci_out = 0;
     int rc = kin_reserve(h, max_loci, 6);
@@ -1192,17 +1144,13 @@ int pg_kin_append_sync_text(pg_kin *h, const pg_filter *filter, const char *text
     int64_t L = 0;
     size_t line_cap = 0;
     for (int attempt = 0; attempt < 2; attempt++) {
-        KCUDA(ctx, pg::text_parse_async(&h->text, text, n_bytes, h->n, (uint32_t *)h->d_counts, max_loci, line_cap,
-                                        ctx->sm_count, h->stream));
-        L = pg::text_parse_finish(h->text, h->stream, &ce, &at);
+        PG_CUDA(ctx, pg::text_parse_async(&h->text, text, n_bytes, h->n, h->d_counts.get(), max_loci, line_cap,
+                                          ctx->sm_count, h->stream));
+        L = pg::text_parse_finish(&h->text, h->stream, &ce, &at);
         if (L != -5) break;
         line_cap = (size_t)at + 1;  // more comment / blank lines than the default bound: repeat with the exact number
     }
-    if (L == -1) return kfail(ctx, PG_ERR_CUDA, "pg_kin_append_sync_text: %s", cudaGetErrorString(ce));
-    if (L == -2) return kfail(ctx, PG_ERR_ARG, "pg_kin_append_sync_text: more loci in the chunk than max_loci %lld", (long long)max_loci);
-    if (L == -3) return kfail(ctx, PG_ERR_ARG, "pg_kin_append_sync_text: the line at byte %llu does not hold %d pools", (unsigned long long)at, h->n);
-    if (L == -4) return kfail(ctx, PG_ERR_ARG, "pg_kin_append_sync_text: malformed pool field at byte %llu", (unsigned long long)at);
-    if (L < 0) return kfail(ctx, PG_ERR_ARG, "pg_kin_append_sync_text: the chunk could not be parsed (%lld)", (long long)L);
+    if (L < 0) return pg::text_parse_fail(ctx, "pg_kin_append_sync_text", L, ce, at, h->n, max_loci);
     if (n_loci_out) *n_loci_out = L;
     if (L == 0) return PG_OK;
     static const uint8_t sync_codes[6] = {0, 1, 2, 3, 4, 5};
@@ -1211,32 +1159,32 @@ int pg_kin_append_sync_text(pg_kin *h, const pg_filter *filter, const char *text
 
 int pg_kin_text_labels(pg_kin *h, const uint64_t **line_offsets, const uint64_t **positions) {
     if (!h) return PG_ERR_ARG;
-    if (!h->text) return kfail(h->ctx, PG_ERR_STATE, "pg_kin_text_labels before pg_kin_append_sync_text");
-    KCUDA(h->ctx, cudaStreamSynchronize(h->stream));  // the label copy was enqueued by the parse
-    if (line_offsets) *line_offsets = pg::text_offsets(h->text);
-    if (positions) *positions = pg::text_positions(h->text);
+    if (!h->text.parsed) return fail(h->ctx, PG_ERR_STATE, "pg_kin_text_labels before pg_kin_append_sync_text");
+    PG_CUDA(h->ctx, cudaStreamSynchronize(h->stream));  // the label copy was enqueued by the parse
+    if (line_offsets) *line_offsets = h->text.h_out_offset.get();
+    if (positions) *positions = h->text.h_out_pos.get();
     return PG_OK;
 }
 
 int pg_kin_last_labels(pg_kin *h, int64_t n_cols, int64_t *col_locus, uint8_t *col_allele) {
     if (!h || n_cols < 0) return PG_ERR_ARG;
     if (n_cols == 0) return PG_OK;
-    KCUDA(h->ctx, cudaMemcpyAsync(col_locus, h->d_col_locus, (size_t)n_cols * 8, cudaMemcpyDeviceToHost, h->stream));
-    KCUDA(h->ctx, cudaMemcpyAsync(col_allele, h->d_col_allele, (size_t)n_cols, cudaMemcpyDeviceToHost, h->stream));
-    KCUDA(h->ctx, cudaStreamSynchronize(h->stream));
+    PG_CUDA(h->ctx, cudaMemcpyAsync(col_locus, h->d_col_locus.get(), (size_t)n_cols * 8, cudaMemcpyDeviceToHost, h->stream));
+    PG_CUDA(h->ctx, cudaMemcpyAsync(col_allele, h->d_col_allele.get(), (size_t)n_cols, cudaMemcpyDeviceToHost, h->stream));
+    PG_CUDA(h->ctx, cudaStreamSynchronize(h->stream));
     return PG_OK;
 }
 
 int pg_kin_synth(pg_kin *h, uint64_t seed, int64_t first_locus, int64_t n_loci) {
     if (!h || n_loci < 0) return PG_ERR_ARG;
     pg_ctx *ctx = h->ctx;
-    if (h->P + 2 * n_loci > h->cap) return kfail(ctx, PG_ERR_ARG, "pg_kin_synth: capacity");
-    KCUDA(ctx, cudaSetDevice(ctx->device));
+    if (h->P + 2 * n_loci > h->cap) return fail(ctx, PG_ERR_ARG, "pg_kin_synth: capacity");
+    PG_CUDA(ctx, cudaSetDevice(ctx->device));
     if (n_loci == 0) return PG_OK;
     const int grid = (int)std::min<int64_t>((n_loci * h->ldg + 255) / 256, (int64_t)ctx->sm_count * 16);
     pg::kin_synth_kernel<<<grid, 256, 0, h->stream>>>(seed, first_locus, n_loci, h->n, h->ldg,
-                                                      h->d_G + (size_t)h->P * h->ldg);
-    KCUDA(ctx, cudaGetLastError());
+                                                      h->d_G.get() + (size_t)h->P * h->ldg);
+    PG_CUDA(ctx, cudaGetLastError());
     h->P += 2 * n_loci;
     return PG_OK;
 }
@@ -1244,9 +1192,9 @@ int pg_kin_synth(pg_kin *h, uint64_t seed, int64_t first_locus, int64_t n_loci) 
 int pg_kin_get_columns(pg_kin *h, int64_t first, int64_t count, double *out) {
     if (!h || first < 0 || count < 0 || first + count > h->P || (!out && count)) return PG_ERR_ARG;
     if (!count) return PG_OK;
-    KCUDA(h->ctx, cudaMemcpy2DAsync(out, (size_t)h->n * 8, h->d_G + (size_t)first * h->ldg, (size_t)h->ldg * 8,
+    PG_CUDA(h->ctx, cudaMemcpy2DAsync(out, (size_t)h->n * 8, h->d_G.get() + (size_t)first * h->ldg, (size_t)h->ldg * 8,
                                     (size_t)h->n * 8, (size_t)count, cudaMemcpyDeviceToHost, h->stream));
-    KCUDA(h->ctx, cudaStreamSynchronize(h->stream));
+    PG_CUDA(h->ctx, cudaStreamSynchronize(h->stream));
     return PG_OK;
 }
 
@@ -1258,39 +1206,32 @@ static int gram_launch(pg_kin *h, bool accumulate) {
     int n_slices = (int)std::max<int64_t>(1, std::min<int64_t>((8LL * ctx->sm_count + ntiles - 1) / ntiles, P_pad / pg::kKC));
     int64_t slice_cols = round_up((P_pad + n_slices - 1) / n_slices, pg::kKC);
     n_slices = (int)((P_pad + slice_cols - 1) / slice_cols);
-    const size_t ws = (size_t)n_slices * ntiles * pg::kTile * pg::kTile * 8;
-    if (h->ws_bytes < ws) {
-        KCUDA(ctx, cudaStreamSynchronize(h->stream));
-        cudaFree(h->d_ws);
-        h->d_ws = nullptr;
-        KCUDA(ctx, cudaMalloc(&h->d_ws, ws));
-        h->ws_bytes = ws;
-    }
+    PG_CUDA(ctx, h->d_ws.reserve((size_t)n_slices * ntiles * pg::kTile * pg::kTile, h->stream));
     h->n_slices = n_slices;
     pg::GramParams gp;
-    gp.G = h->d_G;
+    gp.G = h->d_G.get();
     gp.P_pad = P_pad;
     gp.ldg = h->ldg;
     gp.n = h->n;
     gp.nt = h->nt;
     gp.n_slices = n_slices;
     gp.slice_cols = slice_cols;
-    gp.ws = h->d_ws;
+    gp.ws = h->d_ws.get();
     const size_t smem = 128 + (size_t)pg::kStages * 2 * pg::kKC * pg::kPitch * 8;
-    KCUDA(ctx, cudaFuncSetAttribute(pg::gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    PG_CUDA(ctx, cudaFuncSetAttribute(pg::gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int64_t items = (int64_t)ntiles * n_slices;
     const int grid = (int)std::min<int64_t>(items, ctx->sm_count);
     pg::gram_kernel<<<grid, (pg::kGramWarps + 1) * 32, smem, h->stream>>>(gp);
-    KCUDA(ctx, cudaGetLastError());
-    pg::gram_reduce_kernel<<<ctx->sm_count * 4, 256, 0, h->stream>>>(h->d_ws, h->nt, n_slices, h->n, accumulate ? 1 : 0,
-                                                                     h->d_K);
-    KCUDA(ctx, cudaGetLastError());
+    PG_CUDA(ctx, cudaGetLastError());
+    pg::gram_reduce_kernel<<<ctx->sm_count * 4, 256, 0, h->stream>>>(h->d_ws.get(), h->nt, n_slices, h->n,
+                                                                     accumulate ? 1 : 0, h->d_K.get());
+    PG_CUDA(ctx, cudaGetLastError());
     return PG_OK;
 }
 
 int pg_kin_gram(pg_kin *h) {
     if (!h) return PG_ERR_ARG;
-    KCUDA(h->ctx, cudaSetDevice(h->ctx->device));
+    PG_CUDA(h->ctx, cudaSetDevice(h->ctx->device));
     return gram_launch(h, false);
 }
 
@@ -1298,93 +1239,116 @@ int pg_kin_gram(pg_kin *h) {
 // pg_kin_gram_accumulate on the others, pg_kin_reset in between), and K ends up the Gram matrix of all of them
 int pg_kin_gram_accumulate(pg_kin *h) {
     if (!h) return PG_ERR_ARG;
-    KCUDA(h->ctx, cudaSetDevice(h->ctx->device));
+    PG_CUDA(h->ctx, cudaSetDevice(h->ctx->device));
     return gram_launch(h, true);
 }
 
 int pg_kin_gram_time(pg_kin *h, int iters, float *ms_total) {
     if (!h || iters < 1 || !ms_total) return PG_ERR_ARG;
     pg_ctx *ctx = h->ctx;
-    KCUDA(ctx, cudaSetDevice(ctx->device));
-    KCUDA(ctx, cudaStreamSynchronize(h->stream));
-    KCUDA(ctx, cudaEventRecord(h->ev0, h->stream));
+    PG_CUDA(ctx, cudaSetDevice(ctx->device));
+    PG_CUDA(ctx, cudaStreamSynchronize(h->stream));
+    PG_CUDA(ctx, cudaEventRecord(h->ev0, h->stream));
     for (int i = 0; i < iters; i++) {
         int rc = gram_launch(h, false);
         if (rc) return rc;
     }
-    KCUDA(ctx, cudaEventRecord(h->ev1, h->stream));
-    KCUDA(ctx, cudaEventSynchronize(h->ev1));
-    KCUDA(ctx, cudaEventElapsedTime(ms_total, h->ev0, h->ev1));
+    PG_CUDA(ctx, cudaEventRecord(h->ev1, h->stream));
+    PG_CUDA(ctx, cudaEventSynchronize(h->ev1));
+    PG_CUDA(ctx, cudaEventElapsedTime(ms_total, h->ev0, h->ev1));
     return PG_OK;
 }
 
 int pg_kin_partial(pg_kin *h, double **dev_ptr, size_t *n_elems) {
     if (!h || !dev_ptr) return PG_ERR_ARG;
-    KCUDA(h->ctx, cudaStreamSynchronize(h->stream));
-    *dev_ptr = h->d_K;
+    PG_CUDA(h->ctx, cudaStreamSynchronize(h->stream));
+    *dev_ptr = h->d_K.get();
     if (n_elems) *n_elems = (size_t)h->n * h->n;
     return PG_OK;
 }
 
 int pg_kin_partial_get(pg_kin *h, double *out) {
     if (!h || !out) return PG_ERR_ARG;
-    KCUDA(h->ctx, cudaMemcpyAsync(out, h->d_K, (size_t)h->n * h->n * 8, cudaMemcpyDeviceToHost, h->stream));
-    KCUDA(h->ctx, cudaStreamSynchronize(h->stream));
+    PG_CUDA(h->ctx, cudaMemcpyAsync(out, h->d_K.get(), (size_t)h->n * h->n * 8, cudaMemcpyDeviceToHost, h->stream));
+    PG_CUDA(h->ctx, cudaStreamSynchronize(h->stream));
     return PG_OK;
 }
 
 int pg_kin_partial_set(pg_kin *h, const double *in) {
     if (!h || !in) return PG_ERR_ARG;
-    KCUDA(h->ctx, cudaMemcpyAsync(h->d_K, in, (size_t)h->n * h->n * 8, cudaMemcpyHostToDevice, h->stream));
-    KCUDA(h->ctx, cudaStreamSynchronize(h->stream));
+    PG_CUDA(h->ctx, cudaMemcpyAsync(h->d_K.get(), in, (size_t)h->n * h->n * 8, cudaMemcpyHostToDevice, h->stream));
+    PG_CUDA(h->ctx, cudaStreamSynchronize(h->stream));
     return PG_OK;
+}
+
+// h->C = the m covariates, covariate l at pool i being cov[i * pool_stride + l * cov_stride]; h->Q = an orthonormal
+// basis of [1 | C] (modified Gram-Schmidt, twice).  Returns the first column of [1 | C] found collinear with the
+// columns before it, -1 when there is none.
+static int kin_set_basis(pg_kin *h, int m, const double *cov, ptrdiff_t pool_stride, ptrdiff_t cov_stride) {
+    const int n = h->n, ldg = h->ldg, nq = 1 + m;
+    h->Q.assign((size_t)nq * ldg, 0.0);
+    for (int i = 0; i < n; i++) h->Q[i] = 1.0;
+    for (int l = 0; l < m; l++)
+        for (int i = 0; i < n; i++) h->Q[(size_t)(1 + l) * ldg + i] = cov[i * pool_stride + l * cov_stride];
+    h->C.assign(h->Q.begin() + ldg, h->Q.end());
+    for (int c = 0; c < nq; c++) {
+        double *qc = &h->Q[(size_t)c * ldg];
+        for (int pass = 0; pass < 2; pass++)
+            for (int b = 0; b < c; b++) {
+                const double *qb = &h->Q[(size_t)b * ldg];
+                double d = 0.0;
+                for (int i = 0; i < n; i++) d += qb[i] * qc[i];
+                for (int i = 0; i < n; i++) qc[i] -= d * qb[i];
+            }
+        double nn = 0.0;
+        for (int i = 0; i < n; i++) nn += qc[i] * qc[i];
+        nn = sqrt(nn);
+        if (!(nn > 1e-12)) return c;
+        for (int i = 0; i < n; i++) qc[i] /= nn;
+    }
+    return -1;
 }
 
 // K = (sum of the partial Gram matrices) / P_total; eigen-decomposition; number of PCs by the reference's rule
 int pg_kin_eig_select(pg_kin *h, int64_t P_total, double threshold, int *m_out) {
     if (!h || P_total < 0) return PG_ERR_ARG;
     if (P_total == 0) P_total = h->P_total > 0 ? h->P_total : h->P;  // the count pg_kin_allreduce summed, else the resident columns
-    if (P_total < 1) return kfail(h->ctx, PG_ERR_STATE, "pg_kin_eig_select: no columns");
+    if (P_total < 1) return fail(h->ctx, PG_ERR_STATE, "pg_kin_eig_select: no columns");
     pg_ctx *ctx = h->ctx;
     const int n = h->n;
-    KCUDA(ctx, cudaSetDevice(ctx->device));
-    KCUDA(ctx, cudaStreamSynchronize(h->stream));
-    double *dA = nullptr, *dW = nullptr, *dwork = nullptr;
-    int *dinfo = nullptr;
-    int rc = PG_OK;
+    PG_CUDA(ctx, cudaSetDevice(ctx->device));
+    PG_CUDA(ctx, cudaStreamSynchronize(h->stream));
     std::vector<double> A((size_t)n * n), W(n);
     if (h->warm.joinable()) h->warm.join();  // the handle the background thread of pg_kin_open creates
     const CusolverApi &sol = cusolver_api();
-    if (!sol.ok) return kfail(ctx, PG_ERR_CUDA, "pg_kin_eig_select: libcusolver could not be loaded (%s)", dlerror() ? dlerror() : "missing symbols");
+    if (!sol.ok) return fail(ctx, PG_ERR_CUDA, "pg_kin_eig_select: libcusolver could not be loaded (%s)", dlerror() ? dlerror() : "missing symbols");
     if (!h->solver) {
         cusolverDnHandle_t made = nullptr;
-        if (sol.create(&made) != CUSOLVER_STATUS_SUCCESS) return kfail(ctx, PG_ERR_CUDA, "cusolverDnCreate failed");
+        if (sol.create(&made) != CUSOLVER_STATUS_SUCCESS) return fail(ctx, PG_ERR_CUDA, "cusolverDnCreate failed");
         h->solver = made;
     }
     cusolverDnHandle_t cs = static_cast<cusolverDnHandle_t>(h->solver);
-    do {
-        sol.set_stream(cs, h->stream);
-        if (cudaMalloc(&dA, (size_t)n * n * 8) != cudaSuccess || cudaMalloc(&dW, (size_t)n * 8) != cudaSuccess ||
-            cudaMalloc(&dinfo, 4) != cudaSuccess) { rc = kfail(ctx, PG_ERR_CUDA, "pg_kin_eig_select: out of device memory"); break; }
-        // scale on the host path is avoided: eigenvectors do not depend on the scale, eigenvalue SHARES neither
-        cudaMemcpyAsync(dA, h->d_K, (size_t)n * n * 8, cudaMemcpyDeviceToDevice, h->stream);
-        int lwork = 0;
-        if (sol.syevd_buffer(cs, CUSOLVER_EIG_MODE_VECTOR, CUBLAS_FILL_MODE_LOWER, n, dA, n, dW, &lwork) !=
-            CUSOLVER_STATUS_SUCCESS) { rc = kfail(ctx, PG_ERR_CUDA, "Dsyevd_bufferSize failed"); break; }
-        if (cudaMalloc(&dwork, (size_t)lwork * 8) != cudaSuccess) { rc = kfail(ctx, PG_ERR_CUDA, "syevd workspace"); break; }
-        if (sol.syevd(cs, CUSOLVER_EIG_MODE_VECTOR, CUBLAS_FILL_MODE_LOWER, n, dA, n, dW, dwork, lwork, dinfo) !=
-            CUSOLVER_STATUS_SUCCESS) { rc = kfail(ctx, PG_ERR_CUDA, "Dsyevd failed"); break; }
-        int info = 0;
-        cudaMemcpyAsync(&info, dinfo, 4, cudaMemcpyDeviceToHost, h->stream);
-        cudaMemcpyAsync(A.data(), dA, (size_t)n * n * 8, cudaMemcpyDeviceToHost, h->stream);
-        cudaMemcpyAsync(W.data(), dW, (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream);
-        if (cudaStreamSynchronize(h->stream) != cudaSuccess || info != 0) { rc = kfail(ctx, PG_ERR_CUDA, "Dsyevd info %d", info); break; }
-    } while (0);
-    cudaFree(dA);
-    cudaFree(dW);
-    cudaFree(dwork);
-    cudaFree(dinfo);
-    if (rc) return rc;
+    sol.set_stream(cs, h->stream);
+    pg::DeviceBuffer<double> dA, dW, dwork;
+    pg::DeviceBuffer<int> dinfo;
+    if (dA.reserve((size_t)n * n, h->stream) != cudaSuccess || dW.reserve((size_t)n, h->stream) != cudaSuccess ||
+        dinfo.reserve(1, h->stream) != cudaSuccess)
+        return fail(ctx, PG_ERR_CUDA, "pg_kin_eig_select: out of device memory");
+    // scale on the host path is avoided: eigenvectors do not depend on the scale, eigenvalue SHARES neither
+    cudaMemcpyAsync(dA.get(), h->d_K.get(), (size_t)n * n * 8, cudaMemcpyDeviceToDevice, h->stream);
+    int lwork = 0;
+    if (sol.syevd_buffer(cs, CUSOLVER_EIG_MODE_VECTOR, CUBLAS_FILL_MODE_LOWER, n, dA.get(), n, dW.get(), &lwork) !=
+        CUSOLVER_STATUS_SUCCESS)
+        return fail(ctx, PG_ERR_CUDA, "Dsyevd_bufferSize failed");
+    if (dwork.reserve((size_t)lwork, h->stream) != cudaSuccess) return fail(ctx, PG_ERR_CUDA, "syevd workspace");
+    if (sol.syevd(cs, CUSOLVER_EIG_MODE_VECTOR, CUBLAS_FILL_MODE_LOWER, n, dA.get(), n, dW.get(), dwork.get(), lwork,
+                  dinfo.get()) != CUSOLVER_STATUS_SUCCESS)
+        return fail(ctx, PG_ERR_CUDA, "Dsyevd failed");
+    int info = 0;
+    cudaMemcpyAsync(&info, dinfo.get(), 4, cudaMemcpyDeviceToHost, h->stream);
+    cudaMemcpyAsync(A.data(), dA.get(), (size_t)n * n * 8, cudaMemcpyDeviceToHost, h->stream);
+    cudaMemcpyAsync(W.data(), dW.get(), (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream);
+    if (cudaStreamSynchronize(h->stream) != cudaSuccess || info != 0) return fail(ctx, PG_ERR_CUDA, "Dsyevd info %d", info);
     // syevd returns ascending eigenvalues, column j of A (column-major) = eigenvector j; the reference walks them
     // "sorted from high to low" (ols.rs:296)
     h->eigvals.resize(n);
@@ -1411,28 +1375,9 @@ int pg_kin_eig_select(pg_kin *h, int64_t P_total, double threshold, int *m_out) 
         for (int i = 0; i < n; i++) h->Q[i] = 1.0 / sqrt((double)n);
         return PG_OK;
     }
-    // Q = orthonormal basis of [1 | v_1 .. v_m] (modified Gram-Schmidt, twice)
-    const int nq = 1 + m, ldg = h->ldg;
-    h->Q.assign((size_t)nq * ldg, 0.0);
-    for (int i = 0; i < n; i++) h->Q[i] = 1.0;
-    for (int l = 0; l < m; l++)
-        for (int i = 0; i < n; i++) h->Q[(size_t)(1 + l) * ldg + i] = A[(size_t)(n - 1 - l) * n + i];
-    h->C.assign(h->Q.begin() + ldg, h->Q.end());
-    for (int c = 0; c < nq; c++) {
-        double *qc = &h->Q[(size_t)c * ldg];
-        for (int pass = 0; pass < 2; pass++)
-            for (int b = 0; b < c; b++) {
-                const double *qb = &h->Q[(size_t)b * ldg];
-                double d = 0.0;
-                for (int i = 0; i < n; i++) d += qb[i] * qc[i];
-                for (int i = 0; i < n; i++) qc[i] -= d * qb[i];
-            }
-        double nn = 0.0;
-        for (int i = 0; i < n; i++) nn += qc[i] * qc[i];
-        nn = sqrt(nn);
-        if (!(nn > 1e-12)) return kfail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_eig_select: covariate %d is collinear with the intercept", c);
-        for (int i = 0; i < n; i++) qc[i] /= nn;
-    }
+    // the covariates are v_1 .. v_m: column n - 1 - l of A (column-major)
+    const int c = kin_set_basis(h, m, A.data() + (size_t)(n - 1) * n, 1, -(ptrdiff_t)n);
+    if (c >= 0) return fail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_eig_select: covariate %d is collinear with the intercept", c);
     return PG_OK;
 }
 
@@ -1440,8 +1385,8 @@ int pg_kin_eig_select(pg_kin *h, int64_t P_total, double threshold, int *m_out) 
 // outcome -- number of PCs, the orthonormal basis of [1 | PCs], the eigenvalues
 int pg_kin_copy_covariates(pg_kin *dst, const pg_kin *src) {
     if (!dst || !src) return PG_ERR_ARG;
-    if (src->m < 0) return kfail(dst->ctx, PG_ERR_STATE, "pg_kin_copy_covariates: the source has no covariates yet");
-    if (dst->n != src->n) return kfail(dst->ctx, PG_ERR_ARG, "pg_kin_copy_covariates: %d vs %d pools", dst->n, src->n);
+    if (src->m < 0) return fail(dst->ctx, PG_ERR_STATE, "pg_kin_copy_covariates: the source has no covariates yet");
+    if (dst->n != src->n) return fail(dst->ctx, PG_ERR_ARG, "pg_kin_copy_covariates: %d vs %d pools", dst->n, src->n);
     dst->m = src->m;
     dst->minnorm = src->minnorm;
     dst->Q = src->Q;
@@ -1461,30 +1406,12 @@ int pg_kin_eigvals(pg_kin *h, double *out, int count) {
 int pg_kin_set_covariates(pg_kin *h, const double *cov, int m) {
     if (!h || m < 0 || (m > 0 && !cov)) return PG_ERR_ARG;
     pg_ctx *ctx = h->ctx;
-    const int n = h->n, ldg = h->ldg, nq = 1 + m;
-    if (m + 2 > n) return kfail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_set_covariates: %d covariates for %d pools", m, n);
+    const int n = h->n;
+    if (m + 2 > n) return fail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_set_covariates: %d covariates for %d pools", m, n);
     h->m = m;
     h->minnorm = false;
-    h->Q.assign((size_t)nq * ldg, 0.0);
-    for (int i = 0; i < n; i++) h->Q[i] = 1.0;
-    for (int l = 0; l < m; l++)
-        for (int i = 0; i < n; i++) h->Q[(size_t)(1 + l) * ldg + i] = cov[(size_t)i * m + l];
-    h->C.assign(h->Q.begin() + ldg, h->Q.end());
-    for (int c = 0; c < nq; c++) {
-        double *qc = &h->Q[(size_t)c * ldg];
-        for (int pass = 0; pass < 2; pass++)
-            for (int b = 0; b < c; b++) {
-                const double *qb = &h->Q[(size_t)b * ldg];
-                double d = 0.0;
-                for (int i = 0; i < n; i++) d += qb[i] * qc[i];
-                for (int i = 0; i < n; i++) qc[i] -= d * qb[i];
-            }
-        double nn = 0.0;
-        for (int i = 0; i < n; i++) nn += qc[i] * qc[i];
-        nn = sqrt(nn);
-        if (!(nn > 1e-12)) return kfail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_set_covariates: covariate %d is collinear", c);
-        for (int i = 0; i < n; i++) qc[i] /= nn;
-    }
+    const int c = kin_set_basis(h, m, cov, m, 1);
+    if (c >= 0) return fail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_set_covariates: covariate %d is collinear", c);
     return PG_OK;
 }
 
@@ -1539,14 +1466,14 @@ static int covar_launch_generic(pg_kin *h, const pg::CovarParams &cp) {
     const int nv = cp.nq + cp.k;
     const size_t per_warp = (size_t)(cp.ldg + nv) * 8;
     const int warps = (int)std::min<size_t>(8, (200 * 1024) / per_warp);
-    if (warps < 1) return kfail(ctx, PG_ERR_UNSUPPORTED, "covariate scan: %d pools x %d vectors exceed shared memory", cp.n, nv);
+    if (warps < 1) return fail(ctx, PG_ERR_UNSUPPORTED, "covariate scan: %d pools x %d vectors exceed shared memory", cp.n, nv);
     const size_t smem = per_warp * warps;
     cudaError_t e = cudaFuncSetAttribute(pg::covar_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e == cudaSuccess) {
         pg::covar_generic_kernel<<<ctx->sm_count, warps * 32, smem, h->stream>>>(cp);
         e = cudaGetLastError();
     }
-    if (e != cudaSuccess) return kfail(ctx, PG_ERR_CUDA, "covar_generic_kernel: %s", cudaGetErrorString(e));
+    if (e != cudaSuccess) return fail(ctx, PG_ERR_CUDA, "covar_generic_kernel: %s", cudaGetErrorString(e));
     return PG_OK;
 }
 
@@ -1588,19 +1515,11 @@ static int covar_launch(pg_kin *h, const pg::CovarParams &cp_in) {
     const bool mma = !no_mma && nv >= 5 && fits_nv(cp_in.nq + kk);
     // the list of columns the streaming kernels leave to the explicit-residual forms: [count | columns], at most one
     // entry per column and pass
-    const size_t need = ((size_t)cp_in.P * (size_t)(mma ? (cp_in.k + kk - 1) / kk : 1) + 2) * 8;
-    if (h->defer_bytes < need) {
-        KCUDA(ctx, cudaStreamSynchronize(h->stream));
-        cudaFree(h->d_defer);
-        h->d_defer = nullptr;
-        h->defer_bytes = 0;
-        KCUDA(ctx, cudaMalloc(&h->d_defer, need));
-        h->defer_bytes = need;
-    }
-    KCUDA(ctx, cudaMemsetAsync(h->d_defer, 0, 8, h->stream));
+    PG_CUDA(ctx, h->d_defer.reserve((size_t)cp_in.P * (size_t)(mma ? (cp_in.k + kk - 1) / kk : 1) + 2, h->stream));
+    PG_CUDA(ctx, cudaMemsetAsync(h->d_defer.get(), 0, 8, h->stream));
     pg::CovarParams cp = cp_in;
-    cp.defer_count = reinterpret_cast<unsigned *>(h->d_defer);
-    cp.defer_list = reinterpret_cast<int64_t *>(h->d_defer) + 1;
+    cp.defer_count = reinterpret_cast<unsigned *>(h->d_defer.get());
+    cp.defer_list = h->d_defer.get() + 1;
     const bool fits = (size_t)nv * cp.ldg * 8 <= 227 * 1024;  // the vectors in shared memory (covar_kernel)
     if (mma) {
         for (int y0 = 0; y0 < cp.k; y0 += kk) {
@@ -1610,31 +1529,21 @@ static int covar_launch(pg_kin *h, const pg::CovarParams &cp_in) {
             const int nvp = pp.nq + pp.k, mt = nvp <= 8 ? 1 : 2;
             int per = 0;
             const int np = pool_plan(nvp, &per);
-            if (np > 1) {
-                const size_t need_part = (size_t)((cp.P + 7) / 8) * (size_t)(8 * mt + 1) * 8 * 8;
-                if (h->part_bytes < need_part) {
-                    KCUDA(ctx, cudaStreamSynchronize(h->stream));
-                    cudaFree(h->d_part);
-                    h->d_part = nullptr;
-                    h->part_bytes = 0;
-                    KCUDA(ctx, cudaMalloc(&h->d_part, need_part));
-                    h->part_bytes = need_part;
-                }
-            }
+            if (np > 1) PG_CUDA(ctx, h->d_part.reserve((size_t)((cp.P + 7) / 8) * (size_t)(8 * mt + 1) * 8, h->stream));
             auto kern = mt == 1 ? pg::covar_mma_kernel<1> : pg::covar_mma_kernel<2>;
             for (int ip = 0; ip < np; ip++) {
                 pp.pr0 = ip * per;
                 pp.pn = std::min(per, cp.n - pp.pr0);
                 pp.part_mode = (ip + 1 < np ? 1 : 0) | (ip > 0 ? 2 : 0);
-                pp.part = h->d_part;
+                pp.part = h->d_part.get();
                 if (!covar_mma_fits(pp, nvp, &ldq, &warps, &smem_mma, pp.pn))
-                    return kfail(ctx, PG_ERR_UNSUPPORTED, "covariate scan: %d vectors x %d pools do not fit a pool pass", nvp, pp.pn);
+                    return fail(ctx, PG_ERR_UNSUPPORTED, "covariate scan: %d vectors x %d pools do not fit a pool pass", nvp, pp.pn);
                 e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_mma);
                 if (e == cudaSuccess) {
                     kern<<<ctx->sm_count, warps * 32, smem_mma, h->stream>>>(pp, ldq, warps);
                     e = cudaGetLastError();
                 }
-                if (e != cudaSuccess) return kfail(ctx, PG_ERR_CUDA, "covar_mma_kernel: %s", cudaGetErrorString(e));
+                if (e != cudaSuccess) return fail(ctx, PG_ERR_CUDA, "covar_mma_kernel: %s", cudaGetErrorString(e));
             }
         }
     } else {
@@ -1662,7 +1571,7 @@ static int covar_launch(pg_kin *h, const pg::CovarParams &cp_in) {
                 return covar_launch_generic(h, pp);
             }
         }
-        if (e != cudaSuccess) return kfail(ctx, PG_ERR_CUDA, "covar_kernel: %s", cudaGetErrorString(e));
+        if (e != cudaSuccess) return fail(ctx, PG_ERR_CUDA, "covar_kernel: %s", cudaGetErrorString(e));
     }
     // the deferred columns (a centred g'g or a residual sum of squares lost to cancellation): explicit residuals, every
     // phenotype; an empty list costs one tiny launch
@@ -1684,7 +1593,7 @@ static int covar_launch(pg_kin *h, const pg::CovarParams &cp_in) {
         case 16: e = covar_launch_list<16>(cp, ctx->sm_count, h->stream); break;
         default: return covar_launch_generic(h, cp);
     }
-    if (e != cudaSuccess) return kfail(ctx, PG_ERR_CUDA, "covariate scan (deferred columns): %s", cudaGetErrorString(e));
+    if (e != cudaSuccess) return fail(ctx, PG_ERR_CUDA, "covariate scan (deferred columns): %s", cudaGetErrorString(e));
     return PG_OK;
 }
 
@@ -1692,27 +1601,20 @@ static int covar_launch(pg_kin *h, const pg::CovarParams &cp_in) {
 static int kin_prepare_records(pg_kin *h, int k) {
     pg_ctx *ctx = h->ctx;
     const double df = (double)h->n - 1.0;
-    if (!h->d_ptab) {
+    if (!h->d_ptab.get()) {
         pg::PTable tab = pg::build_ptable(df);
         if (tab.max_err < 2e-9) {
-            KCUDA(ctx, cudaMalloc(&h->d_ptab, tab.coef.size() * 8));
-            KCUDA(ctx, cudaMemcpyAsync(h->d_ptab, tab.coef.data(), tab.coef.size() * 8, cudaMemcpyHostToDevice, h->stream));
-            KCUDA(ctx, cudaStreamSynchronize(h->stream));
+            PG_CUDA(ctx, h->d_ptab.reserve(tab.coef.size(), h->stream));
+            PG_CUDA(ctx, cudaMemcpyAsync(h->d_ptab.get(), tab.coef.data(), tab.coef.size() * 8, cudaMemcpyHostToDevice, h->stream));
+            PG_CUDA(ctx, cudaStreamSynchronize(h->stream));
             h->ptab_M = tab.M;
             h->ptab_isd = tab.inv_sqrt_df;
             h->ptab_bits = tab.bits;
         }
     }
     const size_t elems = (size_t)3 * k * std::max<int64_t>(h->P, 1);
-    if (h->res_elems < elems) {
-        KCUDA(ctx, cudaStreamSynchronize(h->stream));
-        cudaFree(h->d_res);
-        if (h->h_res) cudaFreeHost(h->h_res);
-        h->d_res = nullptr, h->h_res = nullptr;
-        KCUDA(ctx, cudaMalloc(&h->d_res, elems * 8));
-        KCUDA(ctx, cudaHostAlloc((void **)&h->h_res, elems * 8, cudaHostAllocDefault));
-        h->res_elems = elems;
-    }
+    PG_CUDA(ctx, h->d_res.reserve(elems, h->stream));
+    PG_CUDA(ctx, h->h_res.reserve(elems, h->stream));
     h->k = k;
     return PG_OK;
 }
@@ -1725,11 +1627,11 @@ int pg_kin_covar_scan(pg_kin *h, const double *phen, int k, int iters, float *ms
                       const double **var, const double **pval) {
     if (!h || !phen || k < 1) return PG_ERR_ARG;
     pg_ctx *ctx = h->ctx;
-    if (h->m < 0) return kfail(ctx, PG_ERR_STATE, "pg_kin_covar_scan before pg_kin_eig_select / pg_kin_set_covariates");
+    if (h->m < 0) return fail(ctx, PG_ERR_STATE, "pg_kin_covar_scan before pg_kin_eig_select / pg_kin_set_covariates");
     const int n = h->n, ldg = h->ldg, nq = h->minnorm ? 1 : 1 + h->m;
     if (k > pg::kMaxPhenPerPass * 4)
-        return kfail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_covar_scan: %d phenotypes > %d per call", k, pg::kMaxPhenPerPass * 4);
-    KCUDA(ctx, cudaSetDevice(ctx->device));
+        return fail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_covar_scan: %d phenotypes > %d per call", k, pg::kMaxPhenPerPass * 4);
+    PG_CUDA(ctx, cudaSetDevice(ctx->device));
     // y~ = y - Q Q'y on the host (n x k, tiny)
     std::vector<double> V((size_t)(nq + k) * ldg, 0.0);
     std::copy(h->Q.begin(), h->Q.end(), V.begin());
@@ -1755,57 +1657,50 @@ int pg_kin_covar_scan(pg_kin *h, const double *phen, int k, int iters, float *ms
         for (int i = 0; i < n; i++) yy += yt[i] * yt[i];
         cp.yy[j] = yy;
     }
-    const size_t vb = V.size() * 8;
-    if (h->V_bytes < vb) {
-        KCUDA(ctx, cudaStreamSynchronize(h->stream));
-        cudaFree(h->d_V);
-        h->d_V = nullptr;
-        KCUDA(ctx, cudaMalloc(&h->d_V, vb));
-        h->V_bytes = vb;
-    }
-    KCUDA(ctx, cudaMemcpyAsync(h->d_V, V.data(), vb, cudaMemcpyHostToDevice, h->stream));
-    KCUDA(ctx, cudaStreamSynchronize(h->stream));
+    PG_CUDA(ctx, h->d_V.reserve(V.size(), h->stream));
+    PG_CUDA(ctx, cudaMemcpyAsync(h->d_V.get(), V.data(), V.size() * 8, cudaMemcpyHostToDevice, h->stream));
+    PG_CUDA(ctx, cudaStreamSynchronize(h->stream));
     const double df = (double)n - 1.0;
     if (int rc = kin_prepare_records(h, k)) return rc;
-    cp.G = h->d_G;
+    cp.G = h->d_G.get();
     cp.P = h->P;
     cp.ldg = ldg;
     cp.n = n;
     cp.nq = nq;
     cp.k = k;
-    cp.V = h->d_V;
+    cp.V = h->d_V.get();
     cp.dfe = (double)n - (double)(2 + h->m);
     cp.minnorm = h->minnorm ? 1 : 0;
     cp.nf = (double)n;
     cp.sqrt_n = sqrt((double)n);
     cp.df = df;
-    cp.ptab = h->d_ptab;
+    cp.ptab = h->d_ptab.get();
     cp.ptab_isd = h->ptab_isd;
     cp.ptab_bits = h->ptab_bits;
     cp.ptab_M = h->ptab_M;
     cp.ln_beta = pg::statrs::ln_gamma(df / 2.0 + 0.5) - pg::statrs::ln_gamma(df / 2.0) - pg::statrs::ln_gamma(0.5);
-    cp.beta = h->d_res;
-    cp.var = h->d_res + (size_t)k * h->P;
-    cp.pval = h->d_res + (size_t)2 * k * h->P;
+    cp.beta = h->d_res.get();
+    cp.var = h->d_res.get() + (size_t)k * h->P;
+    cp.pval = h->d_res.get() + (size_t)2 * k * h->P;
     const int reps = iters > 0 ? iters : 1;
-    if (iters > 0) KCUDA(ctx, cudaEventRecord(h->ev0, h->stream));
+    if (iters > 0) PG_CUDA(ctx, cudaEventRecord(h->ev0, h->stream));
     for (int i = 0; i < reps; i++) {
         int rc = covar_launch(h, cp);
         if (rc) return rc;
     }
-    if (iters > 0) KCUDA(ctx, cudaEventRecord(h->ev1, h->stream));
-    KCUDA(ctx, cudaMemcpyAsync(h->h_res, h->d_res, (size_t)3 * k * h->P * 8, cudaMemcpyDeviceToHost, h->stream));
-    KCUDA(ctx, cudaStreamSynchronize(h->stream));
-    if (iters > 0 && ms_total) KCUDA(ctx, cudaEventElapsedTime(ms_total, h->ev0, h->ev1));
+    if (iters > 0) PG_CUDA(ctx, cudaEventRecord(h->ev1, h->stream));
+    PG_CUDA(ctx, cudaMemcpyAsync(h->h_res.get(), h->d_res.get(), (size_t)3 * k * h->P * 8, cudaMemcpyDeviceToHost, h->stream));
+    PG_CUDA(ctx, cudaStreamSynchronize(h->stream));
+    if (iters > 0 && ms_total) PG_CUDA(ctx, cudaEventElapsedTime(ms_total, h->ev0, h->ev1));
     static const bool debug = getenv("PG_COVAR_DEBUG") != nullptr;  // how many columns took the explicit-residual forms
-    if (debug && h->d_defer) {
+    if (debug && h->d_defer.get()) {
         unsigned cnt = 0;
-        cudaMemcpy(&cnt, h->d_defer, 4, cudaMemcpyDeviceToHost);
+        cudaMemcpy(&cnt, h->d_defer.get(), 4, cudaMemcpyDeviceToHost);
         fprintf(stderr, "pg_kin_covar_scan: %u of %lld columns deferred to the explicit-residual kernel\n", cnt, (long long)h->P);
     }
-    if (beta) *beta = h->h_res;
-    if (var) *var = h->h_res + (size_t)k * h->P;
-    if (pval) *pval = h->h_res + (size_t)2 * k * h->P;
+    if (beta) *beta = h->h_res.get();
+    if (var) *var = h->h_res.get() + (size_t)k * h->P;
+    if (pval) *pval = h->h_res.get() + (size_t)2 * k * h->P;
     return PG_OK;
 }
 
@@ -1816,15 +1711,15 @@ int pg_kin_mle_scan(pg_kin *h, const double *phen, int k, float *ms, const doubl
                     const double **pval) {
     if (!h || !phen || k < 1) return PG_ERR_ARG;
     pg_ctx *ctx = h->ctx;
-    if (h->m < 0) return kfail(ctx, PG_ERR_STATE, "pg_kin_mle_scan before pg_kin_eig_select / pg_kin_set_covariates");
+    if (h->m < 0) return fail(ctx, PG_ERR_STATE, "pg_kin_mle_scan before pg_kin_eig_select / pg_kin_set_covariates");
     const int n = h->n, ldg = h->ldg, m = h->m;
     if (h->minnorm || m + 2 > n)
-        return kfail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_mle_scan: %d covariates for %d pools (the n < p form of mle.rs:130-140)", m, n);
+        return fail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_mle_scan: %d covariates for %d pools (the n < p form of mle.rs:130-140)", m, n);
     if (m > pg::kKinMleMaxM)
-        return kfail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_mle_scan: %d covariates > %d (simplex of at most 16 parameters)", m, pg::kKinMleMaxM);
-    if (k > 16) return kfail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_mle_scan: %d phenotypes > 16 per call", k);
-    if ((int)h->C.size() != m * ldg) return kfail(ctx, PG_ERR_STATE, "pg_kin_mle_scan: covariates missing");
-    KCUDA(ctx, cudaSetDevice(ctx->device));
+        return fail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_mle_scan: %d covariates > %d (simplex of at most 16 parameters)", m, pg::kKinMleMaxM);
+    if (k > 16) return fail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_mle_scan: %d phenotypes > 16 per call", k);
+    if ((int)h->C.size() != m * ldg) return fail(ctx, PG_ERR_STATE, "pg_kin_mle_scan: covariates missing");
+    PG_CUDA(ctx, cudaSetDevice(ctx->device));
     const int nfix = m + 2 * m * m + k * (2 + m);
     std::vector<double> Z((size_t)(m + k) * ldg + nfix, 0.0);
     double *fix = Z.data() + (size_t)(m + k) * ldg;
@@ -1853,7 +1748,7 @@ int pg_kin_mle_scan(pg_kin *h, const double *phen, int k, float *ms, const doubl
             for (int r = c + 1; r < m; r++)
                 if (fabs(M[(size_t)r * 2 * m + c]) > fabs(M[(size_t)pr * 2 * m + c])) pr = r;
             if (!(fabs(M[(size_t)pr * 2 * m + c]) > 1e-12 * fabs(Szz[c * m + c])))
-                return kfail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_mle_scan: covariate %d is collinear with the others", c);
+                return fail(ctx, PG_ERR_UNSUPPORTED, "pg_kin_mle_scan: covariate %d is collinear with the others", c);
             for (int e = 0; e < 2 * m; e++) std::swap(M[(size_t)c * 2 * m + e], M[(size_t)pr * 2 * m + e]);
             const double piv = 1.0 / M[(size_t)c * 2 * m + c];
             for (int e = 0; e < 2 * m; e++) M[(size_t)c * 2 * m + e] *= piv;
@@ -1884,47 +1779,39 @@ int pg_kin_mle_scan(pg_kin *h, const double *phen, int k, float *ms, const doubl
             pf[2 + l] = c;
         }
     }
-    const size_t zb = Z.size() * 8;
-    if (h->mle_bytes < zb) {
-        KCUDA(ctx, cudaStreamSynchronize(h->stream));
-        cudaFree(h->d_mle);
-        h->d_mle = nullptr;
-        h->mle_bytes = 0;
-        KCUDA(ctx, cudaMalloc(&h->d_mle, zb));
-        h->mle_bytes = zb;
-    }
-    KCUDA(ctx, cudaMemcpyAsync(h->d_mle, Z.data(), zb, cudaMemcpyHostToDevice, h->stream));
-    KCUDA(ctx, cudaStreamSynchronize(h->stream));
+    PG_CUDA(ctx, h->d_mle.reserve(Z.size(), h->stream));
+    PG_CUDA(ctx, cudaMemcpyAsync(h->d_mle.get(), Z.data(), Z.size() * 8, cudaMemcpyHostToDevice, h->stream));
+    PG_CUDA(ctx, cudaStreamSynchronize(h->stream));
     if (int rc = kin_prepare_records(h, k)) return rc;
     const double df = (double)n - 1.0;
     pg::KinMleParams mp;
     memset(&mp, 0, sizeof mp);
-    mp.G = h->d_G;
+    mp.G = h->d_G.get();
     mp.P = h->P;
     mp.n = n;
     mp.ldg = ldg;
     mp.m = m;
     mp.k = k;
-    mp.Z = h->d_mle;
-    mp.fix = h->d_mle + (size_t)(m + k) * ldg;
+    mp.Z = h->d_mle.get();
+    mp.fix = h->d_mle.get() + (size_t)(m + k) * ldg;
     mp.df = df;
     mp.ln_beta = pg::statrs::ln_gamma(df / 2.0 + 0.5) - pg::statrs::ln_gamma(df / 2.0) - pg::statrs::ln_gamma(0.5);
-    mp.ptab = h->d_ptab;
+    mp.ptab = h->d_ptab.get();
     mp.ptab_isd = h->ptab_isd;
     mp.ptab_bits = h->ptab_bits;
     mp.ptab_M = h->ptab_M;
-    mp.beta = h->d_res;
-    mp.var = h->d_res + (size_t)k * h->P;
-    mp.pval = h->d_res + (size_t)2 * k * h->P;
-    KCUDA(ctx, cudaEventRecord(h->ev0, h->stream));
-    KCUDA(ctx, pg::launch_kin_mle(mp, ctx->sm_count, h->stream));
-    KCUDA(ctx, cudaEventRecord(h->ev1, h->stream));
-    KCUDA(ctx, cudaMemcpyAsync(h->h_res, h->d_res, (size_t)3 * k * h->P * 8, cudaMemcpyDeviceToHost, h->stream));
-    KCUDA(ctx, cudaStreamSynchronize(h->stream));
-    if (ms) KCUDA(ctx, cudaEventElapsedTime(ms, h->ev0, h->ev1));
-    if (beta) *beta = h->h_res;
-    if (var) *var = h->h_res + (size_t)k * h->P;
-    if (pval) *pval = h->h_res + (size_t)2 * k * h->P;
+    mp.beta = h->d_res.get();
+    mp.var = h->d_res.get() + (size_t)k * h->P;
+    mp.pval = h->d_res.get() + (size_t)2 * k * h->P;
+    PG_CUDA(ctx, cudaEventRecord(h->ev0, h->stream));
+    PG_CUDA(ctx, pg::launch_kin_mle(mp, ctx->sm_count, h->stream));
+    PG_CUDA(ctx, cudaEventRecord(h->ev1, h->stream));
+    PG_CUDA(ctx, cudaMemcpyAsync(h->h_res.get(), h->d_res.get(), (size_t)3 * k * h->P * 8, cudaMemcpyDeviceToHost, h->stream));
+    PG_CUDA(ctx, cudaStreamSynchronize(h->stream));
+    if (ms) PG_CUDA(ctx, cudaEventElapsedTime(ms, h->ev0, h->ev1));
+    if (beta) *beta = h->h_res.get();
+    if (var) *var = h->h_res.get() + (size_t)k * h->P;
+    if (pval) *pval = h->h_res.get() + (size_t)2 * k * h->P;
     return PG_OK;
 }
 

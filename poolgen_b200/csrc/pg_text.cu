@@ -245,62 +245,13 @@ __global__ void __launch_bounds__(256) text_parse_kernel(const TextParams p) {
     }
 }
 
-struct TextScratch {
-    char *d_text = nullptr;
-    size_t text_cap = 0;
-    uint32_t *d_sep = nullptr;
-    size_t sep_cap = 0;
-    uint64_t *d_tok_blk = nullptr;
-    size_t tok_cap = 0;
-    uint32_t *d_nl = nullptr, *d_first = nullptr, *d_grp = nullptr;
-    uint8_t *d_keep = nullptr;
-    uint64_t *d_line_pos = nullptr;
-    size_t line_cap = 0;
-    uint32_t *d_info = nullptr;  // [4]: n_loci, error code, error offset, n_lines
-    uint32_t *h_info = nullptr;  // pinned copy
-    void *d_tmp = nullptr;
-    size_t tmp_bytes = 0;
-    uint64_t *d_out_offset = nullptr, *d_out_pos = nullptr;
-    uint64_t *h_out_offset = nullptr, *h_out_pos = nullptr;
-    size_t out_cap = 0;
-    cudaEvent_t parsed = nullptr;
-    bool pending = false;  // text_parse_async issued, text_parse_finish not yet called
-    int64_t max_loci = 0;
-};
+TextScratch::~TextScratch() {
+    if (parsed) cudaEventDestroy(parsed);
+}
 
 // capacity with headroom: consecutive chunks of a file differ by a few lines, and a reallocation (cudaFree
 // synchronises the device) in the middle of the stream costs more than the memory
-static cudaError_t grow(void **p, size_t *cap, size_t need, size_t elem) {
-    if (*cap >= need) return cudaSuccess;
-    cudaFree(*p);
-    *p = nullptr;
-    *cap = 0;
-    const size_t want = need + need / 8 + 65536;
-    cudaError_t e = cudaMalloc(p, want * elem);
-    if (e == cudaSuccess) *cap = want;
-    return e;
-}
-
-void text_scratch_free(TextScratch *t) {
-    if (!t) return;
-    cudaFree(t->d_text);
-    cudaFree(t->d_sep);
-    cudaFree(t->d_tok_blk);
-    cudaFree(t->d_nl);
-    cudaFree(t->d_keep);
-    cudaFree(t->d_first);
-    cudaFree(t->d_grp);
-    cudaFree(t->d_line_pos);
-    cudaFree(t->d_info);
-    cudaFree(t->d_tmp);
-    cudaFree(t->d_out_offset);
-    cudaFree(t->d_out_pos);
-    if (t->h_info) cudaFreeHost(t->h_info);
-    if (t->h_out_offset) cudaFreeHost(t->h_out_offset);
-    if (t->h_out_pos) cudaFreeHost(t->h_out_pos);
-    if (t->parsed) cudaEventDestroy(t->parsed);
-    delete t;
-}
+static size_t with_headroom(size_t need) { return need + need / 8 + 65536; }
 
 #define TCK(call)                      \
     do {                               \
@@ -316,116 +267,84 @@ static cudaError_t text_parse_enqueue(TextScratch *t, const char *text, size_t n
                                       int64_t max_loci, size_t line_cap, int sm_count, cudaStream_t s) {
     t->max_loci = max_loci;
     if (!t->parsed) TCK(cudaEventCreateWithFlags(&t->parsed, cudaEventDisableTiming));
-    if (!t->d_info) {
-        TCK(cudaMalloc(&t->d_info, 16));
-        TCK(cudaHostAlloc((void **)&t->h_info, 16, cudaHostAllocDefault));
-    }
-    TCK(cudaMemsetAsync(t->d_info, 0, 16, s));
+    TCK(t->d_info.reserve(4, s));
+    TCK(t->h_info.reserve(4, s));
+    TCK(cudaMemsetAsync(t->d_info.get(), 0, 16, s));
     if (n_bytes >= 0xFFFFFFF0ull) return cudaErrorInvalidValue;
     if (n_bytes == 0) {
-        TCK(cudaMemcpyAsync(t->h_info, t->d_info, 16, cudaMemcpyDeviceToHost, s));
+        TCK(cudaMemcpyAsync(t->h_info.get(), t->d_info.get(), 16, cudaMemcpyDeviceToHost, s));
         return cudaEventRecord(t->parsed, s);
     }
     const bool add_nl = text[n_bytes - 1] != '\n';  // a last line without its newline
     const size_t nb = n_bytes + (add_nl ? 1 : 0);
     if (line_cap == 0) line_cap = (size_t)max_loci + (size_t)max_loci / 4 + 4096;
     if (line_cap > nb) line_cap = nb;
-    TCK(grow((void **)&t->d_text, &t->text_cap, nb + 32, 1));
-    TCK(cudaMemcpyAsync(t->d_text, text, n_bytes, cudaMemcpyHostToDevice, s));
-    if (add_nl) TCK(cudaMemsetAsync(t->d_text + n_bytes, '\n', 1, s));
+    if (t->d_text.capacity() < nb + 32) TCK(t->d_text.reserve(with_headroom(nb + 32), s));
+    TCK(cudaMemcpyAsync(t->d_text.get(), text, n_bytes, cudaMemcpyHostToDevice, s));
+    if (add_nl) TCK(cudaMemsetAsync(t->d_text.get() + n_bytes, '\n', 1, s));
     const size_t n_tok = (nb + kTokBlock - 1) / kTokBlock;
     const size_t n_grp = (line_cap + kLineGroup - 1) / kLineGroup;
-    TCK(grow((void **)&t->d_sep, &t->sep_cap, nb, 4));  // worst case: every byte is a separator
-    TCK(grow((void **)&t->d_tok_blk, &t->tok_cap, n_tok + 1, 8));
-    if (t->line_cap < line_cap) {
-        cudaFree(t->d_nl);
-        cudaFree(t->d_keep);
-        cudaFree(t->d_first);
-        cudaFree(t->d_grp);
-        cudaFree(t->d_line_pos);
-        t->d_nl = t->d_first = t->d_grp = nullptr;
-        t->d_keep = nullptr;
-        t->d_line_pos = nullptr;
-        t->line_cap = 0;
-        TCK(cudaMalloc(&t->d_nl, line_cap * 4));
-        TCK(cudaMalloc(&t->d_keep, line_cap));
-        TCK(cudaMalloc(&t->d_first, line_cap * 4));
-        TCK(cudaMalloc(&t->d_line_pos, line_cap * 8));
-        TCK(cudaMalloc(&t->d_grp, (n_grp + 2) * 4));
-        t->line_cap = line_cap;
-    }
-    if (t->out_cap < (size_t)max_loci) {
-        cudaFree(t->d_out_offset);
-        cudaFree(t->d_out_pos);
-        if (t->h_out_offset) cudaFreeHost(t->h_out_offset);
-        if (t->h_out_pos) cudaFreeHost(t->h_out_pos);
-        t->d_out_offset = t->d_out_pos = nullptr;
-        t->h_out_offset = t->h_out_pos = nullptr;
-        t->out_cap = 0;
-        TCK(cudaMalloc(&t->d_out_offset, (size_t)max_loci * 8));
-        TCK(cudaMalloc(&t->d_out_pos, (size_t)max_loci * 8));
-        TCK(cudaHostAlloc((void **)&t->h_out_offset, (size_t)max_loci * 8, cudaHostAllocDefault));
-        TCK(cudaHostAlloc((void **)&t->h_out_pos, (size_t)max_loci * 8, cudaHostAllocDefault));
-        t->out_cap = (size_t)max_loci;
-    }
+    if (t->d_sep.capacity() < nb) TCK(t->d_sep.reserve(with_headroom(nb), s));  // worst case: every byte is a separator
+    if (t->d_tok_blk.capacity() < n_tok + 1) TCK(t->d_tok_blk.reserve(with_headroom(n_tok + 1), s));
+    // the per-line arrays are sized for exactly line_cap lines
+    TCK(t->d_nl.reserve(line_cap, s));
+    TCK(t->d_keep.reserve(line_cap, s));
+    TCK(t->d_first.reserve(line_cap, s));
+    TCK(t->d_line_pos.reserve(line_cap, s));
+    TCK(t->d_grp.reserve(n_grp + 2, s));
+    TCK(t->d_out_offset.reserve((size_t)max_loci, s));
+    TCK(t->d_out_pos.reserve((size_t)max_loci, s));
+    TCK(t->h_out_offset.reserve((size_t)max_loci, s));
+    TCK(t->h_out_pos.reserve((size_t)max_loci, s));
     size_t tmp1 = 0, tmp2 = 0;
     cub::DeviceScan::ExclusiveSum(nullptr, tmp1, (uint64_t *)nullptr, (uint64_t *)nullptr, (int)(n_tok + 1), s);
     cub::DeviceScan::ExclusiveSum(nullptr, tmp2, (uint32_t *)nullptr, (uint32_t *)nullptr, (int)(n_grp + 1), s);
-    const size_t tmp = std::max(tmp1, tmp2);
-    if (t->tmp_bytes < tmp) {
-        cudaFree(t->d_tmp);
-        t->d_tmp = nullptr;
-        t->tmp_bytes = 0;
-        TCK(cudaMalloc(&t->d_tmp, tmp));
-        t->tmp_bytes = tmp;
-    }
+    TCK(t->d_tmp.reserve(std::max(tmp1, tmp2), s));
     TextParams tp;
-    tp.text = t->d_text;
+    tp.text = t->d_text.get();
     tp.n_bytes = (uint32_t)nb;
-    tp.sep = t->d_sep;
-    tp.nl = t->d_nl;
-    tp.tok_blk = t->d_tok_blk;
+    tp.sep = t->d_sep.get();
+    tp.nl = t->d_nl.get();
+    tp.tok_blk = t->d_tok_blk.get();
     tp.n_tok_blocks = (uint32_t)n_tok;
     tp.line_cap = (uint32_t)line_cap;
     tp.max_loci = (uint32_t)std::min<int64_t>(max_loci, 0xFFFFFFFFll);
     tp.n_pools = n_pools;
-    tp.keep = t->d_keep;
-    tp.first_sep = t->d_first;
-    tp.line_pos = t->d_line_pos;
-    tp.grp = t->d_grp;
+    tp.keep = t->d_keep.get();
+    tp.first_sep = t->d_first.get();
+    tp.line_pos = t->d_line_pos.get();
+    tp.grp = t->d_grp.get();
     tp.n_groups_max = (uint32_t)n_grp;
     tp.counts = d_counts;
-    tp.out_offset = t->d_out_offset;
-    tp.out_pos = t->d_out_pos;
-    tp.info = t->d_info;
+    tp.out_offset = t->d_out_offset.get();
+    tp.out_pos = t->d_out_pos.get();
+    tp.info = t->d_info.get();
     const int grid_tok = (int)std::min<size_t>(n_tok, (size_t)sm_count * 16);
-    TCK(cudaMemsetAsync(t->d_tok_blk + n_tok, 0, 8, s));
+    TCK(cudaMemsetAsync(t->d_tok_blk.get() + n_tok, 0, 8, s));
     tok_count_kernel<<<grid_tok, kTokThreads, 0, s>>>(tp);
     TCK(cudaGetLastError());
-    size_t tb = t->tmp_bytes;
-    TCK(cub::DeviceScan::ExclusiveSum(t->d_tmp, tb, t->d_tok_blk, t->d_tok_blk, (int)(n_tok + 1), s));
+    size_t tb = t->d_tmp.capacity();
+    TCK(cub::DeviceScan::ExclusiveSum(t->d_tmp.get(), tb, t->d_tok_blk.get(), t->d_tok_blk.get(), (int)(n_tok + 1), s));
     tok_scatter_kernel<<<grid_tok, kTokThreads, 0, s>>>(tp);
     TCK(cudaGetLastError());
-    TCK(cudaMemsetAsync(t->d_grp, 0, (n_grp + 2) * 4, s));
+    TCK(cudaMemsetAsync(t->d_grp.get(), 0, (n_grp + 2) * 4, s));
     const int grid_lines = (int)std::min<size_t>(n_grp, (size_t)sm_count * 8);
     text_lines_kernel<<<grid_lines, kLineGroup, 0, s>>>(tp);
     TCK(cudaGetLastError());
-    tb = t->tmp_bytes;
-    TCK(cub::DeviceScan::ExclusiveSum(t->d_tmp, tb, t->d_grp, t->d_grp, (int)(n_grp + 1), s));
+    tb = t->d_tmp.capacity();
+    TCK(cub::DeviceScan::ExclusiveSum(t->d_tmp.get(), tb, t->d_grp.get(), t->d_grp.get(), (int)(n_grp + 1), s));
     const int grid_parse = (int)std::min<uint64_t>(((uint64_t)line_cap * 32 + 255) / 256, (uint64_t)sm_count * 8);
     text_parse_kernel<<<grid_parse, 256, 0, s>>>(tp);
     TCK(cudaGetLastError());
-    TCK(cudaMemcpyAsync(t->h_info, t->d_info, 16, cudaMemcpyDeviceToHost, s));
+    TCK(cudaMemcpyAsync(t->h_info.get(), t->d_info.get(), 16, cudaMemcpyDeviceToHost, s));
     return cudaEventRecord(t->parsed, s);
 }
 #undef TCK
 
 // a slab is 'pending' only once everything up to the `parsed` event has been enqueued: a failed allocation or launch
 // must not leave text_parse_finish waiting on a stale event and trusting the previous chunk's h_info
-cudaError_t text_parse_async(TextScratch **scratch, const char *text, size_t n_bytes, int n_pools, uint32_t *d_counts,
+cudaError_t text_parse_async(TextScratch *t, const char *text, size_t n_bytes, int n_pools, uint32_t *d_counts,
                              int64_t max_loci, size_t line_cap, int sm_count, cudaStream_t s) {
-    if (!*scratch) *scratch = new TextScratch();
-    TextScratch *t = *scratch;
     t->pending = false;
     const cudaError_t e = text_parse_enqueue(t, text, n_bytes, n_pools, d_counts, max_loci, line_cap, sm_count, s);
     t->pending = (e == cudaSuccess);
@@ -437,22 +356,24 @@ cudaError_t text_parse_async(TextScratch **scratch, const char *text, size_t n_b
 // than the per-line arrays hold (*err_offset = the number of lines: repeat with that line_cap).  On success the copy
 // of the labels (line offsets, positions) to pinned host memory is enqueued on s.
 int64_t text_parse_finish(TextScratch *t, cudaStream_t s, cudaError_t *cuda_err, uint64_t *err_offset) {
-    if (!t || !t->pending) return 0;
+    if (!t->pending) return 0;
     t->pending = false;
     cudaError_t e = cudaEventSynchronize(t->parsed);
     if (e != cudaSuccess) {
         *cuda_err = e;
         return -1;
     }
-    const uint32_t n_loci = t->h_info[0], code = t->h_info[1];
-    *err_offset = t->h_info[2];
+    const uint32_t *info = t->h_info.get();
+    const uint32_t n_loci = info[0], code = info[1];
+    *err_offset = info[2];
     if (code == TEXT_ERR_LINES) return -5;
     if (code == TEXT_ERR_POOLS) return -3;
     if (code == TEXT_ERR_FIELD) return -4;
     if (code == TEXT_ERR_LOCI || (int64_t)n_loci > t->max_loci) return -2;
     if (n_loci == 0) return 0;
-    e = cudaMemcpyAsync(t->h_out_offset, t->d_out_offset, (size_t)n_loci * 8, cudaMemcpyDeviceToHost, s);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(t->h_out_pos, t->d_out_pos, (size_t)n_loci * 8, cudaMemcpyDeviceToHost, s);
+    e = cudaMemcpyAsync(t->h_out_offset.get(), t->d_out_offset.get(), (size_t)n_loci * 8, cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess)
+        e = cudaMemcpyAsync(t->h_out_pos.get(), t->d_out_pos.get(), (size_t)n_loci * 8, cudaMemcpyDeviceToHost, s);
     if (e != cudaSuccess) {
         *cuda_err = e;
         return -1;
@@ -460,9 +381,18 @@ int64_t text_parse_finish(TextScratch *t, cudaStream_t s, cudaError_t *cuda_err,
     return (int64_t)n_loci;
 }
 
-bool text_parse_pending(const TextScratch *t) { return t && t->pending; }
-
-const uint64_t *text_offsets(const TextScratch *t) { return t ? t->h_out_offset : nullptr; }
-const uint64_t *text_positions(const TextScratch *t) { return t ? t->h_out_pos : nullptr; }
+int text_parse_fail(pg_ctx *ctx, const char *who, int64_t status, cudaError_t cuda_err, uint64_t err_offset,
+                    int n_pools, int64_t cap) {
+    const unsigned long long at = err_offset;
+    if (status == -1) return fail(ctx, PG_ERR_CUDA, "%s: %s", who, cudaGetErrorString(cuda_err));
+    if (status == -2) return fail(ctx, PG_ERR_ARG, "%s: more loci in the chunk than the capacity %lld", who, (long long)cap);
+    if (status == -3)
+        return fail(ctx, PG_ERR_ARG, "%s: the line at byte %llu does not hold %d pools (the reference asserts the pool count, "
+                                     "src/base/sync.rs:254-257)", who, at, n_pools);
+    if (status == -4)
+        return fail(ctx, PG_ERR_ARG, "%s: malformed pool field at byte %llu (the reference panics: allele counts are not "
+                                     "valid integers, src/base/sync.rs:146)", who, at);
+    return fail(ctx, PG_ERR_ARG, "%s: the chunk could not be parsed (%lld)", who, (long long)status);
+}
 
 }  // namespace pg
