@@ -126,6 +126,9 @@ extern "C" {
     pub fn pg_kin_last_labels(kin: *mut pg_kin, n_cols: i64, col_locus: *mut i64, col_allele: *mut u8) -> c_int;
     pub fn pg_kin_append_sync_text(kin: *mut pg_kin, filter: *const pg_filter, text: *const c_char, n_bytes: usize, max_loci: i64, keep_p_minus_1: c_int, n_loci: *mut i64, n_cols_added: *mut i64) -> c_int;
     pub fn pg_kin_text_labels(kin: *mut pg_kin, line_offsets: *mut *const u64, positions: *mut *const u64) -> c_int;
+    /// sync2csv rows of columns [first, first + count) of the last text append, formatted on the device; stops at
+    /// the last whole row that fits `capacity` (see pg_kin_format_frequency_rows in poolgen_cuda.h)
+    pub fn pg_kin_format_frequency_rows(kin: *mut pg_kin, first: i64, count: i64, out: *mut c_char, capacity: usize, n_bytes: *mut usize, n_rows: *mut i64) -> c_int;
     pub fn pg_kin_synth(kin: *mut pg_kin, seed: u64, first_locus: i64, n_loci: i64) -> c_int;
     pub fn pg_kin_get_columns(kin: *mut pg_kin, first: i64, count: i64, out: *mut f64) -> c_int;
     pub fn pg_kin_gram(kin: *mut pg_kin) -> c_int;

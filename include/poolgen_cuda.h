@@ -202,6 +202,17 @@ int pg_kin_last_labels(pg_kin *kin, int64_t n_cols, int64_t *col_locus, uint8_t 
 int pg_kin_append_sync_text(pg_kin *kin, const pg_filter *filter, const char *text, size_t n_bytes, int64_t max_loci,
                             int keep_p_minus_1, int64_t *n_loci, int64_t *n_cols_added);
 int pg_kin_text_labels(pg_kin *kin, const uint64_t **line_offsets, const uint64_t **positions);
+/* sync2csv rows formatted on the device from the columns the LAST pg_kin_append_sync_text added (column 0 = its first
+ * column): columns [first, first + count), one row each, equal byte for byte to pg_format_frequency_rows over the same
+ * columns, their pg_kin_last_labels and the text labels of that append with locus_order = NULL
+ * (`chr,pos,allele,f_1,...,f_n\n`, every f through parse_f64_roundup_and_own(x, 6)).  The rows are copied to `out`
+ * (pinned host memory for a full-rate copy); the call stops at the last whole row that fits `capacity` and returns the
+ * rows done and their bytes, so a caller continues at first + *n_rows.  A capacity below one row is PG_ERR_ARG.
+ * PG_ERR_STATE when the last append (or a reset) was not from text; PG_ERR_UNSUPPORTED, nothing written, when a value
+ * of the range is infinite or has |x * 1e6| >= 9e14 (the loader's frequencies never do; pg_format_frequency_rows prints
+ * them).  Synchronises the handle's stream. */
+int pg_kin_format_frequency_rows(pg_kin *kin, int64_t first, int64_t count, char *out, size_t capacity, size_t *n_bytes,
+                                 int64_t *n_rows);
 /* synthetic biallelic columns (two per locus) generated on the device from the integer-hash workload */
 int pg_kin_synth(pg_kin *kin, uint64_t seed, int64_t first_locus, int64_t n_loci);
 int pg_kin_get_columns(pg_kin *kin, int64_t first, int64_t count, double *out /* [count][n_pools] */);

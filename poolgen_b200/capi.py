@@ -35,7 +35,7 @@ ABI_SYMBOLS = [
     "pg_batch_bytes", "pg_scan_stream_begin", "pg_scan_submit_counts", "pg_scan_submit_counts_u16",
     "pg_scan_submit_counts_u8", "pg_scan_submit_freq", "pg_scan_collect", "pg_scan_text_labels",
     "pg_kin_open", "pg_kin_close", "pg_kin_reset", "pg_kin_columns", "pg_kin_append_columns", "pg_kin_append_counts",
-    "pg_kin_last_labels", "pg_kin_append_sync_text", "pg_kin_text_labels", "pg_kin_synth", "pg_kin_get_columns", "pg_kin_gram", "pg_kin_gram_accumulate", "pg_kin_gram_time", "pg_kin_partial",
+    "pg_kin_last_labels", "pg_kin_append_sync_text", "pg_kin_text_labels", "pg_kin_format_frequency_rows", "pg_kin_synth", "pg_kin_get_columns", "pg_kin_gram", "pg_kin_gram_accumulate", "pg_kin_gram_time", "pg_kin_partial",
     "pg_kin_partial_get", "pg_kin_partial_set", "pg_kin_eig_select", "pg_kin_eigvals", "pg_kin_set_covariates",
     "pg_kin_covar_scan", "pg_kin_mle_scan", "pg_format_header", "pg_format_rows", "pg_format_rows_ex", "pg_format_kinship_rows", "pg_format_f64", "pg_sort_loci",
     "pg_format_frequency_header", "pg_format_frequency_rows",
@@ -139,6 +139,7 @@ def lib():
             "pg_kin_last_labels": (i, [vp, i64, vp, vp]),
             "pg_kin_append_sync_text": (i, [vp, C.POINTER(_Filter), vp, C.c_size_t, i64, i, C.POINTER(i64), C.POINTER(i64)]),
             "pg_kin_text_labels": (i, [vp, pvp, pvp]),
+            "pg_kin_format_frequency_rows": (i, [vp, i64, i64, vp, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(i64)]),
             "pg_kin_synth": (i, [vp, u64, i64, i64]),
             "pg_kin_get_columns": (i, [vp, i64, i64, vp]),
             "pg_kin_gram": (i, [vp]),
@@ -658,6 +659,15 @@ class Kinship:
         alle = np.empty(n_add, dtype=np.uint8)
         self._ck(lib().pg_kin_last_labels(self._h, n_add, loc.ctypes.data, alle.ctypes.data), "pg_kin_last_labels")
         return L, off, pos, loc, alle
+
+    def format_frequency_rows(self, first: int, count: int, out) -> tuple:
+        """sync2csv rows of columns [first, first + count) of the last append_sync_text, formatted on the device into
+        `out` (a writable uint8 array, ideally Context.pinned_empty): returns (bytes, rows) of the whole rows that fit"""
+        assert out.dtype == np.uint8 and out.flags["C_CONTIGUOUS"] and out.flags["WRITEABLE"]
+        nb, nr = C.c_size_t(), C.c_int64()
+        self._ck(lib().pg_kin_format_frequency_rows(self._h, int(first), int(count), out.ctypes.data, out.size,
+                                                    C.byref(nb), C.byref(nr)), "pg_kin_format_frequency_rows")
+        return int(nb.value), int(nr.value)
 
     def synth(self, seed: int, first_locus: int, n_loci: int):
         self._ck(lib().pg_kin_synth(self._h, int(seed), int(first_locus), int(n_loci)), "pg_kin_synth")

@@ -45,6 +45,16 @@ struct pg_kin {
     pg::DeviceBuffer<uint32_t> d_counts;
     pg::DeviceBuffer<double> d_w;
     pg::TextScratch text;  // sync text parsed on the device (pg_kin_append_sync_text)
+    // the columns the last append took from sync text: [text_first, text_first + text_cols); text_cols = -1 when the
+    // last append (or reset) was anything else
+    int64_t text_first = 0, text_cols = -1;
+    // sync2csv rows formatted on the device (pg_fmt.cu)
+    pg::DeviceBuffer<uint64_t> d_fmt_off;   // [rows + 1] row lengths, then their exclusive scan
+    pg::DeviceBuffer<uint32_t> d_fmt_chr;   // [rows] chromosome bytes
+    pg::DeviceBuffer<uint8_t> d_fmt_tmp;    // scan scratch
+    pg::DeviceBuffer<unsigned long long> d_fmt_info;
+    pg::PinnedBuffer<unsigned long long> h_fmt_info;
+    pg::DeviceBuffer<char> d_fmt_text;      // the rows of one call
     // eigen step: cuSOLVER is mapped and its handle created by a background thread started in pg_kin_open and joined
     // by pg_kin_eig_select / the destructor
     std::thread warm;

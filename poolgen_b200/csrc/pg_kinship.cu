@@ -1020,6 +1020,7 @@ int pg_kin_reset(pg_kin *h) {
     PG_CUDA(h->ctx, cudaMemsetAsync(h->d_G.get(), 0, h->d_G.capacity() * 8, h->stream));
     h->P = 0;
     h->P_total = 0;
+    h->text_cols = -1;
     return PG_OK;
 }
 
@@ -1031,6 +1032,7 @@ int pg_kin_append_columns(pg_kin *h, const double *cols, int64_t P_add) {
     if (h->P + P_add > h->cap) return fail(ctx, PG_ERR_ARG, "pg_kin_append_columns: %lld + %lld columns > capacity %lld",
                                             (long long)h->P, (long long)P_add, (long long)h->cap);
     PG_CUDA(ctx, cudaSetDevice(ctx->device));
+    h->text_cols = -1;
     if (P_add == 0) return PG_OK;
     PG_CUDA(ctx, cudaMemcpy2DAsync(h->d_G.get() + (size_t)h->P * h->ldg, (size_t)h->ldg * 8, cols, (size_t)h->n * 8,
                                  (size_t)h->n * 8, (size_t)P_add, cudaMemcpyHostToDevice, h->stream));
@@ -1117,6 +1119,7 @@ int pg_kin_append_counts(pg_kin *h, const pg_filter *filter, int n_alleles, cons
     if (filter->n_pool_sizes != h->n || !filter->pool_sizes)
         return fail(ctx, PG_ERR_ARG, "pg_kin_append_counts: %d pool sizes for %d pools", filter->n_pool_sizes, h->n);
     PG_CUDA(ctx, cudaSetDevice(ctx->device));
+    h->text_cols = -1;
     if (n_cols_added) *n_cols_added = 0;
     if (n_loci == 0) return PG_OK;
     int rc = kin_reserve(h, n_loci, n_alleles);
@@ -1135,6 +1138,7 @@ int pg_kin_append_sync_text(pg_kin *h, const pg_filter *filter, const char *text
     if (filter->n_pool_sizes != h->n || !filter->pool_sizes)
         return fail(ctx, PG_ERR_ARG, "pg_kin_append_sync_text: %d pool sizes for %d pools", filter->n_pool_sizes, h->n);
     PG_CUDA(ctx, cudaSetDevice(ctx->device));
+    h->text_cols = -1;
     if (n_cols_added) *n_cols_added = 0;
     if (n_loci_out) *n_loci_out = 0;
     int rc = kin_reserve(h, max_loci, 6);
@@ -1152,9 +1156,16 @@ int pg_kin_append_sync_text(pg_kin *h, const pg_filter *filter, const char *text
     }
     if (L < 0) return pg::text_parse_fail(ctx, "pg_kin_append_sync_text", L, ce, at, h->n, max_loci);
     if (n_loci_out) *n_loci_out = L;
-    if (L == 0) return PG_OK;
-    static const uint8_t sync_codes[6] = {0, 1, 2, 3, 4, 5};
-    return kin_load_resident(h, filter, 6, sync_codes, L, keep_p_minus_1, n_cols_added, "pg_kin_append_sync_text");
+    int64_t added = 0;
+    if (L > 0) {
+        static const uint8_t sync_codes[6] = {0, 1, 2, 3, 4, 5};
+        rc = kin_load_resident(h, filter, 6, sync_codes, L, keep_p_minus_1, &added, "pg_kin_append_sync_text");
+        if (rc) return rc;
+    }
+    if (n_cols_added) *n_cols_added = added;
+    h->text_first = h->P - added;  // pg_kin_format_frequency_rows formats these columns
+    h->text_cols = added;
+    return PG_OK;
 }
 
 int pg_kin_text_labels(pg_kin *h, const uint64_t **line_offsets, const uint64_t **positions) {
@@ -1180,6 +1191,7 @@ int pg_kin_synth(pg_kin *h, uint64_t seed, int64_t first_locus, int64_t n_loci) 
     pg_ctx *ctx = h->ctx;
     if (h->P + 2 * n_loci > h->cap) return fail(ctx, PG_ERR_ARG, "pg_kin_synth: capacity");
     PG_CUDA(ctx, cudaSetDevice(ctx->device));
+    h->text_cols = -1;
     if (n_loci == 0) return PG_OK;
     const int grid = (int)std::min<int64_t>((n_loci * h->ldg + 255) / 256, (int64_t)ctx->sm_count * 16);
     pg::kin_synth_kernel<<<grid, 256, 0, h->stream>>>(seed, first_locus, n_loci, h->n, h->ldg,

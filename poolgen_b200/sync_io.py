@@ -12,6 +12,7 @@ import ctypes as C
 import os
 import threading
 import time
+from concurrent.futures import ThreadPoolExecutor
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -293,21 +294,6 @@ class _LoadedColumns:
     positions: np.ndarray  # uint64 [L]
 
 
-def _load_all(ctx: Context, fname: str, n_pools: int, fs: FilterStats, keep_p_minus_1: bool, max_columns: int,
-              block_bytes: int) -> _LoadedColumns:
-    """LoadAll::load over the whole file, block by block through the device parser and loader"""
-    kin = capi.Kinship(ctx, n_pools, max_columns)
-    max_loci = block_bytes // _line_min_bytes(n_pools) + 2
-    lab = _Labels()
-    try:
-        for _, block in _text_blocks(fname, block_bytes):
-            lab.add(block, *kin.append_sync_text(block, fs, max_loci, keep_p_minus_1))
-    except Exception:
-        kin.close()
-        raise
-    return lab.finish(kin)
-
-
 # ---- columns beyond one device: the handle holds a device block of columns at a time -------------------------------
 _COLS_PER_LINE = 6  # a locus emits at most six allele columns (--keep-ns with MAF 0 and no --keep-p-minus-1)
 _KIN_RESERVE_BYTES = 1 << 30  # outside the handle: cuSOLVER's and cuBLAS' handles, kernel modules loaded on first use
@@ -428,32 +414,162 @@ def _count_columns_bound(fname: str) -> int:
     return _COLS_PER_LINE * lines
 
 
+_FMT_CHUNK_BYTES = 16 << 20  # rows per device formatter call: each of the two pinned buffers holds this many bytes
+
+
+def _kept_lines(block: bytes, at: int, off, pos, loc, names: list, index_of: dict):
+    """pass 1 of sync2csv over one text block: for every locus that emitted columns, the absolute byte offset of its
+    line, the bytes pass 2 gathers for it (its line, plus a newline where the file's last line has none), its
+    chromosome index, its position and its column count"""
+    keep, cols = np.unique(loc, return_counts=True)  # the loader emits columns grouped by ascending locus
+    o = off[keep].astype(np.int64)
+    buf = np.frombuffer(block, dtype=np.uint8)
+    nl = np.flatnonzero(buf == 10)
+    k = np.searchsorted(nl, o)
+    ends = nl[np.minimum(k, nl.size - 1)] + 1 if nl.size else np.zeros(o.size, np.int64)
+    ends = np.where(k < nl.size, ends, len(block))
+    size = ends - o + (ends == len(block)) * int(not block.endswith(b"\n"))
+    tabs = np.flatnonzero(buf == 9)
+    tab = tabs[np.searchsorted(tabs, o)]  # a locus line holds tabs
+    chr_idx = np.empty(o.size, dtype=np.uint32)
+    for j, (a, b) in enumerate(zip(o.tolist(), tab.tolist())):
+        nm = block[a:b]
+        if nm not in index_of:
+            index_of[nm] = len(names)
+            names.append(nm)
+        chr_idx[j] = index_of[nm]
+    return at + o, size, chr_idx, pos[keep], cols
+
+
 def write_csv(self, ctx: Context, filter_stats: FilterStats, keep_p_minus_1: bool, out: str, n_threads: int,
-              block_bytes: int = 32 << 20) -> str:
+              block_bytes: int = 32 << 20, timings: dict = None) -> str:
     """sync2csv: `SaveCsv::write_csv(&self, &FilterStats, keep_p_minus_1, out, n_threads)` of FileSyncPhen
     (src/base/sync.rs:1182-1262): header `#chr,pos,allele,<pool names>`, one row per kept allele of every kept locus,
-    loci in LoadAll's order (stable by chromosome, position), frequencies through parse_f64_roundup_and_own(x, 6)"""
+    loci in LoadAll's order (stable by chromosome, position), frequencies through parse_f64_roundup_and_own(x, 6).
+
+    One code path for any file size; the kinship handle holds one text block's columns at most.  Pass 1 loads every
+    text block on the device and keeps, per locus that emits columns, where its line is, its chromosome, position and
+    column count; no column leaves the device.  The loci are sorted on the host (pg_sort_loci).  Pass 2 gathers the
+    kept lines in that order into line-aligned blocks of at most block_bytes (contiguous runs of the file in one
+    read), loads each block again, checks that every line gives its pass-1 column count, and formats the rows on the
+    device into two pinned buffers in turn; a writer thread writes one while the next is formatted.  The rows of a
+    block are the sorted loci's rows: within a locus, the columns keep the loader's order.
+    `timings` (measurement only): filled with wall seconds per phase."""
     if out == "":
         bname = ".".join(self.filename_sync.split(".")[:-1])
         out = f"{bname}-{time.time()}-allele_frequencies.csv"
     if os.path.exists(out):
         raise PgError("Cannot write to output file")
-    ld = _load_all(ctx, self.filename_sync, len(self.pool_names), filter_stats, keep_p_minus_1,
-                   _count_columns_bound(self.filename_sync), block_bytes)
+    fname = self.filename_sync
+    n = len(self.pool_names)
+    max_loci = block_bytes // _line_min_bytes(n) + 2
+    clock = time.perf_counter
+    tm = {"pass1_s": 0.0, "sort_s": 0.0, "gather_s": 0.0, "parse_s": 0.0, "format_s": 0.0, "write_wait_s": 0.0}
+    kin = capi.Kinship(ctx, n, text_block_columns(block_bytes, n))
+    pinned = []
     try:
-        if ld.col_locus.size == 0:
+        t0 = clock()
+        names, index_of, parts = [], {}, []
+        for at, block in _text_blocks(fname, block_bytes):
+            kin.reset()
+            _L, off, pos, loc, _alle = kin.append_sync_text(block, filter_stats, max_loci, keep_p_minus_1)
+            if loc.size:
+                parts.append(_kept_lines(block, at, off, pos, loc, names, index_of))
+        if not parts:
             raise PgError("No data passed the filtering variables. Please decrease minimum depth, and/or minimum "
                           "allele frequency.")  # assert at src/base/sync.rs:1219
-        G = ld.kin.get_columns(0, ld.kin.columns)
+        line_at, size, chr_idx, positions, cols = (np.concatenate(x) for x in zip(*parts))
+        del parts
+        tm["pass1_s"] = clock() - t0
+        t0 = clock()
+        order = capi.sort_loci(positions, chr_names=names, chr_index=chr_idx)
+        line_at, size, positions, cols = line_at[order], size[order], positions[order], cols[order]
+        tm["sort_s"] = clock() - t0
+        row_max = max(len(nm) for nm in names) + 25 + 19 * n  # chr,pos,allele + n numbers of at most 19 bytes + newline
+        bufs = []
+        for _ in range(2):
+            arr, h = ctx.pinned_empty((max(_FMT_CHUNK_BYTES, row_max),), np.uint8)
+            pinned.append(h)
+            bufs.append(arr)
+        _sync2csv_pass2(kin, fname, out, self.pool_names, filter_stats, keep_p_minus_1, block_bytes, max_loci,
+                        line_at, size, positions, cols, bufs, tm)
     finally:
-        ld.kin.close()
-    order = capi.sort_loci(ld.positions, chr_names=ld.chr_names, chr_index=ld.chr_index)
-    rows = capi.format_frequency_rows(G, ld.col_locus, ld.col_allele, ld.positions, locus_order=order,
-                                      n_threads=max(1, n_threads), chr_names=ld.chr_names, chr_index=ld.chr_index)
-    with open(out, "xb") as fo:
-        fo.write(capi.format_frequency_header(self.pool_names))
-        fo.write(rows)
+        kin.close()
+        for h in pinned:
+            ctx.pinned_free(h)
+    if timings is not None:
+        timings.update(tm, loci=int(cols.size), columns=int(cols.sum()))
     return out
+
+
+def _sync2csv_pass2(kin, fname, out, pool_names, fs, keep_p_minus_1, block_bytes, max_loci, line_at, size, positions,
+                    cols, bufs, tm):
+    """pass 2 of write_csv over the loci in output order; the output file is removed again if anything fails"""
+    clock = time.perf_counter
+    cum = np.cumsum(size)
+    # the lines [i, j) of a run are contiguous in the file
+    brk = np.flatnonzero(line_at[1:] != line_at[:-1] + size[:-1]) + 1
+    writer = ThreadPoolExecutor(max_workers=1)
+    pending = [None, None]
+    fo = open(out, "xb")
+    try:
+        fo.write(capi.format_frequency_header(pool_names))
+        with open(fname, "rb") as fh:
+            i, N, b = 0, int(size.size), 0
+            while i < N:
+                t0 = clock()
+                j = int(np.searchsorted(cum, (cum[i - 1] if i else 0) + block_bytes, side="right"))
+                if j == i:
+                    raise PgError(f"a line of {fname} is longer than the block size {block_bytes}")
+                block = bytearray()
+                starts = [i] + brk[np.searchsorted(brk, i, side="right"):np.searchsorted(brk, j)].tolist() + [j]
+                for s, e in zip(starts[:-1], starts[1:]):
+                    want = int(line_at[e - 1] + size[e - 1] - line_at[s])
+                    fh.seek(int(line_at[s]))
+                    data = fh.read(want)
+                    if len(data) == want - 1 and not data.endswith(b"\n") and not fh.read(1):
+                        data += b"\n"  # the file's last line, which has no newline
+                    if len(data) != want:
+                        raise PgError(f"{fname} changed between passes: {len(data)} of the {want} bytes at offset "
+                                      f"{int(line_at[s])}")
+                    block += data
+                tm["gather_s"] += clock() - t0
+                t0 = clock()
+                kin.reset()
+                try:
+                    L, _off, pos, loc, _alle = kin.append_sync_text(block, fs, max_loci, keep_p_minus_1)
+                except PgError as e:  # these lines parsed in pass 1
+                    raise PgError(f"{fname} changed between passes: {e}") from None
+                tm["parse_s"] += clock() - t0
+                got = np.bincount(loc, minlength=L) if loc.size else np.zeros(L, np.int64)
+                if L != j - i or not np.array_equal(got, cols[i:j]) or not np.array_equal(pos, positions[i:j]):
+                    raise PgError(f"{fname} changed between passes: the {j - i} kept lines from offset "
+                                  f"{int(line_at[i])} on no longer give the loci and columns of pass 1")
+                P, first = int(loc.size), 0
+                while first < P:
+                    if pending[b] is not None:
+                        t0 = clock()
+                        pending[b].result()
+                        tm["write_wait_s"] += clock() - t0
+                    t0 = clock()
+                    nb, nr = kin.format_frequency_rows(first, P - first, bufs[b])
+                    tm["format_s"] += clock() - t0
+                    pending[b] = writer.submit(fo.write, memoryview(bufs[b])[:nb])
+                    first += nr
+                    b ^= 1
+                i = j
+        t0 = clock()
+        for p in pending:
+            if p is not None:
+                p.result()
+        tm["write_wait_s"] += clock() - t0
+        fo.close()
+    except BaseException:
+        writer.shutdown(wait=True)
+        fo.close()
+        os.remove(out)
+        raise
+    writer.shutdown(wait=True)
 
 
 def _iter_with_kinship(self, ctx: Context, filter_stats: FilterStats, keep_p_minus_1: bool,
