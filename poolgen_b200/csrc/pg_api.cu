@@ -272,6 +272,8 @@ int pg_scan_open(pg_ctx *ctx, int kind, const pg_filter *filter, int n_pools, in
                 s->ptab_M = tab.M;
                 s->ptab_isd = tab.inv_sqrt_df;
                 s->ptab_bits = tab.bits;
+                s->ptab_t1 = tab.t_one;
+                s->ptab_t0 = tab.t_zero;
                 s->ptab_err = tab.max_err;
             }
         }
@@ -616,6 +618,8 @@ static int run_once(pg_batch *b, int *launches) {
             p.ptab = s->d_ptab.get();
             p.ptab_isd = s->ptab_isd;
             p.ptab_bits = s->ptab_bits;
+            p.ptab_t1 = s->ptab_t1;
+            p.ptab_t0 = s->ptab_t0;
             p.ptab_M = s->ptab_M;
             p.K = std::min(kpass, s->k - base);
             p.y_has_nan = s->y_has_nan;
@@ -660,6 +664,8 @@ static int run_once(pg_batch *b, int *launches) {
             q.ptab = s->d_ptab.get();
             q.ptab_isd = s->ptab_isd;
             q.ptab_bits = s->ptab_bits;
+            q.ptab_t1 = s->ptab_t1;
+            q.ptab_t0 = s->ptab_t0;
             q.ptab_M = s->ptab_M;
             for (int j = 0; j < s->A_dev; j++) q.codes[j] = s->codes_dev[j];
             q.meta = b->d_meta.get();

@@ -123,17 +123,21 @@ __device__ __forceinline__ double beta_reg_dev(double a, double b, double x, dou
 // (src/gwas/ols.rs:153, src/gwas/correlation_test.rs:66) including the cancellation 1 - (1 - ib).
 static __device__ __noinline__ double student_two_sided(double t_abs, double df, double ln_beta) {
     if (isinf(df)) return 2.0 * (1.0 - 0.5 * erfc(-t_abs / sqrt(2.0)));
-    const double h = df / (df + t_abs * t_abs);
+    // x rounded as the reference rounds it (no FMA): near t_one one ulp of x moves p by up to 1e-8 relative, and it
+    // decides statrs' cut-offs
+    const double h = df / __dadd_rn(df, __dmul_rn(t_abs, t_abs));
     const double ib = 0.5 * beta_reg_dev(df / 2.0, 0.5, h, ln_beta);
     const double cdf = t_abs <= 0.0 ? ib : 1.0 - ib;
     return 2.0 * (1.0 - cdf);
 }
 
 // Same quantity through the per-scan table of ln p indexed by the bits of 1 + |t| / sqrt(df) (pg_ptable.h).  The final
-// 2 * (1 - (1 - ib)) reproduces the reference's quantisation of small p-values.
+// 2 * (1 - (1 - ib)) reproduces the reference's quantisation of small p-values.  |t| <= t_one and |t| >= t_zero are
+// statrs' cut-offs, where the reference's p is exactly 1 resp. 0 (pg_ptable.h, student_t_cutoffs).
 struct PTableDev {
     const double4 *coef;
     double inv_sqrt_df, bits;  // bits: intervals per octave of w = 1 + |t| / sqrt(df) as a power of two
+    double t_one, t_zero;
     int M;
 };
 // interval and fraction of w = 1 + x from the bits of the double: idx = octave * 2^B + the top B mantissa bits
@@ -149,7 +153,7 @@ __device__ __forceinline__ int ptab_locate(double w, int B, double &s) {
 __device__ __forceinline__ double student_two_sided_tab(double t_abs, double df, const PTableDev &tb) {
     const double w = fma(t_abs, tb.inv_sqrt_df, 1.0);
     double ptrue = 0.0;
-    if (w < 1.7e308) {
+    if (t_abs < tb.t_zero) {  // (NaN fails this test and the one below and gets p = 0 as before)
         double s;
         const int i = ptab_locate(w, (int)tb.bits, s);
         if (i < tb.M) {
@@ -159,7 +163,7 @@ __device__ __forceinline__ double student_two_sided_tab(double t_abs, double df,
         }
     }
     const double ib = 0.5 * ptrue;
-    const double cdf = t_abs <= 0.0 ? ib : 1.0 - ib;
+    const double cdf = t_abs <= tb.t_one ? 0.5 : 1.0 - ib;  // p = 1 up to t_one (t = 0 included)
     return 2.0 * (1.0 - cdf);
 }
 

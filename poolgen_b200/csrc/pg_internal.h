@@ -83,7 +83,7 @@ struct ScanParams {
     double inv_n, inv_nm2; // 1 / n, 1 / (n - 2)
     double ln_beta;       // lnG(df/2 + 1/2) - lnG(df/2) - lnG(1/2)
     const void *ptab;     // per-scan table of ln p(v) (double4 per interval), NULL = continued fraction on the device
-    double ptab_isd, ptab_bits;
+    double ptab_isd, ptab_bits, ptab_t1, ptab_t0;  // t1 / t0: PTable::t_one / t_zero
     int ptab_M;
     const double *yc;     // [K][n_pad] centred phenotypes of this pass (device)
     const double *w;      // [n_pad] s_i / sum(s) (device)
@@ -131,7 +131,7 @@ struct NmParams {
     double gw_sig, gw_min, gw_max;
     double df, ln_beta;    // Student-t(n - 1)
     const void *ptab;
-    double ptab_isd, ptab_bits;
+    double ptab_isd, ptab_bits, ptab_t1, ptab_t0;  // t1 / t0: PTable::t_one / t_zero
     int ptab_M;
     uint8_t codes[8];      // allele code of device column j
     uint64_t *meta;
@@ -149,7 +149,7 @@ struct KinMleParams {
     const double *fix;   // zbar[m] | Szz[m][m] | Szz^-1 [m][m] | per phenotype: ybar, Syy, Szy[m]
     double df, ln_beta;  // Student-t(n - 1)
     const void *ptab;
-    double ptab_isd, ptab_bits;
+    double ptab_isd, ptab_bits, ptab_t1, ptab_t0;  // t1 / t0: PTable::t_one / t_zero
     int ptab_M;
     double *beta, *var, *pval;  // [k][P]
 };
@@ -315,7 +315,7 @@ struct pg_scan {
     pg::DeviceBuffer<double> d_yraw;  // mle_iter: raw phenotypes [k][n_pad]; gwalpha: bins [n_pad], q [n_pad]
     double gw_sig = 0, gw_min = 0, gw_max = 0;  // gwalpha_fmt: sig, MIN, MAX
     pg::DeviceBuffer<double> d_ptab;
-    double ptab_isd = 0, ptab_bits = 0, ptab_err = 0;
+    double ptab_isd = 0, ptab_bits = 0, ptab_err = 0, ptab_t1 = 0, ptab_t0 = 0;
     int ptab_M = 0;
     int n_slots = 0;
     // streaming

@@ -28,7 +28,7 @@ struct pg_kin {
     pg::DeviceBuffer<double> d_mle;  // pg_kin_mle_scan: centred covariates and phenotypes, then the fixed moments
     pg::DeviceBuffer<double> d_V;    // [(1+m) + k][ldg]
     pg::DeviceBuffer<double> d_ptab;
-    double ptab_isd = 0, ptab_bits = 0;
+    double ptab_isd = 0, ptab_bits = 0, ptab_t1 = 0, ptab_t0 = 0;
     int ptab_M = 0;
     // results
     int k = 0;

@@ -397,7 +397,7 @@ struct CovarParams {
     double nf, sqrt_n;
     double sy[kMaxPhenPerPass * 4];  // sum of the raw phenotype
     const void *ptab;
-    double ptab_isd, ptab_bits;
+    double ptab_isd, ptab_bits, ptab_t1, ptab_t0;  // t1 / t0: PTable::t_one / t_zero
     int ptab_M;
     double ln_beta;
     double *beta, *var, *pval;  // [k][P]
@@ -432,7 +432,7 @@ __global__ void __launch_bounds__(512) covar_kernel(const CovarParams p) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-    const PTableDev ptab = {reinterpret_cast<const double4 *>(p.ptab), p.ptab_isd, p.ptab_bits, p.ptab_M};
+    const PTableDev ptab = {reinterpret_cast<const double4 *>(p.ptab), p.ptab_isd, p.ptab_bits, p.ptab_t1, p.ptab_t0, p.ptab_M};
     const int nq = p.nq, k = p.k;
     // LIST: the columns a streaming kernel (this one with LIST = false, or the DMMA form) left to the explicit-residual
     // forms; the streaming instantiations carry none of that code
@@ -630,7 +630,7 @@ __global__ void __launch_bounds__(kCmMaxWarps * 32, 1) covar_mma_kernel(const Co
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, g = lane >> 2, t = lane & 3;
     constexpr int SCR = (8 * MT + 1) * 8;
     double *scr = cm_sm + (size_t)NV * ldq + (size_t)wib * SCR;  // U [8 MT][8] | g'g [8]
-    const PTableDev ptab = {reinterpret_cast<const double4 *>(p.ptab), p.ptab_isd, p.ptab_bits, p.ptab_M};
+    const PTableDev ptab = {reinterpret_cast<const double4 *>(p.ptab), p.ptab_isd, p.ptab_bits, p.ptab_t1, p.ptab_t0, p.ptab_M};
     const int64_t n_blocks = (p.P + 7) / 8;
     const int64_t wg = (int64_t)blockIdx.x * n_warps + wib, nwg = (int64_t)gridDim.x * n_warps;
     // vector rows of this lane in each M tile.  A row of D depends on its own row of A only and a column on its own
@@ -816,7 +816,7 @@ __global__ void __launch_bounds__(256) covar_generic_kernel(const CovarParams p)
     double *u = gcol + ldg;
     const int64_t warp = (int64_t)blockIdx.x * (blockDim.x >> 5) + wib;
     const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
-    const PTableDev ptab = {reinterpret_cast<const double4 *>(p.ptab), p.ptab_isd, p.ptab_bits, p.ptab_M};
+    const PTableDev ptab = {reinterpret_cast<const double4 *>(p.ptab), p.ptab_isd, p.ptab_bits, p.ptab_t1, p.ptab_t0, p.ptab_M};
     const int64_t n_items = p.defer_list ? (int64_t)*p.defer_count : p.P;
     for (int64_t item = warp; item < n_items; item += nwarps) {
         const int64_t c = p.defer_list ? p.defer_list[item] : item;
@@ -1622,6 +1622,8 @@ static int kin_prepare_records(pg_kin *h, int k) {
             h->ptab_M = tab.M;
             h->ptab_isd = tab.inv_sqrt_df;
             h->ptab_bits = tab.bits;
+            h->ptab_t1 = tab.t_one;
+            h->ptab_t0 = tab.t_zero;
         }
     }
     const size_t elems = (size_t)3 * k * std::max<int64_t>(h->P, 1);
@@ -1689,6 +1691,8 @@ int pg_kin_covar_scan(pg_kin *h, const double *phen, int k, int iters, float *ms
     cp.ptab = h->d_ptab.get();
     cp.ptab_isd = h->ptab_isd;
     cp.ptab_bits = h->ptab_bits;
+    cp.ptab_t1 = h->ptab_t1;
+    cp.ptab_t0 = h->ptab_t0;
     cp.ptab_M = h->ptab_M;
     cp.ln_beta = pg::statrs::ln_gamma(df / 2.0 + 0.5) - pg::statrs::ln_gamma(df / 2.0) - pg::statrs::ln_gamma(0.5);
     cp.beta = h->d_res.get();
@@ -1811,6 +1815,8 @@ int pg_kin_mle_scan(pg_kin *h, const double *phen, int k, float *ms, const doubl
     mp.ptab = h->d_ptab.get();
     mp.ptab_isd = h->ptab_isd;
     mp.ptab_bits = h->ptab_bits;
+    mp.ptab_t1 = h->ptab_t1;
+    mp.ptab_t0 = h->ptab_t0;
     mp.ptab_M = h->ptab_M;
     mp.beta = h->d_res.get();
     mp.var = h->d_res.get() + (size_t)k * h->P;

@@ -257,7 +257,7 @@ __global__ void __launch_bounds__(kMleWarps * 32) mle_kernel(const NmParams p) {
     const int64_t warp = (int64_t)blockIdx.x * kMleWarps + wib;
     const int64_t nwarps = (int64_t)gridDim.x * kMleWarps;
     const int n = p.lay.n, n_pad = p.lay.n_pad, S = p.lay.A - 1, k = p.k;
-    const PTableDev ptab = {reinterpret_cast<const double4 *>(p.ptab), p.ptab_isd, p.ptab_bits, p.ptab_M};
+    const PTableDev ptab = {reinterpret_cast<const double4 *>(p.ptab), p.ptab_isd, p.ptab_bits, p.ptab_t1, p.ptab_t0, p.ptab_M};
     const int64_t n_blocks = (p.n_loci + 31) / 32;
     for (int64_t blk = warp; blk < n_blocks; blk += nwarps) {
         const int64_t l0 = blk * 32;
@@ -679,7 +679,7 @@ __global__ void __launch_bounds__(kKmWarps * 32) kin_mle_kernel(const KinMlePara
     const double *zbar = km_sm, *Szz = zbar + m, *Wzz = Szz + m * m, *phf = Wzz + m * m;
     const int mw = 2 + m + k;  // gbar, Sgg, Szg[m], Sgy[k]
     double *mom = km_sm + fix_pad + (size_t)wib * 32 * mw;
-    const PTableDev ptab = {reinterpret_cast<const double4 *>(p.ptab), p.ptab_isd, p.ptab_bits, p.ptab_M};
+    const PTableDev ptab = {reinterpret_cast<const double4 *>(p.ptab), p.ptab_isd, p.ptab_bits, p.ptab_t1, p.ptab_t0, p.ptab_M};
     const double nn = (double)n;
     const int64_t n_blocks = (p.P + 31) / 32;
     for (int64_t blk = (int64_t)blockIdx.x * kKmWarps + wib; blk < n_blocks; blk += (int64_t)gridDim.x * kKmWarps) {

@@ -73,7 +73,38 @@ struct PTable {
     int M = 0;
     // interval i = the top bits of the double w = 1 + |t| / sqrt(df): octave e = i >> bits, 2^bits intervals per octave
     double inv_sqrt_df = 0.0, bits = 0.0, max_err = 1.0;
+    // statrs' cut-offs (student_t_cutoffs): the reference's p is exactly 1 for |t| <= t_one and exactly 0 for
+    // |t| >= t_zero; the table, which holds the converged tail, must not be consulted there
+    double t_one = 0.0, t_zero = 0.0;
 };
+
+// checked_beta_reg sets bt = 0 when x = df / (df + t^2) is below 1e-10 or within 4 ulps of 1, so the reference prints
+// p = 0 resp. p = 1 exactly, whatever the tail is.  x is formed as the reference forms it (pg_statrs_host.h: no
+// contraction); fl(t * t), fl(df + .) and fl(df / .) are monotone, so x is non-increasing in t and each set is an
+// interval of t, found by bisection on the ordered bit patterns of the non-negative doubles.
+//   t_one  = the largest t with ulps_eq_one(x)
+//   t_zero = the smallest t with x < 1e-10
+inline void student_t_cutoffs(double df, double &t_one, double &t_zero) {
+    auto dbl = [](uint64_t u) {
+        double d;
+        memcpy(&d, &u, 8);
+        return d;
+    };
+    auto x_of = [df](double t) { return df / (df + t * t); };
+    const uint64_t inf_bits = 0x7ff0000000000000ull;
+    uint64_t lo = 0, hi = inf_bits;  // ulps_eq_one(x(0)) holds, ulps_eq_one(x(inf)) = ulps_eq_one(0) does not
+    while (hi - lo > 1) {
+        const uint64_t mid = lo + (hi - lo) / 2;
+        (statrs::ulps_eq_one(x_of(dbl(mid))) ? lo : hi) = mid;
+    }
+    t_one = dbl(lo);
+    lo = 0, hi = inf_bits;  // x(0) = 1 is not below 1e-10, x(inf) = 0 is
+    while (hi - lo > 1) {
+        const uint64_t mid = lo + (hi - lo) / 2;
+        (fabs(x_of(dbl(mid))) < 1e-10 ? hi : lo) = mid;
+    }
+    t_zero = dbl(hi);
+}
 
 // ln p as a function of x = |t| / sqrt(df) (t^2 / df = x^2)
 inline double host_ln_tail_x(double x, double df) { return host_ln_tail(sqrt(log1p(x * x)), df); }
@@ -85,6 +116,7 @@ inline double host_ln_tail_x(double x, double df) { return host_ln_tail(sqrt(log
 inline PTable build_ptable(double df) {
     PTable t;
     t.inv_sqrt_df = 1.0 / sqrt(df);
+    student_t_cutoffs(df, t.t_one, t.t_zero);
     // x_max: beyond it ib = p/2 < 2^-62, so 1 - ib == 1 and the reference's p is exactly 0
     const double ln_floor = -43.0;
     double lo = 0.0, hi = 0.25;

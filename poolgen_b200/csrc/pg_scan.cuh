@@ -1083,7 +1083,8 @@ __device__ __forceinline__ void student_batch(const ScanParams &p, const PTableD
         const double ta = need[k] ? t_abs[k] : 0.0;
         const double w = fma(ta, tab.inv_sqrt_df, 1.0);
         int i = ptab_locate(w, B, s[k]);
-        in[k] = need[k] && (w < 1.7e308) && (i < tab.M);
+        // statrs' cut-offs (student_two_sided_tab): p = 0 from t_zero on (w is finite below it)
+        in[k] = need[k] && (ta < tab.t_zero) && (i < tab.M);
         if (!in[k]) i = 0;
         cp[k] = reinterpret_cast<const double2 *>(tab.coef + i);
     }
@@ -1097,7 +1098,8 @@ __device__ __forceinline__ void student_batch(const ScanParams &p, const PTableD
     for (int k = 0; k < K; k++) {
         const double ptrue = in[k] ? exp(fma(s[k], fma(s[k], fma(s[k], c23[k].y, c23[k].x), c01[k].y), c01[k].x)) : 0.0;
         const double ib = 0.5 * ptrue;
-        const double cdf = t_abs[k] <= 0.0 ? ib : 1.0 - ib;  // the reference's 2 * (1 - (1 - ib)) quantisation
+        // the reference's 2 * (1 - (1 - ib)) quantisation; p = 1 up to t_one (t = 0 included)
+        const double cdf = t_abs[k] <= tab.t_one ? 0.5 : 1.0 - ib;
         if (need[k]) pv[k] = 2.0 * (1.0 - cdf);
     }
 }
@@ -1191,7 +1193,7 @@ template <int A, int K, bool W, bool DEFER, int KIND>
 __device__ __noinline__ void epilogue(const ScanParams &p, int64_t locus, bool act, double *tot, const double *ys,
                                       const double *ws, int lane, unsigned dm, unsigned pre_kept) {
     using AC = Acc<A, K, W>;
-    const PTableDev ptab = {reinterpret_cast<const double4 *>(p.ptab), p.ptab_isd, p.ptab_bits, p.ptab_M};
+    const PTableDev ptab = {reinterpret_cast<const double4 *>(p.ptab), p.ptab_isd, p.ptab_bits, p.ptab_t1, p.ptab_t0, p.ptab_M};
     double *tg = tot + (size_t)lane * AC::NP;
     const double tol_rel = 2.0 * ((double)p.lay.n + 8.0) * kEps;
     int status = PG_LOCUS_FILTERED;

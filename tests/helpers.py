@@ -40,6 +40,44 @@ def load_c1():
                 chrom_names=z["chrom_names"], chrom_idx=z["chrom_idx"], pos=z["pos"])
 
 
+def student_t_cutoffs(df):
+    """statrs' two cut-offs of the Student-t tail as (t_one, t_zero): checked_beta_reg sets bt = 0 when
+    x = df / (df + t^2) is within 4 ulps of 1 (x >= 1 - 4 * 2^-53) or below 1e-10, so the reference's two-sided p is
+    exactly 1 for |t| <= t_one and exactly 0 for |t| >= t_zero.  x is formed in f64 without contraction (Python
+    floats), and is non-increasing in t, so each edge is found by bisection on the bit patterns of non-negative doubles
+    (the restatement of pg_ptable.h's student_t_cutoffs)."""
+    import struct
+
+    def dbl(u):
+        return struct.unpack("<d", struct.pack("<Q", u))[0]
+
+    def x_of(t):
+        return df / (df + t * t)
+
+    lo, hi = 0, 0x7FF0000000000000
+    while hi - lo > 1:
+        mid = (lo + hi) // 2
+        if x_of(dbl(mid)) >= 1.0 - 4.0 * 2.0 ** -53:
+            lo = mid
+        else:
+            hi = mid
+    t_one = dbl(lo)
+    lo, hi = 0, 0x7FF0000000000000
+    while hi - lo > 1:
+        mid = (lo + hi) // 2
+        if abs(x_of(dbl(mid))) < 1e-10:
+            hi = mid
+        else:
+            lo = mid
+    return t_one, dbl(hi)
+
+
+def student_t_p(t, df):
+    """the reference's two-sided p of each |t| (src/gwas/ols.rs:153): 2 * (1 - StudentsT(0, 1, df).cdf(|t|))"""
+    t = np.abs(np.asarray(t, dtype=np.float64))
+    return np.array([2.0 * (1.0 - pgo.students_t_cdf(float(v), float(df))) for v in t.ravel()]).reshape(t.shape)
+
+
 def oracle_fs(fs):
     return pgo.FilterStats(pool_sizes=np.asarray(fs.pool_sizes, dtype=np.float64), remove_ns=fs.remove_ns,
                            min_coverage_depth=fs.min_coverage_depth,
