@@ -45,6 +45,7 @@ ABI_SYMBOLS = [
 # include/poolgen_synth.h (libpoolgen_synth.so: host replay of the synthetic workload, no CUDA)
 SYNTH_SYMBOLS = ["pg_synth_counts_host", "pg_synth_phen_host", "pg_synth_sync_text_host"]
 COMM_ID_BYTES = 128
+STREAM_DEPTH = 3  # PG_STREAM_DEPTH: text slabs a scan keeps in flight
 
 
 class PgError(RuntimeError):
@@ -60,6 +61,13 @@ class _Filter(C.Structure):
         ("n_pool_sizes", C.c_int32),
         ("pool_sizes", C.POINTER(C.c_double)),
     ]
+
+
+def _filter(fs) -> tuple:
+    """pg_filter of a FilterStats + the pool sizes array it points into, which must outlive its use"""
+    ps = np.ascontiguousarray(fs.pool_sizes, dtype=np.float64)
+    return _Filter(int(fs.remove_ns), int(fs.min_coverage_depth), float(fs.min_allele_frequency),
+                   float(fs.max_missingness_rate), int(ps.size), ps.ctypes.data_as(C.POINTER(C.c_double))), ps
 
 
 class _Results(C.Structure):
@@ -276,42 +284,42 @@ def format_f64(x: float, n_digits: int = 0) -> str:
 FORMAT_EXACT_P = 1
 
 
-def format_rows(kind: int, results, positions, text: bytes | None = None, line_offsets=None, chr_names=None,
-                chr_index=None, n_threads: int = 0, exact_p_pools: int = 0) -> bytes:
+def _formatted(fn, what: str, *args) -> bytes:
+    """the text of a writer call fn(*args, out, capacity, &n_bytes): once with no buffer for the size, then to fill"""
+    need = C.c_size_t()
+    rc = fn(*args, None, 0, C.byref(need))
+    if need.value == 0:
+        if rc != PG_OK:
+            raise PgError(f"{what}: bad arguments")
+        return b""
+    buf = C.create_string_buffer(need.value)
+    _check(fn(*args, buf, need.value, C.byref(need)), None, what)
+    return buf.raw[:need.value]
+
+
+def format_rows(kind: int, results, positions, text=None, line_offsets=None, chr_names=None, chr_index=None,
+                n_threads: int = 0, exact_p_pools: int = 0) -> bytes:
     """CSV rows of the per-locus callbacks for a slab of records (`results`: ScanResults or the raw pg_results of
-    Scan.collect(copy=False)).  Chromosome names come from the sync text the loci were parsed from (text +
-    line_offsets, as Batch.upload_sync_text returns them) or from chr_names[chr_index[locus]].
+    Scan.collect(copy=False)).  Chromosome names come from the sync text the loci were parsed from (text as bytes or a
+    uint8 array, + line_offsets, as Batch.upload_sync_text returns them) or from chr_names[chr_index[locus]].
     exact_p_pools = n_pools > 0: PG_FORMAT_EXACT_P, the printed p-values are re-derived from t with the reference's own
     arithmetic (ols_iter / pearson_corr)."""
     keep = None
     if isinstance(results, ScanResults):
         results, keep = results.to_c()
-    pos = np.ascontiguousarray(positions, dtype=np.uint64)
-    lab = _RowLabels()
-    lab.positions = pos.ctypes.data_as(C.POINTER(C.c_uint64))
-    if text is not None:
-        off = np.ascontiguousarray(line_offsets, dtype=np.uint64)
-        lab.text = text
-        lab.line_offsets = off.ctypes.data_as(C.POINTER(C.c_uint64))
-    else:
-        names = (C.c_char_p * len(chr_names))(*[n.encode() if isinstance(n, str) else n for n in chr_names])
-        idx = np.ascontiguousarray(chr_index, dtype=np.uint32)
-        lab.chr_names = names
-        lab.chr_index = idx.ctypes.data_as(C.POINTER(C.c_uint32))
-    n_threads = n_threads or (os.cpu_count() or 1)
-    need = C.c_size_t()
+    lab, keep_lab = _row_labels(positions, text, line_offsets, chr_names, chr_index)
     flags = FORMAT_EXACT_P if exact_p_pools > 0 else 0
-    rc = lib().pg_format_rows_ex(int(kind), C.byref(results), C.byref(lab), flags, int(exact_p_pools), n_threads, None, 0,
-                                 C.byref(need))
-    if need.value == 0:
-        if rc != PG_OK:
-            raise PgError("pg_format_rows: bad arguments")
-        return b""
-    buf = C.create_string_buffer(need.value)
-    _check(lib().pg_format_rows_ex(int(kind), C.byref(results), C.byref(lab), flags, int(exact_p_pools), n_threads, buf,
-                                   need.value, C.byref(need)), None, "pg_format_rows_ex")
-    del keep
-    return buf.raw[:need.value]
+    return _formatted(lib().pg_format_rows_ex, "pg_format_rows_ex", int(kind), C.byref(results), C.byref(lab), flags,
+                      int(exact_p_pools), n_threads or (os.cpu_count() or 1))
+
+
+def _text_arg(text):
+    """sync text as the library takes it: (bytes object or address of a C-contiguous uint8 array, length), no copy"""
+    if isinstance(text, np.ndarray):
+        assert text.dtype == np.uint8 and text.flags["C_CONTIGUOUS"]
+        return text.ctypes.data, int(text.size)
+    buf = bytes(text)
+    return buf, len(buf)
 
 
 def _row_labels(positions, text=None, line_offsets=None, chr_names=None, chr_index=None):
@@ -322,7 +330,7 @@ def _row_labels(positions, text=None, line_offsets=None, chr_names=None, chr_ind
     keep = [pos]
     if text is not None:
         off = np.ascontiguousarray(line_offsets, dtype=np.uint64)
-        lab.text = text
+        lab.text = _text_arg(text)[0]
         lab.line_offsets = off.ctypes.data_as(C.POINTER(C.c_uint64))
         keep += [text, off]
     else:
@@ -345,12 +353,7 @@ def sort_loci(positions, **label_kw) -> np.ndarray:
 
 def format_frequency_header(pool_names) -> bytes:
     names = (C.c_char_p * len(pool_names))(*[n.encode() if isinstance(n, str) else n for n in pool_names])
-    need = C.c_size_t()
-    lib().pg_format_frequency_header(names, len(pool_names), None, 0, C.byref(need))
-    buf = C.create_string_buffer(need.value)
-    _check(lib().pg_format_frequency_header(names, len(pool_names), buf, need.value, C.byref(need)), None,
-           "pg_format_frequency_header")
-    return buf.raw[:need.value]
+    return _formatted(lib().pg_format_frequency_header, "pg_format_frequency_header", names, len(pool_names))
 
 
 def format_frequency_rows(columns, col_locus, col_allele, positions, locus_order=None, n_threads: int = 0, **label_kw) -> bytes:
@@ -362,15 +365,9 @@ def format_frequency_rows(columns, col_locus, col_allele, positions, locus_order
     lab, keep = _row_labels(positions, **label_kw)
     order = None if locus_order is None else np.ascontiguousarray(locus_order, dtype=np.int64)
     P, n = (cols.shape if cols.ndim == 2 else (0, 1))
-    n_threads = n_threads or (os.cpu_count() or 1)
-    args = (P, n, cols.ctypes.data, cl.ctypes.data, ca.ctypes.data, C.byref(lab),
-            None if order is None else order.ctypes.data, 0 if order is None else order.size, n_threads)
-    need = C.c_size_t()
-    lib().pg_format_frequency_rows(*args, None, 0, C.byref(need))
-    buf = C.create_string_buffer(max(1, need.value))
-    _check(lib().pg_format_frequency_rows(*args, buf, need.value, C.byref(need)), None, "pg_format_frequency_rows")
-    del keep
-    return buf.raw[:need.value]
+    return _formatted(lib().pg_format_frequency_rows, "pg_format_frequency_rows", P, n, cols.ctypes.data,
+                      cl.ctypes.data, ca.ctypes.data, C.byref(lab), None if order is None else order.ctypes.data,
+                      0 if order is None else order.size, n_threads or (os.cpu_count() or 1))
 
 
 def format_kinship_rows(chromosome, position, allele, beta, pval, n_threads: int = 0) -> bytes:
@@ -383,19 +380,24 @@ def format_kinship_rows(chromosome, position, allele, beta, pval, n_threads: int
     cn = (C.c_char_p * P)(*[enc(v) for v in chromosome[:P]])
     an = (C.c_char_p * P)(*[enc(v) for v in allele[:P]])
     pos = np.ascontiguousarray(position[:P], dtype=np.uint64)
-    n_threads = n_threads or (os.cpu_count() or 1)
-    need = C.c_size_t()
-    lib().pg_format_kinship_rows(P, k, cn, pos.ctypes.data, an, b.ctypes.data, p.ctypes.data, n_threads, None, 0, C.byref(need))
-    buf = C.create_string_buffer(max(1, need.value))
-    _check(lib().pg_format_kinship_rows(P, k, cn, pos.ctypes.data, an, b.ctypes.data, p.ctypes.data, n_threads, buf,
-                                        need.value, C.byref(need)), None, "pg_format_kinship_rows")
-    return buf.raw[:need.value]
+    return _formatted(lib().pg_format_kinship_rows, "pg_format_kinship_rows", P, k, cn, pos.ctypes.data, an,
+                      b.ctypes.data, p.ctypes.data, n_threads or (os.cpu_count() or 1))
 
 
 def _check(rc: int, ctx=None, what: str = ""):
     if rc != PG_OK:
         msg = lib().pg_last_error(ctx)
         raise PgError(f"{what} failed ({rc}): {msg.decode() if msg else ''}")
+
+
+def _parse_labels(n_loci: int, rc_of, ctx, what: str):
+    """(line byte offsets, positions) of the n_loci loci of a text parse, copied out of the library's arrays, which
+    rc_of(&offsets, &positions) points at"""
+    po, pp = C.c_void_p(), C.c_void_p()
+    _check(rc_of(C.byref(po), C.byref(pp)), ctx, what)
+    if n_loci == 0:
+        return np.zeros(0, np.uint64), np.zeros(0, np.uint64)
+    return tuple(np.ctypeslib.as_array(C.cast(p, C.POINTER(C.c_uint64)), shape=(n_loci,)).copy() for p in (po, pp))
 
 
 class Context:
@@ -449,10 +451,8 @@ class Scan:
         self.ctx = ctx
         self.kind = kind
         codes = np.ascontiguousarray(allele_codes, dtype=np.uint8)
-        ps = np.ascontiguousarray(fs.pool_sizes, dtype=np.float64)
+        f, ps = _filter(fs)
         self._keep = (codes, ps)
-        f = _Filter(int(fs.remove_ns), int(fs.min_coverage_depth), float(fs.min_allele_frequency),
-                    float(fs.max_missingness_rate), int(ps.size), ps.ctypes.data_as(C.POINTER(C.c_double)))
         if phen is not None:
             y = np.ascontiguousarray(phen, dtype=np.float64)
             if y.ndim == 1:
@@ -553,12 +553,8 @@ class Batch:
         n = C.c_int64()
         self._ck(lib().pg_batch_upload_sync_text(self._h, buf, len(buf), C.byref(n)), "pg_batch_upload_sync_text")
         L = int(n.value)
-        po, pp = C.c_void_p(), C.c_void_p()
-        self._ck(lib().pg_batch_text_labels(self._h, C.byref(po), C.byref(pp)), "pg_batch_text_labels")
-        if L == 0:
-            return 0, np.zeros(0, np.uint64), np.zeros(0, np.uint64)
-        off = np.ctypeslib.as_array(C.cast(po, C.POINTER(C.c_uint64)), shape=(L,)).copy()
-        pos = np.ctypeslib.as_array(C.cast(pp, C.POINTER(C.c_uint64)), shape=(L,)).copy()
+        off, pos = _parse_labels(L, lambda po, pp: lib().pg_batch_text_labels(self._h, po, pp), self.scan.ctx._h,
+                                 "pg_batch_text_labels")
         return L, off, pos
 
     def run(self):
@@ -624,9 +620,7 @@ class Kinship:
         """counts: uint32 [L, A, n_pools]; returns (col_locus int64 [P_add], col_allele uint8 [P_add])."""
         c = np.ascontiguousarray(counts, dtype=np.uint32)
         codes = np.ascontiguousarray(allele_codes, dtype=np.uint8)
-        ps = np.ascontiguousarray(fs.pool_sizes, dtype=np.float64)
-        f = _Filter(int(fs.remove_ns), int(fs.min_coverage_depth), float(fs.min_allele_frequency),
-                    float(fs.max_missingness_rate), int(ps.size), ps.ctypes.data_as(C.POINTER(C.c_double)))
+        f, _ps = _filter(fs)
         added = C.c_int64()
         self._ck(lib().pg_kin_append_counts(self._h, C.byref(f), int(codes.size),
                                             codes.ctypes.data_as(C.POINTER(C.c_uint8)), c.ctypes.data, int(c.shape[0]),
@@ -637,24 +631,17 @@ class Kinship:
         self._ck(lib().pg_kin_last_labels(self._h, n_add, loc.ctypes.data, alle.ctypes.data), "pg_kin_last_labels")
         return loc, alle
 
-    def append_sync_text(self, text: bytes, fs: FilterStats, max_loci: int, keep_p_minus_1: bool = False):
-        """a line-aligned chunk of sync text through the device parser and LoadAll: returns (n_loci, line offsets,
-        positions, col_locus, col_allele)"""
-        buf = bytes(text)
-        ps = np.ascontiguousarray(fs.pool_sizes, dtype=np.float64)
-        f = _Filter(int(fs.remove_ns), int(fs.min_coverage_depth), float(fs.min_allele_frequency),
-                    float(fs.max_missingness_rate), int(ps.size), ps.ctypes.data_as(C.POINTER(C.c_double)))
+    def append_sync_text(self, text, fs: FilterStats, max_loci: int, keep_p_minus_1: bool = False):
+        """a line-aligned chunk of sync text (bytes or a uint8 array) through the device parser and LoadAll: returns
+        (n_loci, line offsets, positions, col_locus, col_allele)"""
+        buf, size = _text_arg(text)
+        f, _ps = _filter(fs)
         nl, added = C.c_int64(), C.c_int64()
-        self._ck(lib().pg_kin_append_sync_text(self._h, C.byref(f), buf, len(buf), int(max_loci), int(keep_p_minus_1),
+        self._ck(lib().pg_kin_append_sync_text(self._h, C.byref(f), buf, size, int(max_loci), int(keep_p_minus_1),
                                                C.byref(nl), C.byref(added)), "pg_kin_append_sync_text")
         L, n_add = int(nl.value), int(added.value)
-        po, pp = C.c_void_p(), C.c_void_p()
-        self._ck(lib().pg_kin_text_labels(self._h, C.byref(po), C.byref(pp)), "pg_kin_text_labels")
-        if L:
-            off = np.ctypeslib.as_array(C.cast(po, C.POINTER(C.c_uint64)), shape=(L,)).copy()
-            pos = np.ctypeslib.as_array(C.cast(pp, C.POINTER(C.c_uint64)), shape=(L,)).copy()
-        else:
-            off, pos = np.zeros(0, np.uint64), np.zeros(0, np.uint64)
+        off, pos = _parse_labels(L, lambda po, pp: lib().pg_kin_text_labels(self._h, po, pp), self.ctx._h,
+                                 "pg_kin_text_labels")
         loc = np.empty(n_add, dtype=np.int64)
         alle = np.empty(n_add, dtype=np.uint8)
         self._ck(lib().pg_kin_last_labels(self._h, n_add, loc.ctypes.data, alle.ctypes.data), "pg_kin_last_labels")
@@ -734,13 +721,7 @@ class Kinship:
         pb, pv, pp = C.c_void_p(), C.c_void_p(), C.c_void_p()
         self._ck(lib().pg_kin_covar_scan(self._h, y.ctypes.data, int(k), int(iters), C.byref(ms), C.byref(pb), C.byref(pv),
                                          C.byref(pp)), "pg_kin_covar_scan")
-        P = self.columns
-
-        def arr(p):
-            if P == 0:
-                return np.zeros((k, 0))
-            return np.ctypeslib.as_array(C.cast(p, C.POINTER(C.c_double)), shape=(k, P)).copy()
-        out = (arr(pb), arr(pv), arr(pp))
+        out = self._records(k, (pb, pv, pp))
         return out + (float(ms.value),) if iters > 0 else out
 
     def mle_scan(self, phen, timed: bool = False):
@@ -754,14 +735,15 @@ class Kinship:
         pb, pv, pp = C.c_void_p(), C.c_void_p(), C.c_void_p()
         self._ck(lib().pg_kin_mle_scan(self._h, y.ctypes.data, int(k), C.byref(ms), C.byref(pb), C.byref(pv), C.byref(pp)),
                  "pg_kin_mle_scan")
-        P = self.columns
-
-        def arr(p):
-            if P == 0:
-                return np.zeros((k, 0))
-            return np.ctypeslib.as_array(C.cast(p, C.POINTER(C.c_double)), shape=(k, P)).copy()
-        out = (arr(pb), arr(pv), arr(pp))
+        out = self._records(k, (pb, pv, pp))
         return out + (float(ms.value),) if timed else out
+
+    def _records(self, k: int, ptrs) -> tuple:
+        """copies of the scan's [k, columns] f64 record arrays behind ptrs"""
+        P = self.columns
+        if P == 0:
+            return tuple(np.zeros((k, 0)) for _ in ptrs)
+        return tuple(np.ctypeslib.as_array(C.cast(p, C.POINTER(C.c_double)), shape=(k, P)).copy() for p in ptrs)
 
     def close(self):
         if self._h:
@@ -858,24 +840,19 @@ def submit_sync_text(scan: "Scan", text: bytes, deferred: bool = False):
     deferred=True passes n_loci = NULL: the call only enqueues the copy and the parse (n_loci comes back as None, the
     count is in the collected records) and the slab's scan is launched by the next submit or by its collect."""
     t, n = C.c_int(), C.c_int64()
-    buf = bytes(text)
+    buf, size = _text_arg(text)
     if not hasattr(scan, "_keep_text"):
         scan._keep_text = {}
-    _check(lib().pg_scan_submit_sync_text(scan._h, buf, len(buf), C.byref(t), None if deferred else C.byref(n)),
+    _check(lib().pg_scan_submit_sync_text(scan._h, buf, size, C.byref(t), None if deferred else C.byref(n)),
            scan.ctx._h, "pg_scan_submit_sync_text")
-    scan._keep_text[t.value] = buf  # the chunk must stay alive until its ticket is collected
+    scan._keep_text[t.value] = (text, buf)  # the chunk must stay alive until its ticket is collected
     return t.value, (None if deferred else int(n.value))
 
 
 def text_labels(scan: "Scan", ticket: int, n_loci: int):
     """pg_scan_text_labels after the collect of `ticket`: (line byte offsets, positions) of its loci"""
-    po, pp = C.c_void_p(), C.c_void_p()
-    _check(lib().pg_scan_text_labels(scan._h, int(ticket), C.byref(po), C.byref(pp)), scan.ctx._h, "pg_scan_text_labels")
-    if n_loci == 0:
-        return np.zeros(0, np.uint64), np.zeros(0, np.uint64)
-    off = np.ctypeslib.as_array(C.cast(po, C.POINTER(C.c_uint64)), shape=(n_loci,)).copy()
-    pos = np.ctypeslib.as_array(C.cast(pp, C.POINTER(C.c_uint64)), shape=(n_loci,)).copy()
-    return off, pos
+    return _parse_labels(int(n_loci), lambda po, pp: lib().pg_scan_text_labels(scan._h, int(ticket), po, pp),
+                         scan.ctx._h, "pg_scan_text_labels")
 
 
 def synth_counts_host(seed: int, first_locus: int, n_loci: int, n_pools: int, n_alleles: int) -> np.ndarray:

@@ -8,7 +8,6 @@ appends the rows `pg_format_rows` returns.  Nothing here computes on the CPU; wi
 """
 from __future__ import annotations
 
-import ctypes as C
 import os
 import threading
 import time
@@ -103,10 +102,6 @@ def find_file_splits(fname: str, n_threads: int) -> list:
     return dedup
 
 
-_KIND_NAMES = {KIND_OLS: "ols_iter", KIND_CORR: "pearson_corr", KIND_CHISQ: "chisq_test", KIND_FISHER: "fisher_exact_test",
-               KIND_MLE: "mle_iter", KIND_GWALPHA_LS: "gwalpha", KIND_GWALPHA_ML: "gwalpha"}
-
-
 def _kind_of(function) -> int:
     """the reference passes the callback itself (gwas::ols_iterate, gwas::correlation, tables::chisq, tables::fisher)"""
     if isinstance(function, int):
@@ -125,84 +120,72 @@ def _default_out(fname: str, test: str) -> str:
     return f"{bname}-{time.time()}-{test}.csv"
 
 
+def _last_line_end(view) -> int:
+    """the length of view up to and including its last newline, 0 if it has none; searched back from the end"""
+    hi = view.size
+    while hi:
+        lo = max(hi - (1 << 16), 0)
+        nl = np.flatnonzero(view[lo:hi] == 10)
+        if nl.size:
+            return lo + int(nl[-1]) + 1
+        hi = lo
+    return 0
+
+
+def _line_blocks(fname: str, start: int, end: int, block_bytes: int, bufs: list):
+    """(absolute byte offset, uint8 view) of line-aligned blocks of at most block_bytes bytes over [start, end) of the
+    file, read into the arrays `bufs` in turn.  While bytes of the range remain, a block ends at its last newline and
+    the rest moves to the head of the next buffer; the last block takes what is left, so a last line without a newline
+    joins it where it fits.  Block i + len(bufs) reuses the buffer of block i: the caller is done with block i before
+    it asks for that one (with one buffer, before it asks for the next block)."""
+    with open(fname, "rb", buffering=0) as fh:
+        fh.seek(start)
+        at, left, tail, i = start, end - start, bufs[0][:0], 0
+        while left > 0 or tail.size:
+            buf, nc = bufs[i % len(bufs)], tail.size
+            buf[:nc] = tail
+            got = fh.readinto(memoryview(buf)[nc:nc + min(left, block_bytes - nc)]) if left > 0 else 0
+            left = left - got if got else 0  # the file ended before the range did
+            fill = cut = nc + got
+            if left:
+                cut = _last_line_end(buf[:fill])
+                if cut == 0:
+                    raise PgError(f"a line of {fname} is longer than the block size {block_bytes}")
+            if cut:
+                yield at, buf[:cut]
+            at, tail, i = at + cut, buf[cut:fill], i + 1
+
+
 def _chunk_worker(ctx: Context, kind: int, fs: FilterStats, n_pools: int, phen, fname: str, start: int, end: int,
                   block_bytes: int, fmt_threads: int, sink: list, errors: list):
     """the body of `per_chunk` (src/base/sync.rs:794-870 / 612-687) for the byte range [start, end)"""
-    lib = capi.lib()
     scan = None
     pinned = []
     try:
         scan = Scan(ctx, kind, fs, n_pools, np.arange(6, dtype=np.uint8), phen)
-        # a locus line holds at least "c\\t0\\tN" + n_pools * "\\t0:0:0:0:0:0" bytes
-        max_loci = block_bytes // (12 * n_pools + 5) + 2
-        scan.stream_begin(max_loci)
+        scan.stream_begin(_max_loci(block_bytes, n_pools))
         bufs = []
-        for _ in range(capi_stream_depth()):
+        for _ in range(capi.STREAM_DEPTH):
             arr, h = ctx.pinned_empty((block_bytes,), np.uint8)
             pinned.append(h)
             bufs.append(arr)
         out = bytearray()
-        pending = []  # (ticket, buffer index)
+        pending = []  # (ticket, block)
 
-        def finish(item):
-            ticket, bi = item
+        def finish(ticket, block):
             res = scan.collect(ticket, copy=False)
-            if res.n_loci == 0:
-                return
-            po, pp = C.c_void_p(), C.c_void_p()
-            capi._check(lib.pg_scan_text_labels(scan._h, int(ticket), C.byref(po), C.byref(pp)), ctx._h,
-                        "pg_scan_text_labels")
-            lab = capi._RowLabels()
-            lab.positions = C.cast(pp, C.POINTER(C.c_uint64))
-            lab.text = C.cast(bufs[bi].ctypes.data, C.c_char_p)
-            lab.line_offsets = C.cast(po, C.POINTER(C.c_uint64))
-            need = C.c_size_t()
-            # the output file carries the reference's own p-value digits (PG_FORMAT_EXACT_P)
-            lib.pg_format_rows_ex(kind, C.byref(res), C.byref(lab), capi.FORMAT_EXACT_P, scan.n_pools, fmt_threads,
-                                  None, 0, C.byref(need))
-            if need.value:
-                rows = C.create_string_buffer(need.value)
-                capi._check(lib.pg_format_rows_ex(kind, C.byref(res), C.byref(lab), capi.FORMAT_EXACT_P, scan.n_pools,
-                                                  fmt_threads, rows, need.value, C.byref(need)), ctx._h,
-                            "pg_format_rows_ex")
-                out.extend(rows.raw[:need.value])
+            if res.n_loci:
+                off, pos = capi.text_labels(scan, ticket, res.n_loci)
+                # the output file carries the reference's own p-value digits (PG_FORMAT_EXACT_P)
+                out.extend(capi.format_rows(kind, res, pos, text=block, line_offsets=off, n_threads=fmt_threads,
+                                            exact_p_pools=n_pools))
 
-        with open(fname, "rb", buffering=0) as fh:
-            fh.seek(start)
-            left = end - start
-            carry = b""
-            bi = 0
-            while left > 0 or carry:
-                buf = bufs[bi]
-                nc = len(carry)
-                if nc:
-                    buf[:nc] = np.frombuffer(carry, dtype=np.uint8)
-                want = min(left, block_bytes - nc)
-                got = fh.readinto(memoryview(buf)[nc:nc + want]) if want > 0 else 0
-                left -= got
-                fill = nc + got
-                if left > 0 and got > 0:
-                    # cut at the last newline; the tail opens the next block
-                    view = buf[:fill]
-                    nl = np.flatnonzero(view[::-1] == 10)
-                    if nl.size == 0:
-                        raise PgError(f"a line of {fname} is longer than the block size {block_bytes}")
-                    cut = fill - int(nl[0])
-                    carry = bytes(view[cut:])
-                    fill = cut
-                else:
-                    carry = b""
-                    if got == 0 and left > 0:
-                        left = 0  # the file shrank
-                ticket = C.c_int()
-                capi._check(lib.pg_scan_submit_sync_text(scan._h, buf.ctypes.data, fill, C.byref(ticket), None), ctx._h,
-                            "pg_scan_submit_sync_text")
-                pending.append((ticket.value, bi))
-                bi = (bi + 1) % len(bufs)
-                if len(pending) == len(bufs):
-                    finish(pending.pop(0))
-            while pending:
-                finish(pending.pop(0))
+        for _, block in _line_blocks(fname, start, end, block_bytes, bufs):
+            pending.append((capi.submit_sync_text(scan, block, deferred=True)[0], block))
+            if len(pending) == len(bufs):
+                finish(*pending.pop(0))
+        while pending:
+            finish(*pending.pop(0))
         sink.append((start, bytes(out)))
     except Exception as e:  # noqa: BLE001 -- re-raised by the caller, like a panicking reader thread
         errors.append(e)
@@ -211,10 +194,6 @@ def _chunk_worker(ctx: Context, kind: int, fs: FilterStats, n_pools: int, phen, 
             scan.close()
         for h in pinned:
             ctx.pinned_free(h)
-
-
-def capi_stream_depth() -> int:
-    return 3  # PG_STREAM_DEPTH
 
 
 def _read_analyse_write(ctx, kind, fs, n_pools, phen, fname, test, out, n_threads, block_bytes):
@@ -286,7 +265,6 @@ class FileSync:
 # (into_genotypes_and_phenotypes + ols_with_covariate, src/base/sync.rs:1106-1179, src/gwas/ols.rs:278-436) ----------
 @dataclass
 class _LoadedColumns:
-    kin: object            # capi.Kinship holding the allele columns on the device, in file order
     col_locus: np.ndarray  # int64 [P] locus ordinal (over the kept loci of the whole file) of every column
     col_allele: np.ndarray # uint8 [P]
     chr_names: list        # distinct chromosome names
@@ -302,6 +280,11 @@ _KIN_RESERVE_BYTES = 1 << 30  # outside the handle: cuSOLVER's and cuBLAS' handl
 def _line_min_bytes(n_pools: int) -> int:
     """a locus line holds at least "c\\t0\\tN" + n_pools * "\\t0:0:0:0:0:0" bytes"""
     return 12 * n_pools + 5
+
+
+def _max_loci(block_bytes: int, n_pools: int) -> int:
+    """the loci a text block of block_bytes bytes can hold at most: the max_loci of the device loaders"""
+    return block_bytes // _line_min_bytes(n_pools) + 2
 
 
 def text_block_columns(n_bytes: int, n_pools: int, n_lines: int = None) -> int:
@@ -334,7 +317,7 @@ def kin_device_bytes(n_pools: int, columns: int, k: int, block_bytes: int, sm_co
     # eigen step: the matrix, the eigenvalues, syevd's workspace (1 + 6 n + 2 n^2 doubles), info
     total += n * n * 8 + n * 8 + (1 + 6 * n + 2 * n * n) * 8 + 4
     # loader scratch of one text block (max_loci loci of six columns) and the device parser's buffers
-    L = block_bytes // _line_min_bytes(n) + 2
+    L = _max_loci(block_bytes, n)
     total += L * 4 + (L + 1) * 8 + L * 6 * 8 + L * 6 + (8 * L + (64 << 10)) + L * 6 * n * 4 + n * 8
     nb = block_bytes + 1
     total += _grow(nb + 32, 1) + _grow(nb, 4) + _grow(-(-nb // 4096) + 1, 8)
@@ -358,53 +341,38 @@ def kin_block_columns(device_bytes: int, n_pools: int, k: int, block_bytes: int,
     return lo
 
 
-def _text_blocks(fname: str, block_bytes: int):
-    """(byte offset, text) of line-aligned blocks of at most block_bytes bytes over the whole file"""
-    with open(fname, "rb") as fh:
-        at, carry = 0, b""
-        while True:
-            data = fh.read(block_bytes - len(carry))
-            if not data and not carry:
-                return
-            block = carry + data
-            if data:
-                cut = block.rfind(b"\n") + 1
-                if cut == 0:
-                    raise PgError(f"a line of {fname} is longer than the block size {block_bytes}")
-                block, carry = block[:cut], block[cut:]
-            else:
-                carry = b""
-            yield at, block
-            at += len(block)
-            if not data:
-                return
+def _chr_index(block, off, index_of: dict) -> np.ndarray:
+    """uint32 chromosome index of the lines that start at `off` in block (uint8): the name is the text up to the
+    line's first tab, numbered in order of first appearance in index_of (name -> index), which spans the blocks"""
+    end = np.array(off, dtype=np.int64)
+    todo = np.arange(end.size)
+    while todo.size:  # every name to its tab at once, a byte a step (a locus line holds tabs)
+        todo = todo[block[end[todo]] != 9]
+        end[todo] += 1
+    mv = memoryview(block)
+    return np.array([index_of.setdefault(mv[a:b].tobytes(), len(index_of))
+                     for a, b in zip(np.asarray(off, dtype=np.int64).tolist(), end.tolist())], dtype=np.uint32)
 
 
 class _Labels:
     """labels of the loaded loci over the text blocks of a file, in file order"""
 
     def __init__(self):
-        self.names, self.index_of = [], {}
+        self.index_of = {}
         self.chr_index, self.positions, self.col_locus, self.col_allele = [], [], [], []
         self.base = 0
 
     def add(self, block, L, off, pos, loc, alle):
-        for o in off:  # chromosome = the text up to the first tab of the locus' line
-            o = int(o)
-            nm = block[o:block.index(b"\t", o)]
-            if nm not in self.index_of:
-                self.index_of[nm] = len(self.names)
-                self.names.append(nm)
-            self.chr_index.append(self.index_of[nm])
+        self.chr_index.append(_chr_index(block, off, self.index_of))
         self.positions.append(pos)
         self.col_locus.append(loc + self.base)
         self.col_allele.append(alle)
         self.base += L
 
-    def finish(self, kin) -> _LoadedColumns:
+    def finish(self) -> _LoadedColumns:
         cat = lambda parts, dt: np.concatenate(parts).astype(dt) if parts else np.zeros(0, dt)
-        return _LoadedColumns(kin, cat(self.col_locus, np.int64), cat(self.col_allele, np.uint8), self.names,
-                              np.array(self.chr_index, dtype=np.uint32), cat(self.positions, np.uint64))
+        return _LoadedColumns(cat(self.col_locus, np.int64), cat(self.col_allele, np.uint8), list(self.index_of),
+                              cat(self.chr_index, np.uint32), cat(self.positions, np.uint64))
 
 
 def _count_columns_bound(fname: str) -> int:
@@ -417,28 +385,18 @@ def _count_columns_bound(fname: str) -> int:
 _FMT_CHUNK_BYTES = 16 << 20  # rows per device formatter call: each of the two pinned buffers holds this many bytes
 
 
-def _kept_lines(block: bytes, at: int, off, pos, loc, names: list, index_of: dict):
+def _kept_lines(block, at: int, off, pos, loc, index_of: dict):
     """pass 1 of sync2csv over one text block: for every locus that emitted columns, the absolute byte offset of its
     line, the bytes pass 2 gathers for it (its line, plus a newline where the file's last line has none), its
     chromosome index, its position and its column count"""
     keep, cols = np.unique(loc, return_counts=True)  # the loader emits columns grouped by ascending locus
     o = off[keep].astype(np.int64)
-    buf = np.frombuffer(block, dtype=np.uint8)
-    nl = np.flatnonzero(buf == 10)
+    nl = np.flatnonzero(block == 10)
     k = np.searchsorted(nl, o)
     ends = nl[np.minimum(k, nl.size - 1)] + 1 if nl.size else np.zeros(o.size, np.int64)
-    ends = np.where(k < nl.size, ends, len(block))
-    size = ends - o + (ends == len(block)) * int(not block.endswith(b"\n"))
-    tabs = np.flatnonzero(buf == 9)
-    tab = tabs[np.searchsorted(tabs, o)]  # a locus line holds tabs
-    chr_idx = np.empty(o.size, dtype=np.uint32)
-    for j, (a, b) in enumerate(zip(o.tolist(), tab.tolist())):
-        nm = block[a:b]
-        if nm not in index_of:
-            index_of[nm] = len(names)
-            names.append(nm)
-        chr_idx[j] = index_of[nm]
-    return at + o, size, chr_idx, pos[keep], cols
+    ends = np.where(k < nl.size, ends, block.size)
+    size = ends - o + (ends == block.size) * int(block[-1] != 10)
+    return at + o, size, _chr_index(block, o, index_of), pos[keep], cols
 
 
 def write_csv(self, ctx: Context, filter_stats: FilterStats, keep_p_minus_1: bool, out: str, n_threads: int,
@@ -456,25 +414,24 @@ def write_csv(self, ctx: Context, filter_stats: FilterStats, keep_p_minus_1: boo
     block are the sorted loci's rows: within a locus, the columns keep the loader's order.
     `timings` (measurement only): filled with wall seconds per phase."""
     if out == "":
-        bname = ".".join(self.filename_sync.split(".")[:-1])
-        out = f"{bname}-{time.time()}-allele_frequencies.csv"
+        out = _default_out(self.filename_sync, "allele_frequencies")
     if os.path.exists(out):
         raise PgError("Cannot write to output file")
     fname = self.filename_sync
     n = len(self.pool_names)
-    max_loci = block_bytes // _line_min_bytes(n) + 2
+    max_loci = _max_loci(block_bytes, n)
     clock = time.perf_counter
     tm = {"pass1_s": 0.0, "sort_s": 0.0, "gather_s": 0.0, "parse_s": 0.0, "format_s": 0.0, "write_wait_s": 0.0}
     kin = capi.Kinship(ctx, n, text_block_columns(block_bytes, n))
     pinned = []
     try:
         t0 = clock()
-        names, index_of, parts = [], {}, []
-        for at, block in _text_blocks(fname, block_bytes):
+        index_of, parts = {}, []
+        for at, block in _line_blocks(fname, 0, os.path.getsize(fname), block_bytes, [np.empty(block_bytes, np.uint8)]):
             kin.reset()
             _L, off, pos, loc, _alle = kin.append_sync_text(block, filter_stats, max_loci, keep_p_minus_1)
             if loc.size:
-                parts.append(_kept_lines(block, at, off, pos, loc, names, index_of))
+                parts.append(_kept_lines(block, at, off, pos, loc, index_of))
         if not parts:
             raise PgError("No data passed the filtering variables. Please decrease minimum depth, and/or minimum "
                           "allele frequency.")  # assert at src/base/sync.rs:1219
@@ -482,10 +439,10 @@ def write_csv(self, ctx: Context, filter_stats: FilterStats, keep_p_minus_1: boo
         del parts
         tm["pass1_s"] = clock() - t0
         t0 = clock()
-        order = capi.sort_loci(positions, chr_names=names, chr_index=chr_idx)
+        order = capi.sort_loci(positions, chr_names=list(index_of), chr_index=chr_idx)
         line_at, size, positions, cols = line_at[order], size[order], positions[order], cols[order]
         tm["sort_s"] = clock() - t0
-        row_max = max(len(nm) for nm in names) + 25 + 19 * n  # chr,pos,allele + n numbers of at most 19 bytes + newline
+        row_max = max(map(len, index_of)) + 25 + 19 * n  # chr,pos,allele + n numbers of at most 19 bytes + newline
         bufs = []
         for _ in range(2):
             arr, h = ctx.pinned_empty((max(_FMT_CHUNK_BYTES, row_max),), np.uint8)
@@ -598,7 +555,7 @@ def _iter_with_kinship(self, ctx: Context, filter_stats: FilterStats, keep_p_min
     if cap < need:
         raise PgError(f"device_bytes {device_bytes} cannot hold one text block of {block_bytes} bytes: its "
                       f"{need} columns take {kin_device_bytes(n, need, k, block_bytes, sm_count)} bytes")
-    max_loci = block_bytes // _line_min_bytes(n) + 2
+    max_loci = _max_loci(block_bytes, n)
     clock = time.perf_counter
     tm = {"pass1_load_s": 0.0, "pass1_gram_s": 0.0, "eig_s": 0.0, "pass2_load_s": 0.0, "scan_s": 0.0}
     kin = capi.Kinship(ctx, n, cap)
@@ -612,8 +569,9 @@ def _iter_with_kinship(self, ctx: Context, filter_stats: FilterStats, keep_p_min
                 kin.partial_device_ptr()  # synchronises the handle's stream
             tm["pass1_gram_s"] += clock() - t0
 
-        for at, block in _text_blocks(self.filename_sync, block_bytes):
-            if kin.columns + text_block_columns(len(block), n, block.count(b"\n")) > cap:
+        for at, block in _line_blocks(self.filename_sync, 0, os.path.getsize(self.filename_sync), block_bytes,
+                                      [np.empty(block_bytes, np.uint8)]):
+            if kin.columns + text_block_columns(block.size, n, int(np.count_nonzero(block == 10))) > cap:
                 flush()
                 kin.reset()
                 dev_blocks.append([])
@@ -621,8 +579,8 @@ def _iter_with_kinship(self, ctx: Context, filter_stats: FilterStats, keep_p_min
             L, off, pos, loc, alle = kin.append_sync_text(block, filter_stats, max_loci, keep_p_minus_1)
             tm["pass1_load_s"] += clock() - t0
             lab.add(block, L, off, pos, loc, alle)
-            dev_blocks[-1].append((at, len(block), int(loc.size)))
-        ld = lab.finish(kin)
+            dev_blocks[-1].append((at, block.size, int(loc.size)))
+        ld = lab.finish()
         P = int(ld.col_locus.size)
         if P == 0:
             raise PgError("No data passed the filtering variables.")

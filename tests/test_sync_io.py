@@ -225,3 +225,45 @@ def test_mle_iter_with_kinship_file(ctx, tmp_path):
             ep = abs(got_p - op[i, j]) / max(op[i, j], 1e-12)
             worst = max(worst, eb, ep)
     assert worst < 1e-3, worst
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("entry", ["write_csv", "ols_iter_with_kinship"])
+def test_file_without_last_newline(ctx, tmp_path, entry):
+    """the file-level entries on a file whose last line has no newline: the same output as with the newline, at a
+    block size where that line is a block of its own and at one where it joins the block before it"""
+    from tests.test_text_gpu import _sync_text
+    c1 = H.load_c1()
+    L = 1200
+    chroms = [["chrB", "chrA"][(l // 250) % 2] for l in range(L)]
+    text = _sync_text(c1["counts"][:L], chroms, [int(p) for p in c1["pos"][:L]])
+    last = len(text) - 1 - text.rfind(b"\n", 0, len(text) - 1) - 1  # the last line without its newline
+    files = {}
+    for newline in (True, False):
+        files[newline] = str(tmp_path / f"k{int(newline)}.sync")
+        with open(files[newline], "wb") as fh:
+            fh.write(text if newline else text[:-1])
+    layouts = {}  # last line alone in its block -> block size
+    for bb in range(32 << 10, 31 << 10, -1):
+        sizes = [v.size for _, v in pb.sync_io._line_blocks(files[False], 0, len(text) - 1, bb,
+                                                             [np.empty(bb, np.uint8)])]
+        layouts.setdefault(len(sizes) > 1 and sizes[-1] == last, bb)
+        if len(layouts) == 2:
+            break
+    assert set(layouts) == {True, False}
+    fphen = str(tmp_path / "k.csv")
+    _write_c1_phen(fphen)
+    phen = pb.FilePhen(fphen, ",", 0, 1, [2, 3]).lparse()
+    fs = pb.FilterStats(pool_sizes=phen.pool_sizes, min_coverage_depth=5, min_allele_frequency=0.01)
+    outs = {}
+    for newline, fsync in files.items():
+        src = pb.FileSyncPhen(fsync, phen.pool_names, phen.pool_sizes, phen.phen_matrix, entry)
+        for alone, bb in layouts.items():
+            out = str(tmp_path / f"{entry}_{int(newline)}_{int(alone)}.csv")
+            if entry == "write_csv":
+                src.write_csv(ctx, fs, False, out, 2, block_bytes=bb)
+            else:
+                src.ols_iter_with_kinship(ctx, fs, True, 0.75, out, 2, block_bytes=bb)
+            outs[newline, alone] = open(out, "rb").read()
+    for alone in (True, False):
+        assert outs[False, alone] == outs[True, alone] and outs[True, alone].count(b"\n") > 1000

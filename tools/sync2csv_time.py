@@ -55,7 +55,7 @@ def formatter_alone(ctx, n):
     text = text[:text.rfind(b"\n", 0, BLOCK) + 1]
     fs = pb.FilterStats(pool_sizes=np.full(n, 1.0 / n), min_allele_frequency=0.001)
     kin = pb.Kinship(ctx, n, sync_io.text_block_columns(len(text), n))
-    L, off, pos, loc, alle = kin.append_sync_text(text, fs, len(text) // (12 * n + 5) + 2)
+    L, off, pos, loc, alle = kin.append_sync_text(text, fs, sync_io._max_loci(len(text), n))
     P = kin.columns
     G = kin.get_columns(0, P)
     host_rows = pb.format_frequency_rows(G, loc, alle, pos, text=text, line_offsets=off)
@@ -112,12 +112,14 @@ def parent_write_csv(src, ctx, fs, keep_p_minus_1, out, n_threads, block_bytes=B
     host threads"""
     n = len(src.pool_names)
     kin = capi.Kinship(ctx, n, sync_io._count_columns_bound(src.filename_sync))
-    max_loci = block_bytes // sync_io._line_min_bytes(n) + 2
+    max_loci = sync_io._max_loci(block_bytes, n)
     lab = sync_io._Labels()
+    fname = src.filename_sync
     try:
-        for _, block in sync_io._text_blocks(src.filename_sync, block_bytes):
+        for _, block in sync_io._line_blocks(fname, 0, os.path.getsize(fname), block_bytes,
+                                             [np.empty(block_bytes, np.uint8)]):
             lab.add(block, *kin.append_sync_text(block, fs, max_loci, keep_p_minus_1))
-        ld = lab.finish(kin)
+        ld = lab.finish()
         G = kin.get_columns(0, kin.columns)
     finally:
         kin.close()
