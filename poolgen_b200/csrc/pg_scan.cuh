@@ -413,6 +413,27 @@ __device__ __forceinline__ bool kind_is_ols(const ScanParams &p) {
     else return p.kind == PG_KIND_OLS;
 }
 
+// The reference's mean of a frequency column that holds the same value c in each of the m pools it averages: a
+// sequential sum of m copies of c, divided by m (pearsons_correlation, src/gwas/correlation_test.rs:7-71).  That need
+// not be c, and the centred values are then this rounding residue rather than 0: r comes out as noise that rounds to 0
+// (p = 1), and only where the mean is exactly c is r 0 / 0 = NaN.  A warp's tree sum of the same copies can land on c
+// when the sequential sum does not (or the other way round), so the correlation paths below take the mean of a
+// constant column from here.  Called by every lane (each gets the same value); constant columns are rare.
+static __device__ __noinline__ double ref_mean_of_constant(double c, double m) {
+    double s = 0.0;
+    for (double i = 0.0; i < m; i += 1.0) s = __dadd_rn(s, c);
+    return __ddiv_rn(s, m);
+}
+
+// smallest and largest value over the warp (every lane gets both)
+__device__ __forceinline__ void warp_min_max(double &lo, double &hi) {
+#pragma unroll
+    for (int off = 16; off >= 1; off >>= 1) {
+        lo = fmin(lo, __shfl_xor_sync(PG_FULL_MASK, lo, off));
+        hi = fmax(hi, __shfl_xor_sync(PG_FULL_MASK, hi, off));
+    }
+}
+
 // Reference-style two-pass evaluation of one locus straight from global memory by the whole warp (lane = pool):
 // explicit centred moments and explicit residuals e = y - Xb as src/gwas/ols.rs:98-104.  Used when the single-pass
 // Gram form would lose digits to cancellation (near-perfect fits, nearly constant or nearly collinear allele
@@ -430,9 +451,13 @@ __device__ __noinline__ int redo_locus(const ScanParams &p, int64_t locus, unsig
     double cntv = nn;
     // pass 0: means (the totals of the fast path are not trusted here)
     {
-        double sx[MS], sy[K], cnt = 0.0;
+        double sx[MS], sy[K], cnt = 0.0, lo[MS], hi[MS];
 #pragma unroll
-        for (int a = 0; a < MS; a++) sx[a] = 0.0;
+        for (int a = 0; a < MS; a++) {
+            sx[a] = 0.0;
+            lo[a] = INFINITY;
+            hi[a] = -INFINITY;
+        }
 #pragma unroll
         for (int k = 0; k < K; k++) sy[k] = 0.0;
         for_rows_coop<A>(p, locus, lane, [&](int i, const double(&f)[A], uint32_t d) {
@@ -451,13 +476,21 @@ __device__ __noinline__ int redo_locus(const ScanParams &p, int64_t locus, unsig
             if (mode == REDO_CORR_NAN && !valid) return;
             cnt += 1.0;
 #pragma unroll
-            for (int a = 0; a < MS; a++) sx[a] += x[a];
+            for (int a = 0; a < MS; a++) {
+                sx[a] += x[a];
+                lo[a] = fmin(lo[a], x[a]);
+                hi[a] = fmax(hi[a], x[a]);
+            }
 #pragma unroll
             for (int k = 0; k < K; k++) sy[k] += ys[k * n_pad + i];
         });
         cntv = warp_sum_fixed(cnt);
 #pragma unroll
-        for (int a = 0; a < MS; a++) xbar[a] = warp_sum_fixed(sx[a]) / cntv;
+        for (int a = 0; a < MS; a++) {
+            xbar[a] = warp_sum_fixed(sx[a]) / cntv;
+            warp_min_max(lo[a], hi[a]);
+            if (mode != REDO_OLS && a < m && lo[a] == hi[a] && xbar[a] == xbar[a]) xbar[a] = ref_mean_of_constant(lo[a], cntv);
+        }
 #pragma unroll
         for (int k = 0; k < K; k++) ybar[k] = warp_sum_fixed(sy[k]) / cntv;
     }
@@ -584,12 +617,16 @@ __device__ __noinline__ int corr_pairwise_locus(const ScanParams &p, int64_t loc
     const int n_pad = p.lay.n_pad;
     double xbar[K][MS], ybar[K];
     {
-        double cnt[K], sx[K][MS], sy[K];
+        double cnt[K], sx[K][MS], sy[K], lo[K][MS], hi[K][MS];
 #pragma unroll
         for (int k = 0; k < K; k++) {
             cnt[k] = sy[k] = 0.0;
 #pragma unroll
-            for (int a = 0; a < MS; a++) sx[k][a] = 0.0;
+            for (int a = 0; a < MS; a++) {
+                sx[k][a] = 0.0;
+                lo[k][a] = INFINITY;
+                hi[k][a] = -INFINITY;
+            }
         }
         for_rows_coop<A>(p, locus, lane, [&](int i, const double(&f)[A], uint32_t d) {
             double F[A], x[MS];
@@ -611,7 +648,11 @@ __device__ __noinline__ int corr_pairwise_locus(const ScanParams &p, int64_t loc
                     cnt[k] += 1.0;
                     sy[k] += y;
 #pragma unroll
-                    for (int a = 0; a < MS; a++) sx[k][a] += x[a];
+                    for (int a = 0; a < MS; a++) {
+                        sx[k][a] += x[a];
+                        lo[k][a] = fmin(lo[k][a], x[a]);
+                        hi[k][a] = fmax(hi[k][a], x[a]);
+                    }
                 }
             }
         });
@@ -620,7 +661,11 @@ __device__ __noinline__ int corr_pairwise_locus(const ScanParams &p, int64_t loc
             const double c = warp_sum_fixed(cnt[k]);
             ybar[k] = warp_sum_fixed(sy[k]) / c;
 #pragma unroll
-            for (int a = 0; a < MS; a++) xbar[k][a] = warp_sum_fixed(sx[k][a]) / c;
+            for (int a = 0; a < MS; a++) {
+                xbar[k][a] = warp_sum_fixed(sx[k][a]) / c;
+                warp_min_max(lo[k][a], hi[k][a]);
+                if (a < m && lo[k][a] == hi[k][a]) xbar[k][a] = ref_mean_of_constant(lo[k][a], c);
+            }
         }
     }
     double sxx[K][MS], sxy[K][MS], syy[K];
