@@ -114,7 +114,9 @@ int pg_pinned_free(pg_ctx *ctx, void *p);
  * n_alleles / allele_codes name the count columns the caller ships per pool (a subset of the six
  * sync columns, in sync order).  When filter->remove_ns is set a column coded N(4) is dropped on
  * the device exactly like src/base/sync.rs:200-213.
- * phen: n_pools x k row-major f64 (Phen.phen_matrix, src/base/phen.rs:86-97); NULL/0 for the table tests. */
+ * phen: n_pools x k row-major f64 (Phen.phen_matrix, src/base/phen.rs:86-97); NULL/0 for the table tests.
+ * n_pools: any count for every kind except PG_KIND_GWALPHA_LS / _ML, which take up to 64 pools (PG_ERR_UNSUPPORTED
+ *   above that). */
 int pg_scan_open(pg_ctx *ctx, int kind, const pg_filter *filter, int n_pools, int n_alleles,
                  const uint8_t *allele_codes, const double *phen, int k, pg_scan **out);
 int pg_scan_close(pg_scan *scan);

@@ -252,12 +252,6 @@ int pg_scan_open(pg_ctx *ctx, int kind, const pg_filter *filter, int n_pools, in
             return fail(ctx, PG_ERR_UNSUPPORTED, "pg_scan_open: ols_iter needs at least 2 pools");
         }
         s->ln_beta = s->df > 0.0 ? pg::statrs::ln_gamma(s->df / 2.0 + 0.5) - pg::statrs::ln_gamma(s->df / 2.0) - pg::statrs::ln_gamma(0.5) : 0.0;
-        // the phenotype (and weight) vectors of a pass stay resident in shared memory next to the warps' rings: at
-        // least one phenotype per pass has to fit beside ~8 warps of 16 KB
-        if ((size_t)2 * np * 8 > 96 * 1024) {
-            delete s;
-            return fail(ctx, PG_ERR_UNSUPPORTED, "pg_scan_open: %d pools exceed the shared-memory resident phenotype budget (6,144 pools)", n);
-        }
         const char *pv_mode = getenv("PG_PVALUE");
         if (s->df > 0.0 && !(pv_mode && strcmp(pv_mode, "cf") == 0)) {
             pg::PTable tab = pg::build_ptable(s->df);
@@ -581,10 +575,11 @@ static int run_once(pg_batch *b, int *launches) {
     if (!b->have_input) return fail(ctx, PG_ERR_STATE, "pg_batch_run: no input uploaded");
     if (b->n_loci == 0) return PG_OK;
     if (is_regression(s)) {
-        // phenotypes per pass: bounded by the accumulator registers and by the shared memory the resident phenotype
-        // vectors may take (96 KB of the 227 KB, the rest belongs to the warps' rings)
+        // phenotypes per pass: bounded by the accumulator registers and, unless the scan reads them from L2
+        // (pg::scan_wide), by the shared memory the resident phenotype vectors may take (96 KB of the 227 KB, the
+        // rest belongs to the warps' rings)
         int kpass = pg::max_phen_per_pass(s->A_dev);
-        {
+        if (!pg::scan_wide(s->lay)) {
             const int fit = (int)((size_t)(96 * 1024) / ((size_t)s->lay.n_pad * 8)) - (s->weighted ? 1 : 0);
             if (kpass > fit) kpass = fit < 1 ? 1 : fit;
         }

@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <stdlib.h>
 #include <string>
 #include <utility>
 #include <vector>
@@ -64,6 +65,16 @@ inline Layout make_layout(int n, int A) {
 constexpr int kMaxPhenPerPass = 4;
 // phenotypes per kernel pass: bounded by the accumulator registers (A + A(A+1)/2 + A*K doubles per lane)
 inline int max_phen_per_pass(int A) { return A <= 4 ? 4 : (A == 5 ? 3 : 2); }
+
+// The OLS / Pearson scan keeps a pass's phenotype vectors and the pool weights resident in shared memory, in at most
+// 96 KB: one phenotype and the weights fit up to 6,144 pools.  Above that scan_kernel_wide (pg_scan.cuh) reads them
+// from L2 and takes as many phenotypes per pass as the registers allow.  PG_SCAN_WIDE (tests, read once per process)
+// takes the wide kernel wherever the scan runs 32 lanes per locus (more than one row chunk).
+constexpr int kResidentPhenPools = 6144;
+inline bool scan_wide(const Layout &lay) {
+    static const bool force = getenv("PG_SCAN_WIDE") != nullptr;
+    return lay.n_chunks > 1 && (lay.n_pad > kResidentPhenPools || force);
+}
 
 // parameters of one ols/corr scan launch (passed by value)
 struct ScanParams {

@@ -1435,13 +1435,26 @@ __global__ void __launch_bounds__(kFixWarps * 32) fixup_kernel(const __grid_cons
     }
 }
 
+// a pair of consecutive phenotype (or weight) entries of phase 1: from shared memory, or (YG) from global memory
+// through the read-only path
+template <bool YG>
+__device__ __forceinline__ double2 ld_pair(const double *a) {
+    if (YG) return __ldg(reinterpret_cast<const double2 *>(a));
+    return *reinterpret_cast<const double2 *>(a);
+}
+
 // ---- the kernel ----------------------------------------------------------------------------------------------
-template <int A, int K, bool W, int P, int KIND>
-__global__ void __launch_bounds__(kScanWarps * 32, 1) scan_kernel(const __grid_constant__ ScanParams p) {
+// YG = false (scan_kernel): every CTA copies the phenotype vectors of the pass and the pool weights into shared memory
+// (common_bytes, at most 96 KB: up to 6,144 pools).  YG = true (scan_kernel_wide, P = 32 only): phase 1 reads them
+// from global memory, where K * n_pad * 8 bytes stay resident in L2 for the whole launch, and the shared memory is all
+// the warps' -- any pool count.  The two read the same values in the same order, so a locus gets the same records
+// bit for bit from either kernel.
+template <int A, int K, bool W, int P, int KIND, bool YG>
+__device__ __forceinline__ void scan_body(const ScanParams &p, unsigned char *smem) {
+    static_assert(!YG || P == 32, "the wide kernel streams row chunks: 32 lanes per locus");
     using AC = Acc<A, K, W>;
     constexpr int LPS = 32 / P;  // loci per stage
     constexpr int RC = chunk_rows(A);
-    extern __shared__ __align__(128) unsigned char smem[];
     // the out-of-line phase-2 functions take the parameter block by reference: give them a shared-memory copy
     // (a reference to the kernel parameter itself would be spilled to per-thread local memory)
     __shared__ __align__(16) ScanParams sp_storage;
@@ -1452,8 +1465,10 @@ __global__ void __launch_bounds__(kScanWarps * 32, 1) scan_kernel(const __grid_c
     const int n_pad = lay.n_pad;
     const int G = p.block_loci;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
-    double *ys = reinterpret_cast<double *>(smem);
-    double *ws = W ? ys + (size_t)K * n_pad : nullptr;
+    double *ys_s = reinterpret_cast<double *>(smem);
+    double *ws_s = W ? ys_s + (size_t)K * n_pad : nullptr;
+    const double *ys = YG ? p.yc : ys_s;
+    const double *ws = YG ? (W ? p.w : nullptr) : ws_s;
     unsigned char *wb = smem + p.common_bytes + (size_t)warp * p.warp_bytes;
     uint64_t *bars = reinterpret_cast<uint64_t *>(wb);
     unsigned char *stage0 = wb + 64;
@@ -1461,9 +1476,11 @@ __global__ void __launch_bounds__(kScanWarps * 32, 1) scan_kernel(const __grid_c
     const int nbuf = p.nbuf;
     const int red_rows = max(1, min((int)(p.stage_bytes / (kRedPitch * 8)), AC::N));  // launch_scan_p keeps a stage >= one row
 
-    for (int i = threadIdx.x; i < K * n_pad; i += blockDim.x) ys[i] = p.yc[i];
-    if (W)
-        for (int i = threadIdx.x; i < n_pad; i += blockDim.x) ws[i] = p.w[i];
+    if (!YG) {
+        for (int i = threadIdx.x; i < K * n_pad; i += blockDim.x) ys_s[i] = p.yc[i];
+        if (W)
+            for (int i = threadIdx.x; i < n_pad; i += blockDim.x) ws_s[i] = p.w[i];
+    }
     if (lane == 0) {
         for (int b = 0; b < nbuf; b++) mbar_init(&bars[b], 1);
         fence_mbar_init();
@@ -1553,7 +1570,23 @@ __global__ void __launch_bounds__(kScanWarps * 32, 1) scan_kernel(const __grid_c
                     const double *wrow = W ? ws + chunk * RC + 2 * lane : nullptr;
                     mbar_wait(&bars[buf], parity);
                     double *fb = reinterpret_cast<double *>(stage0 + (size_t)buf * p.stage_bytes);
-                    if (chunk < n_chunks - 1 || lay.rc_last == RC) {
+                    if (YG && (chunk < n_chunks - 1 || lay.rc_last == RC)) {
+                        // the same row pairs in the same order; at five and six alleles not unrolled: the 64-bit
+                        // global addresses of an unrolled second pair would spill beside the largest accumulator sets
+                        const double *fl = fb + 2 * lane;
+#pragma unroll(A >= 5 ? 1 : RC / 64)
+                        for (int it = 0; it < RC / 64; it++) {
+                            double2 f2[A], y2[K];
+#pragma unroll
+                            for (int j = 0; j < A; j++) f2[j] = *reinterpret_cast<const double2 *>(fl + j * RC + it * 64);
+#pragma unroll
+                            for (int k = 0; k < K; k++) y2[k] = ld_pair<true>(yrow + (size_t)k * n_pad + it * 64);
+                            double2 w2 = make_double2(0.0, 0.0);
+                            if (W) w2 = ld_pair<true>(wrow + it * 64);
+                            if (hinted) renorm_pair<A>(f2, hkept, chunk * RC + it * 64 + 2 * lane, lay.n);
+                            accum_pair<A, K, W>(acc, f2, y2, w2);
+                        }
+                    } else if (chunk < n_chunks - 1 || lay.rc_last == RC) {
                         const double *fl = fb + 2 * lane;
 #pragma unroll
                         for (int it = 0; it < RC / 64; it++) {
@@ -1561,10 +1594,9 @@ __global__ void __launch_bounds__(kScanWarps * 32, 1) scan_kernel(const __grid_c
 #pragma unroll
                             for (int j = 0; j < A; j++) f2[j] = *reinterpret_cast<const double2 *>(fl + j * RC + it * 64);
 #pragma unroll
-                            for (int k = 0; k < K; k++)
-                                y2[k] = *reinterpret_cast<const double2 *>(yrow + (size_t)k * n_pad + it * 64);
+                            for (int k = 0; k < K; k++) y2[k] = ld_pair<YG>(yrow + (size_t)k * n_pad + it * 64);
                             double2 w2 = make_double2(0.0, 0.0);
-                            if (W) w2 = *reinterpret_cast<const double2 *>(wrow + it * 64);
+                            if (W) w2 = ld_pair<YG>(wrow + it * 64);
                             if (hinted) renorm_pair<A>(f2, hkept, chunk * RC + it * 64 + 2 * lane, lay.n);
                             accum_pair<A, K, W>(acc, f2, y2, w2);
                         }
@@ -1575,10 +1607,9 @@ __global__ void __launch_bounds__(kScanWarps * 32, 1) scan_kernel(const __grid_c
 #pragma unroll
                             for (int j = 0; j < A; j++) f2[j] = *reinterpret_cast<const double2 *>(fb + (size_t)j * rcc + r);
 #pragma unroll
-                            for (int k = 0; k < K; k++)
-                                y2[k] = *reinterpret_cast<const double2 *>(ys + chunk * RC + (size_t)k * n_pad + r);
+                            for (int k = 0; k < K; k++) y2[k] = ld_pair<YG>(ys + chunk * RC + (size_t)k * n_pad + r);
                             double2 w2 = make_double2(0.0, 0.0);
-                            if (W) w2 = *reinterpret_cast<const double2 *>(ws + chunk * RC + r);
+                            if (W) w2 = ld_pair<YG>(ws + chunk * RC + r);
                             if (hinted) renorm_pair<A>(f2, hkept, chunk * RC + r, lay.n);
                             accum_pair<A, K, W>(acc, f2, y2, w2);
                         }
@@ -1649,12 +1680,25 @@ __global__ void __launch_bounds__(kScanWarps * 32, 1) scan_kernel(const __grid_c
     }
 }
 
-template <int A, int K, bool W, int P>
+template <int A, int K, bool W, int P, int KIND>
+__global__ void __launch_bounds__(kScanWarps * 32, 1) scan_kernel(const __grid_constant__ ScanParams p) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    scan_body<A, K, W, P, KIND, false>(p, smem);
+}
+
+template <int A, int K, bool W, int KIND>
+__global__ void __launch_bounds__(kScanWarps * 32, 1) scan_kernel_wide(const __grid_constant__ ScanParams p) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    scan_body<A, K, W, 32, KIND, true>(p, smem);
+}
+
+// YG: scan_kernel_wide, which needs no shared memory for the phenotypes (P = 32 only)
+template <int A, int K, bool W, int P, bool YG>
 cudaError_t launch_scan_p(ScanParams p, int sm_count, cudaStream_t s) {
     using AC = Acc<A, K, W>;
     const Layout &lay = p.lay;
     const size_t avail = 227 * 1024 - 512;  // 512 B of static shared memory hold the parameter copy
-    size_t common = (size_t)(K + (W ? 1 : 0)) * lay.n_pad * 8;
+    size_t common = YG ? 0 : (size_t)(K + (W ? 1 : 0)) * lay.n_pad * 8;
     common = (common + 127) / 128 * 128;
     size_t stage = (P == 32) ? (size_t)A * lay.rc * 8 : (size_t)(32 / P) * lay.freq_stride() * 8;
     stage = (stage + 127) / 128 * 128;
@@ -1707,7 +1751,11 @@ cudaError_t launch_scan_p(ScanParams p, int sm_count, cudaStream_t s) {
     p.nbuf = nbuf;
     p.block_loci = G;
     const size_t smem = common + (size_t)nwarps * wbytes;
-    auto kern = (p.kind == PG_KIND_OLS) ? scan_kernel<A, K, W, P, PG_KIND_OLS> : scan_kernel<A, K, W, P, PG_KIND_CORR>;
+    void (*kern)(ScanParams);
+    if constexpr (YG)
+        kern = (p.kind == PG_KIND_OLS) ? scan_kernel_wide<A, K, W, PG_KIND_OLS> : scan_kernel_wide<A, K, W, PG_KIND_CORR>;
+    else
+        kern = (p.kind == PG_KIND_OLS) ? scan_kernel<A, K, W, P, PG_KIND_OLS> : scan_kernel<A, K, W, P, PG_KIND_CORR>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     const int64_t NB = (p.n_loci + G - 1) / G;
@@ -1733,10 +1781,11 @@ cudaError_t launch_scan_t(const ScanParams &p, int sm_count, cudaStream_t s) {
     if (p.lay.n_chunks == 1) {
         // 16 lanes per locus keep the stage at two loci (more resident warps); tiny pool counts use 8
         const int P = p.p_override ? p.p_override : (p.lay.n_pad > 64 ? 16 : 8);
-        if (P == 16) return launch_scan_p<A, K, W, 16>(p, sm_count, s);
-        return launch_scan_p<A, K, W, 8>(p, sm_count, s);
+        if (P == 16) return launch_scan_p<A, K, W, 16, false>(p, sm_count, s);
+        return launch_scan_p<A, K, W, 8, false>(p, sm_count, s);
     }
-    return launch_scan_p<A, K, W, 32>(p, sm_count, s);
+    if (scan_wide(p.lay)) return launch_scan_p<A, K, W, 32, true>(p, sm_count, s);
+    return launch_scan_p<A, K, W, 32, false>(p, sm_count, s);
 }
 
 template <int A>
